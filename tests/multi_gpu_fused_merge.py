@@ -90,7 +90,7 @@ def main():
     las_whole, _ = ops.build_las_pf3(whole, scale=(0.001,) * 3, year=2026, day_of_year=7)
     txt_whole, _ = ops.pcd_ascii_body(whole)
     hdr = LiDARMotionSimulator._pcd_header(N)
-    tmp = os.path.join(tempfile.gettempdir(), "lmc_sharded_files")
+    tmp = os.environ.get("LMC_OUT") or os.path.join(tempfile.gettempdir(), "lmc_sharded_files")
     if rank == 0:
         os.makedirs(tmp, exist_ok=True)
         for f in ("a.lvx", "a.las", "a.pcd"):

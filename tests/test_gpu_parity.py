@@ -1400,7 +1400,7 @@ def test_host_buffer_pipeline_equals_resident(mode):
         assert (hs.out - want.cpu()).abs().max().item() <= 1e-5       # device-built vs host-built table: same to f32 rounding
 
 
-def test_fused_merge_multi_gpu():
+def test_fused_merge_multi_gpu(tmp_path):
     """>= 2 GPUs only (skipped on the 1-GPU test box): peer-store epilogue == NCCL all-gather == single rank."""
     import subprocess
     import sys
@@ -1409,7 +1409,7 @@ def test_fused_merge_multi_gpu():
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",
                         "--master-port", "29641", os.path.join(root, "tests", "multi_gpu_fused_merge.py")],
-                       capture_output=True, text=True, timeout=600, env=dict(os.environ, LMC_F="1500"))
+                       capture_output=True, text=True, timeout=600, env=dict(os.environ, LMC_F="1500", LMC_OUT=str(tmp_path)))
     assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-3000:]
     assert "OK world=2" in r.stdout
 
