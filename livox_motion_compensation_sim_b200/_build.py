@@ -27,7 +27,7 @@ def needs_build() -> bool:
     if not os.path.exists(LIB_PATH):
         return True
     t = os.path.getmtime(LIB_PATH)
-    deps = sources() + glob.glob(os.path.join(CSRC, "*.cuh")) + [os.path.join(PKG_DIR, "..", "include", "lmc_b200.h")]
+    deps = sources() + glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(os.path.join(CSRC, "*.h")) + [os.path.join(PKG_DIR, "..", "include", "lmc_b200.h")]
     return any(os.path.getmtime(d) > t for d in deps)
 
 

@@ -12,7 +12,7 @@
 
 namespace lmc {
 cudaError_t launch_direct(bool f64, int mode, const Params& P, cudaStream_t st);
-cudaError_t launch_tma(bool f64, int mode, const Params& P, cudaStream_t st, bool force, bool* handled);
+cudaError_t launch_stream(bool f64, int mode, const Params& P, const Plan& pl, int dev, cudaStream_t st);
 cudaError_t launch_pose_lookup(const double*, int64_t, const double*, const double*, int32_t, double*, int32_t*, cudaStream_t);
 cudaError_t launch_pcd_size(bool f64, const void* pts, int64_t n, int64_t* tile_off, cudaStream_t st);
 cudaError_t launch_pcd_write(bool f64, const void* pts, int64_t n, const int64_t* tile_off, uint8_t* out, uint32_t* status, cudaStream_t st);
@@ -58,18 +58,23 @@ bool aligned32(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 31u) ==
 // row slice of a frame-major buffer (a rank's shard) can be passed as it is
 bool aligned_row(const void* p, bool f64) { return (reinterpret_cast<uintptr_t>(p) & (f64 ? 31u : 15u)) == 0; }
 
-// the kernels are built for sm_100a only: refuse anything else loudly (no fallback path exists)
+// The device this thread last checked: sm_100 (the kernels are built for sm_100a only and refuse anything else loudly,
+// no fallback path exists), and its SM count, which sizes the persistent grid of the streaming kernels.
+struct DeviceRecord { int dev = -1, sm_count = 0; };
+thread_local DeviceRecord g_dev;
+
 int check_device() {
-    static thread_local int ok_dev = -1;
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return cuda_fail(e, "cudaGetDevice");
-    if (dev == ok_dev) return LMC_OK;
-    int major = 0;
+    if (dev == g_dev.dev) return LMC_OK;
+    int major = 0, sms = 0;
     e = cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev);
     if (e != cudaSuccess) return cuda_fail(e, "cudaDeviceGetAttribute");
     if (major != 10) return fail(LMC_ERR_CUDA, "device %d is sm_%d0; liblmc_b200 is built for sm_100a only", dev, major);
-    ok_dev = dev;
+    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaDeviceGetAttribute");
+    g_dev = { dev, sms };
     return LMC_OK;
 }
 
@@ -122,16 +127,14 @@ int run(bool f64, int mode, lmc::Params& P, const lmc_export* ex, void* stream) 
     rc = fill_export(P, ex);
     if (rc != LMC_OK) return rc;
     if (!P.out && !P.lvx14 && !P.las_x && !P.las_int) return fail(LMC_ERR_INVALID, "no output requested");
+    const lmc::Plan pl = lmc::plan_point_launch(f64, mode, P, g_path.load(std::memory_order_relaxed), g_dev.sm_count);
+    if (pl.rc != LMC_OK) return fail(pl.rc, "%s", pl.msg);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cudaError_t e;
-    bool handled = false;
-    const int path = g_path.load(std::memory_order_relaxed);
-    if (path >= 1 || P.n_peers > 0) {
-        e = lmc::launch_tma(f64, mode, P, st, path == 2 || P.n_peers > 0, &handled);
-        if (handled) return e == cudaSuccess ? LMC_OK : cuda_fail(e, "launch (tma path)");
+    if (pl.stream) {
+        const cudaError_t e = lmc::launch_stream(f64, mode, P, pl, g_dev.dev, st);
+        return e == cudaSuccess ? LMC_OK : cuda_fail(e, "launch (tma path)");
     }
-    if (P.n_peers > 0) return fail(LMC_ERR_INVALID, "peer stores need the streaming kernels (16-byte aligned timestamp / tag arrays)");
-    e = lmc::launch_direct(f64, mode, P, st);
+    const cudaError_t e = lmc::launch_direct(f64, mode, P, st);
     return e == cudaSuccess ? LMC_OK : cuda_fail(e, "launch (direct path)");
 }
 

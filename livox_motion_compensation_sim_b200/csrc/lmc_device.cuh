@@ -9,47 +9,12 @@
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
-#include "../../include/lmc_b200.h"
+#include "lmc_plan.h"
 
 namespace lmc {
 
 constexpr int kMaxBnd    = 30;        // frame boundaries cached per tile (more -> per-point global search)
 constexpr int kSegStride = 22;        // doubles per Mode C sample row
-
-enum Mode : int { kRigid = 0, kGyro = 1, kSlerp = 2, kQuantOnly = 3 };
-
-// One launch = one Params block in constant/param space.
-struct Params {
-    const void*     pts;          // (N,4) f64 or (N) float4
-    void*           out;          // same layout, may be null
-    const void*     ts;           // int64[N] (f64 layout) | uint32[N] ns offsets (f32 layout)
-    const int64_t*  frame_off;    // CSR, n_frames + 1
-    const int64_t*  frame_start;  // int64[n_frames] ns
-    const double*   pose_Rt;      // Mode A: (n_frames, 12)
-    const int64_t*  samp_ts;      // Mode B: imu_ts | Mode C: sample_ts
-    const double*   samp_tab;     // Mode B: imu_gyro (S,3) | Mode C: seg (S,20)
-    const int32_t*  hold_idx;     // Mode C hold-next (optional)
-    int64_t         n_samp;
-    int64_t         n_points, p_begin, p_end;
-    int32_t         n_frames;
-    // fused export epilogues
-    uint8_t*        lvx14;
-    const uint8_t*  tag;
-    int32_t*        las_x;
-    int32_t*        las_y;
-    int32_t*        las_z;
-    uint16_t*       las_int;
-    uint32_t*       status;
-    double          las_scale[3], las_rcp[3], las_off[3];      // las_rcp = 1/scale (host, correctly rounded)
-    int32_t         lvx_mode, las_int_mode;
-    // fused merged-cloud assembly: peer-mapped copies of out / lvx14 on the other ranks
-    int32_t         n_peers;
-    void*           peer_out[LMC_MAX_PEERS];
-    uint8_t*        peer_lvx[LMC_MAX_PEERS];
-    // the same through the NVSwitch multicast mapping of the symmetric buffers (multimem.st)
-    void*           mc_out;
-    uint8_t*        mc_lvx;
-};
 
 struct Pt { double x, y, z, w; };
 

@@ -215,13 +215,9 @@ static cudaError_t launch_fused(const Params& P, cudaStream_t st) {
 }
 
 cudaError_t launch_direct(bool f64, int mode, const Params& P, cudaStream_t st) {
-    switch (mode) {
-    case kRigid:     return f64 ? launch_fused<true, kRigid>(P, st)     : launch_fused<false, kRigid>(P, st);
-    case kGyro:      return f64 ? launch_fused<true, kGyro>(P, st)      : launch_fused<false, kGyro>(P, st);
-    case kSlerp:     return f64 ? launch_fused<true, kSlerp>(P, st)     : launch_fused<false, kSlerp>(P, st);
-    case kQuantOnly: return f64 ? launch_fused<true, kQuantOnly>(P, st) : launch_fused<false, kQuantOnly>(P, st);
-    }
-    return cudaErrorInvalidValue;
+    return dispatch_layout_mode(f64, mode, [&](auto f64_c, auto mode_c) {
+        return launch_fused<decltype(f64_c)::value, decltype(mode_c)::value>(P, st);
+    });
 }
 
 cudaError_t launch_pose_lookup(const double* traj_t, int64_t n_t, const double* traj_Rt, const double* frame_t,

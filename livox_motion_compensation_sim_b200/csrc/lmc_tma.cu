@@ -16,31 +16,18 @@
 //                   output side needs no CTA-wide barrier at all.
 //
 // Edge tiles (a shard's ragged first / last tile) skip TMA and take guarded global loads.
-#include <cstdlib>
 #include <type_traits>
 #include "lmc_device.cuh"
 
 namespace lmc {
 
-#ifndef LMC_CW
-#define LMC_CW 15
-#endif
-constexpr int kCW            = LMC_CW;                   // consumer warps (15 + producer = 512 threads -> 128 regs each)
 constexpr int kStreamThreads = 32 * (kCW + 1);           // + producer warp
 
-// Tile shape per kernel family (measured on B200, see profiles/): Mode C on float4 points amortises its
-// per-tile bookkeeping best with 3 pairs per thread over a 3-stage ring; everything else runs 2 pairs
-// (f32) / 1 pair (f64) per thread over 4 stages.
-#ifndef LMC_PPT_SLERP
-#define LMC_PPT_SLERP 3
-#endif
-#ifndef LMC_STAGES
-#define LMC_STAGES 4
-#endif
+// tile shape: lmc_plan.h (the launch plan sizes the grid with the same tile)
 template <bool F64, int MODE> struct StreamCfg {
-    static constexpr int PPT      = F64 ? 1 : (MODE == kSlerp ? LMC_PPT_SLERP : 2);   // point pairs per consumer thread per tile
-    static constexpr int STAGES   = (!F64 && MODE == kSlerp && LMC_PPT_SLERP == 3) ? 3 : LMC_STAGES;
-    static constexpr int TP       = kCW * 32 * 2 * PPT;          // points per tile: 960 (f64) / 1920 / 2880 (f32)
+    static constexpr int PPT      = stream_pairs_per_thread(F64, MODE);   // point pairs per consumer thread per tile
+    static constexpr int STAGES   = (!F64 && MODE == kSlerp) ? 3 : 4;
+    static constexpr int TP       = stream_tile_points(F64, MODE);
     static constexpr int PT_BYTES = F64 ? 32 : 16;
     static constexpr int TS_BYTES = F64 ? 8 : 4;
     static constexpr int PTS_STAGE = TP * PT_BYTES;
@@ -89,20 +76,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  :: "r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
-
-// Export configuration known at compile time ("lean" kernels) or tested at run time (kExGeneric).
-// Lean variants also assume what the launcher has verified: LVX records are type-2-of-input without
-// tag bytes, timestamps / frame starts are present where the mode needs them, no hold_idx,
-// 2 <= n_samp < 2^31.
-// kExLvx2 (with kExLvx): the records are CS:365-374 on the COMPENSATED point (+ optional tag bytes) instead of LMC:252-272 on
-// the raw one -- the second simulator's product, lean for Mode B.
-// kExMc (with kExOut | kExLvx): fused merged-cloud assembly through the NVSwitch multicast mapping of the symmetric buffers --
-// every result of a full tile leaves as ONE multimem.st (the switch replicates it into every rank's copy, this rank's
-// included) instead of a local store plus one store per peer; ragged edge tiles fall back to local + per-peer stores.
-// kExPb (with kExOut | kExLvx): fused merged-cloud assembly by TMA BULK stores -- the warp writes its results back over its own
-// points in the stage, and its contiguous run of the tile (aligned cloud) plus its record slab leave as one bulk store per
-// destination (this rank's copy and every peer's over NVLink) instead of one register store per result and peer.
-constexpr int kExOut = 1, kExLvx = 2, kExLas = 4, kExGeneric = 8, kExLvx2 = 16, kExMc = 32, kExPb = 64;
 
 // 16 bytes to the multicast address (PTX multimem.st; the switch fans the write out to every member of the group)
 __device__ __forceinline__ void mc_st128(void* mc, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
@@ -460,84 +433,40 @@ __global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_const
 }
 
 // ---- launcher ----------------------------------------------------------------------------------
-static int sm_count_cached() {
-    static thread_local int dev_cached = -1, sms = 0;
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    if (dev != dev_cached) {
-        if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-        dev_cached = dev;
-    }
-    return sms;
-}
-
 template <bool F64, int MODE, int EX>
-static cudaError_t launch_stream_ex(const Params& P, cudaStream_t st, int grid, int64_t tile0, int64_t n_tiles) {
+static cudaError_t launch_stream_ex(const Params& P, const Plan& pl, int dev, cudaStream_t st) {
     using Cfg = StreamCfg<F64, MODE>;
     static thread_local int attr_dev = -1;
-    int dev = 0;
-    cudaGetDevice(&dev);
     if (attr_dev != dev) {
         cudaError_t e = cudaFuncSetAttribute(k_stream<F64, MODE, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
         if (e != cudaSuccess) return e;
         attr_dev = dev;
     }
-    k_stream<F64, MODE, EX><<<grid, kStreamThreads, Cfg::SMEM, st>>>(P, tile0, n_tiles);
+    k_stream<F64, MODE, EX><<<pl.grid, kStreamThreads, Cfg::SMEM, st>>>(P, pl.tile0, pl.n_tiles);
     return cudaGetLastError();
 }
 
-template <bool F64, int MODE>
-static cudaError_t launch_stream(const Params& P, cudaStream_t st, bool force, bool* handled) {
-    using Cfg = StreamCfg<F64, MODE>;
-    const int sms = sm_count_cached();
-    if (sms <= 0) return cudaErrorInvalidDevice;
-    const int64_t tile0 = (P.p_begin / Cfg::TP) * Cfg::TP;                       // tiles aligned in GLOBAL index space
-    const int64_t n_tiles = (P.p_end - tile0 + Cfg::TP - 1) / Cfg::TP;
-    if (!force && n_tiles < 2 * (int64_t)sms) { *handled = false; return cudaSuccess; }   // too small to fill a persistent grid
-    // TMA sources must be 16-byte aligned: guaranteed by the 32-byte rule for points, checked here for the rest
-    if (P.ts != nullptr && (reinterpret_cast<uintptr_t>(P.ts) & 15u)) { *handled = false; return cudaSuccess; }
-    if (P.tag != nullptr && (reinterpret_cast<uintptr_t>(P.tag) & 15u)) { *handled = false; return cudaSuccess; }
-    *handled = true;
-    const int grid = (int)(n_tiles < sms ? n_tiles : sms);
-    // lean (compile-time export configuration) variants for the common cases of Mode A / Mode C
-    if constexpr (MODE == kRigid || MODE == kSlerp || MODE == kGyro) {
-        const int mask = (P.out ? kExOut : 0) | (P.lvx14 ? kExLvx : 0) | ((P.las_x || P.las_int) ? kExLas : 0);
-        const bool lvx2 = P.lvx14 && P.lvx_mode == LMC_LVX2_OF_OUTPUT;
-        const bool mc = P.mc_out != nullptr && P.mc_lvx != nullptr;           // multicast merge: lean out + LVX kernel, float4 layout
-        static const bool pb_on = [] { const char* e = getenv("LMC_PEER_BULK"); return !(e && e[0] == '0'); }();   // (experiments: LMC_PEER_BULK=0 keeps the register peer stores)
-        const bool pb = pb_on && !mc && P.n_peers > 0 && MODE != kGyro && !F64 && mask == (kExOut | kExLvx) && !lvx2;
-        if (mc && !(MODE != kGyro && !F64 && mask == (kExOut | kExLvx) && !lvx2)) return cudaErrorInvalidValue;
-        bool lean = (P.n_peers == 0 || mc || pb) && (!lvx2 || MODE == kGyro) && (!(mask & kExLas) || (P.las_x && P.las_int));
-        if (MODE == kSlerp) lean = lean && P.hold_idx == nullptr && P.ts != nullptr && P.n_samp >= 2 && P.n_samp < 0x7fffffffLL &&
-                                   (F64 || P.frame_start != nullptr);
-        if (MODE == kGyro)  lean = lean && P.ts != nullptr && P.frame_start != nullptr && P.n_samp >= 2 && P.n_samp < 0x7fffffffLL;
-        if (mc && !lean) return cudaErrorInvalidValue;
-        if constexpr (MODE != kGyro && !F64) {
-            if (lean && mc) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExMc>(P, st, grid, tile0, n_tiles);
-            if (lean && pb) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExPb>(P, st, grid, tile0, n_tiles);
-        }
-        if (lean) {
-            if (mask == kExOut)            return launch_stream_ex<F64, MODE, kExOut>(P, st, grid, tile0, n_tiles);
-            if constexpr (MODE == kGyro) {
-                if (mask == (kExOut | kExLvx) && lvx2) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExLvx2>(P, st, grid, tile0, n_tiles);
+// the variant plan_point_launch chose (the instantiations below are every variant it can choose)
+cudaError_t launch_stream(bool f64, int mode, const Params& P, const Plan& pl, int dev, cudaStream_t st) {
+    return dispatch_layout_mode(f64, mode, [&](auto f64_c, auto mode_c) -> cudaError_t {
+        constexpr bool F64 = decltype(f64_c)::value;
+        constexpr int MODE = decltype(mode_c)::value;
+        if constexpr (MODE != kQuantOnly) {
+            switch (pl.ex) {
+            case kExOut:           return launch_stream_ex<F64, MODE, kExOut>(P, pl, dev, st);
+            case kExOut | kExLvx:  return launch_stream_ex<F64, MODE, kExOut | kExLvx>(P, pl, dev, st);
+            case kExOut | kExLas:  return launch_stream_ex<F64, MODE, kExOut | kExLas>(P, pl, dev, st);
             }
-            if (mask == (kExOut | kExLvx) && !lvx2) return launch_stream_ex<F64, MODE, kExOut | kExLvx>(P, st, grid, tile0, n_tiles);
-            if (mask == (kExOut | kExLas)) return launch_stream_ex<F64, MODE, kExOut | kExLas>(P, st, grid, tile0, n_tiles);
+            if constexpr (MODE == kGyro) {
+                if (pl.ex == (kExOut | kExLvx | kExLvx2)) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExLvx2>(P, pl, dev, st);
+            } else if constexpr (!F64) {
+                if (pl.ex == (kExOut | kExLvx | kExMc)) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExMc>(P, pl, dev, st);
+                if (pl.ex == (kExOut | kExLvx | kExPb)) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExPb>(P, pl, dev, st);
+            }
         }
-    }
-    return launch_stream_ex<F64, MODE, kExGeneric>(P, st, grid, tile0, n_tiles);
-}
-
-cudaError_t launch_tma(bool f64, int mode, const Params& P, cudaStream_t st, bool force, bool* handled) {
-    *handled = false;
-    if (P.p_end <= P.p_begin) { *handled = true; return cudaSuccess; }
-    switch (mode) {
-    case kRigid:     return f64 ? launch_stream<true, kRigid>(P, st, force, handled)     : launch_stream<false, kRigid>(P, st, force, handled);
-    case kGyro:      return f64 ? launch_stream<true, kGyro>(P, st, force, handled)      : launch_stream<false, kGyro>(P, st, force, handled);
-    case kSlerp:     return f64 ? launch_stream<true, kSlerp>(P, st, force, handled)     : launch_stream<false, kSlerp>(P, st, force, handled);
-    case kQuantOnly: return f64 ? launch_stream<true, kQuantOnly>(P, st, force, handled) : launch_stream<false, kQuantOnly>(P, st, force, handled);
-    }
-    return cudaErrorInvalidValue;
+        if (pl.ex == kExGeneric) return launch_stream_ex<F64, MODE, kExGeneric>(P, pl, dev, st);
+        return cudaErrorInvalidValue;
+    });
 }
 
 }  // namespace lmc

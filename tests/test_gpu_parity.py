@@ -1216,6 +1216,23 @@ def test_lean_lvx_bulk_store_epilogue_with_ragged_shards(mode, f64):
         C.set_path(C.PATH_AUTO)
 
 
+def test_multicast_without_a_multicast_kernel_is_an_argument_error():
+    """Multicast merge exists for f32 Mode A / C only: the same pointers on an f64 Mode C call are refused as a bad argument
+    (ERR_INVALID, not a CUDA error) and nothing runs.  The peer and multicast pointers point into this call's own buffers."""
+    F, P = 8, 500
+    st = synth.make_stream(F, P, 3, device=DEV, dtype=torch.float64)
+    ts = dev(st.frame_start[np.repeat(np.arange(F), P)] + st.ts_off.cpu().numpy().astype(np.int64))
+    out = torch.zeros_like(st.pts)
+    lvx = torch.zeros((st.n_points, 14), dtype=torch.uint8, device=DEV)
+    spec = ops.ExportSpec(lvx=True, into=ops.ExportBuffers(lvx14=lvx), peer_out=[out.data_ptr()], peer_lvx14=[lvx.data_ptr()],
+                          mc_out=out.data_ptr(), mc_lvx14=lvx.data_ptr())
+    with pytest.raises(C.LmcError) as e:
+        ops.deskew_slerp(st.pts, ts, dev(st.frame_off), dev(st.frame_start), dev(st.sample_ts), dev(st.seg), out=out, export=spec)
+    assert e.value.code == C.ERR_INVALID
+    torch.cuda.synchronize()
+    assert not out.any() and not lvx.any()
+
+
 # ------------------------------------------------------------------------------------------
 # full-size stream: size-independent properties + spot checks against the oracle
 # ------------------------------------------------------------------------------------------
