@@ -293,32 +293,40 @@ __device__ __forceinline__ void slerp_apply(const double (&s)[kSegStride], doubl
 
 // ------------------------------------------------------------------------------------------
 // Quantisers.  cvt.rzi.s32.f64 saturates, which IS np.clip to the int32 range followed by
-// truncation, so the clip costs nothing; NaN (where the reference raises) sets a status bit.
+// truncation, so the clip costs nothing; NaN (where the reference raises) sets a status bit and
+// quantises to 0, as in the oracle.  The conversion alone does not give 0 for NaN on sm_100
+// (a NaN coordinate or intensity left a non-zero record field), so the 0 is selected explicitly.
 // The NaN test is made on the INPUT value (v*1000 is NaN iff v is): testing the product instead
 // made ptxas keep -- and spill -- every product until a deferred compare.
 // ------------------------------------------------------------------------------------------
+// ZERO_NAN = false leaves the NaN fields to the caller, which zeroes them off its hot path (the lean streaming epilogue:
+// one test per point pair instead of a select per field)
 // (a4) LMC:257-259   int(np.clip(v * 1000, -2147483648, 2147483647))
+template <bool ZERO_NAN = true>
 __device__ __forceinline__ int32_t q_mm_clip(double v, uint32_t& fl) {
     if (v != v) fl |= LMC_FLAG_NAN;
-    return __double2int_rz(__dmul_rn(v, 1000.0));   // NaN -> 0, +-big -> INT_MAX / INT_MIN
+    const int32_t q = __double2int_rz(__dmul_rn(v, 1000.0));   // +-big -> INT_MAX / INT_MIN
+    return ZERO_NAN && v != v ? 0 : q;
 }
 // (a4) LMC:266       int(np.clip(i * 255, 0, 255))
+template <bool ZERO_NAN = true>
 __device__ __forceinline__ uint32_t q_refl(double w, uint32_t& fl) {
     if (w != w) fl |= LMC_FLAG_NAN;
-    return min(__double2uint_rz(__dmul_rn(w, 255.0)), 255u);   // negative -> 0 (saturating), NaN -> 0
+    const uint32_t r = min(__double2uint_rz(__dmul_rn(w, 255.0)), 255u);   // negative -> 0 (saturating)
+    return ZERO_NAN && w != w ? 0u : r;
 }
 // (a9) CS:368-370    int(v * 1000)  -- no clip; '<iii' packing raises outside int32
 __device__ __forceinline__ int32_t q_mm_noclip(double v, uint32_t& fl) {
     const double m = __dmul_rn(v, 1000.0);
     if (v != v) fl |= LMC_FLAG_NAN;
     if (m >= 2147483648.0 || m <= -2147483649.0) fl |= LMC_FLAG_OVERFLOW;
-    return __double2int_rz(m);
+    return v != v ? 0 : __double2int_rz(m);
 }
 // (a9) CS:373        struct.pack('<B', point.intensity)
 __device__ __forceinline__ uint32_t q_u8_copy(double w, uint32_t& fl) {
     if (w != w) fl |= LMC_FLAG_NAN;
     if (w < 0.0 || w > 255.0) fl |= LMC_FLAG_OVERFLOW;
-    return min(__double2uint_rz(w), 255u);
+    return w != w ? 0u : min(__double2uint_rz(w), 255u);
 }
 // (a5)/(a10) laspy: np.round((v - offset) / scale) -> int32   (parity unpinned, see header).
 // The quotient is formed with the host-rounded reciprocal and two Markstein corrections
@@ -335,7 +343,7 @@ __device__ __forceinline__ int2 q_las_exact_body(double v, double scale, double 
     }
     if (v != v) fl |= LMC_FLAG_NAN;
     if (q >= 2147483647.5 || q < -2147483648.5) fl |= LMC_FLAG_OVERFLOW;
-    return make_int2(__double2int_rn(q), (int)fl);  // round-half-even, saturates
+    return make_int2(v != v ? 0 : __double2int_rn(q), (int)fl);  // round-half-even, saturates
 }
 static __device__ __noinline__ int2 q_las_exact(double v, double scale, double rcp, double off) { return q_las_exact_body(v, scale, rcp, off); }
 // OOL: the exact route as a call (Mode A + LAS: +1.6 %) or inline (Mode C + LAS, which is register-starved: the call's register
@@ -360,7 +368,7 @@ __device__ __forceinline__ uint32_t q_las_intensity(double w, int mode, uint32_t
     const double m = mode == LMC_LAS_INTENSITY_UNIT ? __dmul_rn(w, 65535.0) : w;
     if (w != w) fl |= LMC_FLAG_NAN;
     if (m >= 9.2e18 || m <= -9.2e18) { fl |= LMC_FLAG_OVERFLOW; return 0; }
-    return (uint32_t)(__double2ll_rz(m) & 0xffff);
+    return w != w ? 0u : (uint32_t)(__double2ll_rz(m) & 0xffff);
 }
 
 // ------------------------------------------------------------------------------------------

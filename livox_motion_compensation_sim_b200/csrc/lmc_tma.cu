@@ -187,13 +187,23 @@ __device__ __forceinline__ void consume_tile(const Params& P, const TileInfo& ti
             // lean: the LVX record is LMC:252-272 on the RAW input point -- independent of the transform,
             // so pack it first and let its temporaries die before the FP64-heavy part
             if (do_lvx) {
-                uint32_t x[2] = {0, 0}, y[2] = {0, 0}, z[2] = {0, 0}, rt[2] = {0, 0};
+                uint32_t x[2] = {0, 0}, y[2] = {0, 0}, z[2] = {0, 0}, rt[2] = {0, 0}, nan = 0;
 #pragma unroll
                 for (int h = 0; h < 2; ++h)
                     if (FULL || (h == 0 ? va : vb)) {
-                        x[h] = (uint32_t)q_mm_clip(in[h].x, fl); y[h] = (uint32_t)q_mm_clip(in[h].y, fl); z[h] = (uint32_t)q_mm_clip(in[h].z, fl);
-                        rt[h] = q_refl(in[h].w, fl);
+                        x[h] = (uint32_t)q_mm_clip<false>(in[h].x, nan); y[h] = (uint32_t)q_mm_clip<false>(in[h].y, nan);
+                        z[h] = (uint32_t)q_mm_clip<false>(in[h].z, nan); rt[h] = q_refl<false>(in[h].w, nan);
                     }
+                if (nan) {                                       // rare: a NaN field quantises to 0
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        if (in[h].x != in[h].x) x[h] = 0;
+                        if (in[h].y != in[h].y) y[h] = 0;
+                        if (in[h].z != in[h].z) z[h] = 0;
+                        if (in[h].w != in[h].w) rt[h] = 0;
+                    }
+                    fl |= nan;
+                }
                 lvx_pair_words(reinterpret_cast<uint32_t*>(slab) + 7 * (j * 32 + lane), x, y, z, rt);
             }
         }
