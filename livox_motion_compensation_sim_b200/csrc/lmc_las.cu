@@ -157,8 +157,9 @@ __global__ void k_las_header(const __grid_constant__ LasParams L) {
             put_le(h + 131 + 8 * c, (uint64_t)__double_as_longlong(L.scale[c]), 8);
             put_le(h + 155 + 8 * c, (uint64_t)__double_as_longlong(L.off[c]), 8);
             const bool any = L.n > 0;
-            const double vmax = any ? __fma_rn((double)L.minmax[2 * c + 1], L.scale[c], L.off[c]) : 0.0;   // X * scale + offset
-            const double vmin = any ? __fma_rn((double)L.minmax[2 * c], L.scale[c], L.off[c]) : 0.0;
+            // X * scale + offset as NumPy evaluates it: a rounded product, then a rounded sum (an fma differs in the last bit)
+            const double vmax = any ? __dadd_rn(__dmul_rn((double)L.minmax[2 * c + 1], L.scale[c]), L.off[c]) : 0.0;
+            const double vmin = any ? __dadd_rn(__dmul_rn((double)L.minmax[2 * c], L.scale[c]), L.off[c]) : 0.0;
             put_le(h + 179 + 16 * c, (uint64_t)__double_as_longlong(vmax), 8);
             put_le(h + 187 + 16 * c, (uint64_t)__double_as_longlong(vmin), 8);
         }

@@ -322,6 +322,9 @@ def las_pf3_records(pts: torch.Tensor, p_begin: int, p_end: int, file_pos0: int,
     sc = (C.ctypes.c_double * 3)(*[float(v) for v in scale])
     of = (C.ctypes.c_double * 3)(*[float(v) for v in offset])
     fn = C.lib().lmc_las_pf3_records_f64 if f64 else C.lib().lmc_las_pf3_records_f32
+    if size == 0:                                           # an empty shard: no bytes (its buffer has no address), neutral extremes
+        mm[0::2], mm[1::2] = 2 ** 31 - 1, -2 ** 31
+        return out, mm, status
     C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(gps_time, torch.float64, "gps_time"), n, int(p_begin), int(p_end), sc, of,
                int(intensity_mode), out.data_ptr(), int(file_pos0), mm.data_ptr(), status.data_ptr(), _stream_ptr()))
     return out, mm, status

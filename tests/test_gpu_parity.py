@@ -1050,7 +1050,8 @@ def test_las_pf3_file_image():
         assert np.array_equal(rec["gps"], np.zeros(n) if g is None else g)
         mxx, mnx, mxy, mny, mxz, mnz = struct.unpack_from("<6d", b, 179)
         for mx, mn, q, s, o in [(mxx, mnx, X, scale[0], off[0]), (mxy, mny, Y, scale[1], off[1]), (mxz, mnz, Z, scale[2], off[2])]:
-            assert abs(mx - (q.max() * s + o)) <= 1e-9 and abs(mn - (q.min() * s + o)) <= 1e-9
+            # exactly NumPy's X * scale + offset (laspy's update_header): a rounded product, then a rounded sum
+            assert mx == np.float64(q.max()) * s + o and mn == np.float64(q.min()) * s + o
     # f32 rows; a view that starts one row into an allocation breaks the C-ABI's 32-byte alignment contract and is refused
     rdt = np.dtype([("X", "<i4"), ("Y", "<i4"), ("Z", "<i4"), ("I", "<u2"), ("zero6", "u1", 6), ("gps", "<f8"), ("rgb", "<u2", 3)])
     p32 = torch.from_numpy(pts.astype(np.float32)).to(DEV)
@@ -1349,7 +1350,7 @@ def test_full_size_file_images():
     h = img[:227].cpu().numpy().tobytes()
     mx, mn = struct.unpack_from("<6d", h, 179)[0::2], struct.unpack_from("<6d", h, 179)[1::2]
     for c, plane in enumerate((q.las_x, q.las_y, q.las_z)):
-        assert abs(mx[c] - int(plane.max()) * 0.001) <= 1e-9 and abs(mn[c] - int(plane.min()) * 0.001) <= 1e-9
+        assert mx[c] == np.float64(int(plane.max())) * 0.001 + 0.0 and mn[c] == np.float64(int(plane.min())) * 0.001 + 0.0
     assert struct.unpack_from("<I", h, 107)[0] == N
     del img, rec, xyz, q
 
