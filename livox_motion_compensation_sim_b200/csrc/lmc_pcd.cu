@@ -1,15 +1,13 @@
-// lmc_pcd.cu -- (SURVEY 8f N2) ASCII PCD point data on the device: the per-point line of
-// LiDARMotionSimulator.save_pcd (LMC:946-947)
-//     f"{x:.6f} {y:.6f} {z:.6f} {intensity:.6f}\n"
-// for every row of an (N,4) array, byte-identical to CPython's formatting (correctly rounded,
-// round-half-even on the exact binary value -- the same rule as C printf).
+// lmc_pcd.cu -- (SURVEY 8f N2) ASCII text on the device, byte-identical to CPython's "%.{d}f" (correctly rounded,
+// round-half-even on the exact binary value -- the same rule as C printf).  Two writers:
+//   k_pcd_*   the per-point line of LiDARMotionSimulator.save_pcd (LMC:946-947) for every row of an (N,4) array
+//                 f"{x:.6f} {y:.6f} {z:.6f} {intensity:.6f}\n"
+//   k_text_*  generic delimited rows, "%.{d}f" with d = 0..9 per column (the complete simulator's exports, CS:1643-1716)
 //
-// "%.6f" of a double exactly:  |v| = m * 2^e (m < 2^53)  ->  Q = round_half_even(m * 10^6 * 2^e)
-// with the 73-bit product m * 10^6 held in unsigned __int128; then Q / 10^6 and Q % 10^6 are the
-// integer and fractional digits.  Values with |v| >= 9.2e12 (Q would not fit 64 bits) are printed as
-// "inf"-free saturated text and flagged LMC_FLAG_OVERFLOW -- no point cloud coordinate gets there.
-// (The generic row writer below -- k_text_*, the complete simulator's exports CS:1643-1716 -- splits
-// integer and fraction instead and covers |v| < 2^64 with 0..9 decimals per column.)
+// Both print through one exact number core (fmtg_prepare): |v| splits into its integer part ip = trunc(|v|) (< 2^64) and
+// fq = round_half_even(frac * 10^d), all in exact FP64 steps, and emit_number prints (ip, fq) in SWAR groups of four digits.
+// The PCD writer takes the core only for its slow numbers (>= 10^4, nan, inf) and caps their magnitude at 9.2e12 (pcd_prepare);
+// every other number -- every coordinate a LiDAR produces -- takes its branch-free fast path (piece_fast).
 //
 // Lines have variable length, so the text is produced in three launches:
 //   k_pcd_len    per tile of 256 points: total text bytes of the tile.  The length of "%.6f" needs no digits: it is
@@ -18,134 +16,135 @@
 //                (kDigitT) is exact.  Four compares per number; HBM-bound.
 //   k_pcd_scan   one CTA: exclusive prefix sum of the tile sizes -> byte offset of every tile
 //   k_pcd_write  per tile: format, lay the lines out in shared memory (block scan of the line lengths) and copy the
-//                tile's contiguous byte range out as one TMA bulk store.  Numbers below 10^4 (every LiDAR coordinate)
-//                take a branch-free path: digit pairs by arithmetic, characters packed into words in registers and
-//                streamed into the image as aligned 32-bit stores (WordStream below); anything else (>= 10^4, nan,
-//                inf) goes through the general formatter byte by byte.
+//                tile's contiguous byte range out as one TMA bulk store.  Numbers below 10^4 take a branch-free path: digit
+//                pairs by arithmetic, characters packed into words in registers and streamed into the image as aligned
+//                32-bit stores (LineStream below); the slow numbers go through the number core and emit_number.
 #include <cstdlib>
 #include "lmc_device.cuh"
 
 namespace lmc {
 
 constexpr int kPcdTile    = 256;                    // points (= threads) per tile
-constexpr int kNumMax     = 1 + 13 + 1 + 6;         // sign + 13 integer digits + '.' + 6 decimals
-constexpr int kLineMax    = 4 * kNumMax + 4;        // 3 spaces + newline
 
-// One formatted number: integer part, 6 fractional digits as an integer, text length, special-value kind
-struct Num { uint64_t ip; uint32_t fq; uint32_t len; uint32_t kind; bool neg; };   // kind 0 finite, 1 nan, 2 inf
+// ---- the number core: "%.{d}f" of a double, d = 0..9 ------------------------------------------------------------------
+// One formatted number: integer part, d fractional digits as an integer, text length, special-value kind
+struct Num { uint64_t ip; uint32_t fq; uint32_t len; uint8_t kind; bool neg; };   // kind 0 finite, 1 nan, 2 inf
 
-// Exact Q = round_half_even(|v| * 1e6) through the 73-bit integer product (any magnitude below 9.2e12)
-__device__ __noinline__ uint64_t fmt_q_wide(uint64_t m, int e, uint32_t& fl) {
-    uint64_t q;
-    if (e >= 0) {                                    // integer-valued, >= 2^52: beyond the supported magnitude
-        fl |= LMC_FLAG_OVERFLOW; q = 9199999999999999999ull;
-    } else {
-        const int s = -e;
-        const unsigned __int128 P = (unsigned __int128)m * 1000000u;
-        if (s >= 127) q = 0;                         // far below half of the last place
-        else {
-            const unsigned __int128 Qw = P >> s;
-            if (Qw > (unsigned __int128)9199999999999999999ull) { fl |= LMC_FLAG_OVERFLOW; q = 9199999999999999999ull; }
-            else {
-                q = (uint64_t)Qw;
-                const unsigned __int128 rem = P - (Qw << s), half = (unsigned __int128)1 << (s - 1);
-                if (rem > half || (rem == half && (q & 1ull))) q += 1;
-            }
-        }
+__device__ __constant__ uint32_t kPow10[10] = { 1u, 10u, 100u, 1000u, 10000u, 100000u, 1000000u, 10000000u, 100000000u, 1000000000u };
+__device__ __constant__ double kPow10d[10] = { 1.0, 10.0, 100.0, 1.0e3, 1.0e4, 1.0e5, 1.0e6, 1.0e7, 1.0e8, 1.0e9 };
+
+// Digit count of the ROUNDED integer part of "%.{d}f" % a without making a digit: the printed value reaches 10^k exactly when
+// a >= 10^k - 0.5 * 10^-d (a tie there goes to the even neighbour, and 10^(k+d) is even), so the count is found by comparing with
+// kTextT[d][k] = the smallest double >= that real number (generated with exact fractions; tests/test_host.py re-derives the table).
+// Which k to compare with follows from the binary exponent: 2^e <= a < 2^(e+1) has floor(e * log10 2) + 1 or + 2 digits.
+__device__ const double kTextT[10][20] = {
+    { 0.0, 0x1.3000000000000p+3, 0x1.8e00000000000p+6, 0x1.f3c0000000000p+9, 0x1.387c000000000p+13, 0x1.869f800000000p+16, 0x1.e847f00000000p+19, 0x1.312cff0000000p+23, 0x1.7d783fe000000p+26, 0x1.dcd64ffc00000p+29, 0x1.2a05f1ffc0000p+33, 0x1.74876e7ff8000p+36, 0x1.d1a94a1fff000p+39, 0x1.2309ce53fff00p+43, 0x1.6bcc41e8fffe0p+46, 0x1.c6bf52633fffcp+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3e66666666667p+3, 0x1.8fccccccccccdp+6, 0x1.f3f999999999ap+9, 0x1.387f99999999ap+13, 0x1.869ff33333334p+16, 0x1.e847fe6666667p+19, 0x1.312cffe666667p+23, 0x1.7d783ffcccccdp+26, 0x1.dcd64fff9999ap+29, 0x1.2a05f1fff999ap+33, 0x1.74876e7fff334p+36, 0x1.d1a94a1fffe67p+39, 0x1.2309ce53fffe7p+43, 0x1.6bcc41e8ffffdp+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3fd70a3d70a3ep+3, 0x1.8ffae147ae148p+6, 0x1.f3ff5c28f5c29p+9, 0x1.387ff5c28f5c3p+13, 0x1.869ffeb851eb9p+16, 0x1.e847ffd70a3d8p+19, 0x1.312cfffd70a3ep+23, 0x1.7d783fffae148p+26, 0x1.dcd64ffff5c29p+29, 0x1.2a05f1ffff5c3p+33, 0x1.74876e7fffeb9p+36, 0x1.d1a94a1ffffd8p+39, 0x1.2309ce53ffffep+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3ffbe76c8b43ap+3, 0x1.8fff7ced91688p+6, 0x1.f3ffef9db22d1p+9, 0x1.387ffef9db22ep+13, 0x1.869fffdf3b646p+16, 0x1.e847fffbe76c9p+19, 0x1.312cffffbe76dp+23, 0x1.7d783ffff7ceep+26, 0x1.dcd64ffffef9ep+29, 0x1.2a05f1ffffefap+33, 0x1.74876e7ffffe0p+36, 0x1.d1a94a1fffffcp+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3fff972474539p+3, 0x1.8ffff2e48e8a8p+6, 0x1.f3fffe5c91d15p+9, 0x1.387fffe5c91d2p+13, 0x1.869ffffcb923bp+16, 0x1.e847ffff97248p+19, 0x1.312cfffff9725p+23, 0x1.7d783fffff2e5p+26, 0x1.dcd64fffffe5dp+29, 0x1.2a05f1fffffe6p+33, 0x1.74876e7fffffdp+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3ffff583a53b9p+3, 0x1.8ffffeb074a78p+6, 0x1.f3ffffd60e94fp+9, 0x1.387ffffd60e95p+13, 0x1.869fffffac1d3p+16, 0x1.e847fffff583bp+19, 0x1.312cffffff584p+23, 0x1.7d783fffffeb1p+26, 0x1.dcd64ffffffd7p+29, 0x1.2a05f1ffffffep+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3ffffef390860p+3, 0x1.8fffffde7210cp+6, 0x1.f3fffffbce422p+9, 0x1.387fffffbce43p+13, 0x1.869ffffff79c9p+16, 0x1.e847fffffef3ap+19, 0x1.312cffffffef4p+23, 0x1.7d783ffffffdfp+26, 0x1.dcd64fffffffcp+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3fffffe5280d7p+3, 0x1.8ffffffca501bp+6, 0x1.f3ffffff94a04p+9, 0x1.387ffffff94a1p+13, 0x1.869fffffff295p+16, 0x1.e847ffffffe53p+19, 0x1.312cfffffffe6p+23, 0x1.7d783fffffffdp+26, 0x1.dcd6500000000p+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3ffffffd50ce3p+3, 0x1.8fffffffaa19dp+6, 0x1.f3fffffff5434p+9, 0x1.387fffffff544p+13, 0x1.869fffffffea9p+16, 0x1.e847fffffffd6p+19, 0x1.312cffffffffep+23, 0x1.7d78400000000p+26, 0x1.dcd6500000000p+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+    { 0.0, 0x1.3fffffffbb47ep+3, 0x1.8ffffffff7690p+6, 0x1.f3fffffffeed2p+9, 0x1.387fffffffeeep+13, 0x1.869ffffffffdep+16, 0x1.e847ffffffffcp+19, 0x1.312d000000000p+23, 0x1.7d78400000000p+26, 0x1.dcd6500000000p+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
+};
+__device__ __forceinline__ uint32_t text_nd(double a, int d) {        // 0 <= a < 2^64
+    const int e = (int)(((uint32_t)__double2hiint(a) >> 20) & 0x7ffu) - 1023;
+    const int k0 = e > 0 ? (e * 1233) >> 12 : 0;
+    return (uint32_t)k0 + 1u + (a >= __ldg(&kTextT[d][k0 + 1]) ? 1u : 0u);
+}
+
+// q = round_half_even(fr * p10) on the exact product, for 0 <= fr < 1 and p10 = 10^d (d >= 1: at most 21 significant bits).
+// hi + lo = fr * p10 exactly (FMA error term).  RNE(hi) is the answer unless hi sits exactly on a tie k + 0.5 -- the only place
+// where lo can change the decision (k + 0.5 is itself a double and rounding is monotonic); on an exact tie (lo == 0) RNE(hi) is
+// already the even last printed digit.
+__device__ __forceinline__ uint32_t round_frac(double fr, double p10) {
+    const double hi = __dmul_rn(fr, p10);
+    uint32_t q = __double2uint_rn(hi);
+    if (fabs(__dsub_rn(hi, __uint2double_rn(q))) == 0.5) {
+        const double lo = __fma_rn(fr, p10, -hi);
+        const uint32_t dn = __double2uint_rz(hi);
+        if (lo > 0.0) q = dn + 1u; else if (lo < 0.0) q = dn;
     }
     return q;
 }
 
-// "%.6f" of v.  Fast path for |v| < 2^43 (every coordinate a LiDAR produces), all in exact FP64 steps:
-//   ip = trunc(|v|), fr = |v| - ip (exact), hi + lo = fr * 1e6 exactly (FMA error term),
-//   q = floor(hi); the tie test t = (hi - q) - 0.5 is exact whenever |t| is small, and |lo| <= ulp(hi)/2
-//   can only decide when t == 0  ->  round-half-even on the exact binary value, as printf does.
-__device__ __forceinline__ Num fmt_prepare(double v, uint32_t& fl) {
+// ip = trunc(|v|) (exact below 2^64), fr = |v| - ip (exact), q = round_frac(fr, 10^d), carried into ip when it reaches 10^d.
+// Finite |v| >= 2^64 is saturated to 2^64 - 1 and flagged LMC_FLAG_OVERFLOW.
+__device__ __forceinline__ Num fmtg_prepare(double v, int d, uint32_t& fl) {
     Num t;
     const uint64_t bits = (uint64_t)__double_as_longlong(v);
     t.neg = bits >> 63;
-    t.kind = 0;
+    t.ip = 0; t.fq = 0; t.kind = 0;
     const double a = fabs(v);
-    if (a < 8796093022208.0) {                       // 2^43
+    if (d == 0 && a < 18446744073709551616.0) {      // '%.0f': one round-to-nearest-even conversion IS the answer (a < 2^64 - 1024)
+        t.ip = __double2ull_rn(a);
+        t.len = (t.neg ? 1u : 0u) + text_nd(a, 0);
+        return t;
+    }
+    if (a < 18446744073709551616.0) {                // 2^64
         uint64_t ip = __double2ull_rz(a);
         const double fr = __dsub_rn(a, __ull2double_rn(ip));
-        const double hi = __dmul_rn(fr, 1.0e6), lo = __fma_rn(fr, 1.0e6, -hi);
-        uint32_t q = __double2uint_rz(hi);
-        const double d = __dsub_rn(__dsub_rn(hi, __uint2double_rn(q)), 0.5);
-        if (d > 0.0 || (d == 0.0 && (lo > 0.0 || (lo == 0.0 && (q & 1u))))) q += 1;
-        if (q == 1000000u) { q = 0; ip += 1; }
+        uint32_t q = round_frac(fr, kPow10d[d]);
+        if (q >= kPow10[d]) { q -= kPow10[d]; ip += 1; }
         t.ip = ip; t.fq = q;
+        t.len = (t.neg ? 1u : 0u) + text_nd(a, d) + (d ? 1u + (uint32_t)d : 0u);
+        return t;
+    } else if (a != a) {
+        t.kind = 1; t.len = 3u; return t;
+    } else if (isinf(a)) {
+        t.kind = 2; t.len = t.neg ? 4u : 3u; return t;
     } else {
-        const uint32_t ex = (uint32_t)(bits >> 52) & 0x7ffu;
-        const uint64_t frac = bits & 0xfffffffffffffull;
-        t.ip = 0; t.fq = 0;
-        if (ex == 0x7ff) { t.kind = frac ? 1u : 2u; t.len = frac ? 3u : (t.neg ? 4u : 3u); return t; }   // "nan" | "inf" / "-inf"
-        const uint64_t Q = fmt_q_wide(frac | (1ull << 52), (int)ex - 1075, fl);
-        t.ip = Q / 1000000ull; t.fq = (uint32_t)(Q - t.ip * 1000000ull);
+        fl |= LMC_FLAG_OVERFLOW; t.ip = 0xffffffffffffffffull;
     }
-    uint32_t nd;
-    if (t.ip < 1000000ull) {
-        const uint32_t x = (uint32_t)t.ip;
-        nd = 1u + (x >= 10u) + (x >= 100u) + (x >= 1000u) + (x >= 10000u) + (x >= 100000u);
-    } else {
-        nd = 7;
-        for (uint64_t x = t.ip / 1000000ull; x >= 10; x /= 10) ++nd;
-    }
-    t.len = (t.neg ? 1u : 0u) + nd + 7u;
+    t.len = (t.neg ? 1u : 0u) + 20u + (d ? 1u + (uint32_t)d : 0u);     // finite >= 2^64: saturated to 2^64 - 1 (20 digits), flagged
     return t;
 }
 
-__device__ __forceinline__ int fmt_write(uint8_t* dst, const Num& t) {
-    if (t.kind) {
-        int o = 0;
-        if (t.kind == 2 && t.neg) dst[o++] = '-';
-        if (t.kind == 1) { dst[o] = 'n'; dst[o + 1] = 'a'; dst[o + 2] = 'n'; }
-        else             { dst[o] = 'i'; dst[o + 1] = 'n'; dst[o + 2] = 'f'; }
-        return o + 3;
+// ---- the PCD writer's numbers ----------------------------------------------------------------------------------------
+// The PCD writer prints |v| < 9.2e12 only.  That bounds a number at 13 integer digits and a line at kLineMax = 88 bytes, which
+// sizes k_pcd_write's 44 KB tile image; with the core's full range (20 integer digits) a line would take 116 bytes and the image
+// 58 KB, and four f32 CTAs (__launch_bounds__(256, 4)) would no longer fit in an SM's shared memory.  No point cloud coordinate
+// gets near the cap: a finite |v| >= 9.2e12 prints as "9199999999999.999999" (with its sign) and sets LMC_FLAG_OVERFLOW.
+constexpr int kNumMax     = 1 + 13 + 1 + 6;         // sign + 13 integer digits + '.' + 6 decimals
+constexpr int kLineMax    = 4 * kNumMax + 4;        // 3 spaces + newline
+__device__ __forceinline__ Num pcd_prepare(double v, uint32_t& fl) {
+    const double a = fabs(v);
+    if (a >= 9.2e12 && !isinf(a)) {
+        fl |= LMC_FLAG_OVERFLOW;
+        const bool neg = __double_as_longlong(v) < 0;
+        return Num{9199999999999ull, 999999u, (neg ? 1u : 0u) + 20u, 0, neg};
     }
-    int o = (int)t.len;
-    uint32_t fp = t.fq;
-#pragma unroll
-    for (int k = 0; k < 6; ++k) { dst[--o] = (uint8_t)('0' + fp % 10u); fp /= 10u; }
-    dst[--o] = '.';
-    if (t.ip < 1000000000ull) {                      // 32-bit digit loop
-        uint32_t x = (uint32_t)t.ip;
-        do { dst[--o] = (uint8_t)('0' + x % 10u); x /= 10u; } while (x);
-    } else {
-        uint64_t x = t.ip;
-        do { dst[--o] = (uint8_t)('0' + (uint32_t)(x % 10ull)); x /= 10ull; } while (x);
-    }
-    if (t.neg) dst[--o] = '-';
-    return (int)t.len;
+    return fmtg_prepare(v, 6, fl);
 }
 
 // ---- fast path: |v| below 10^4 after rounding (at most 4 integer digits) ------------------------------------------
-// kDigitT[k-1] = the smallest double >= 10^k - 5e-7 (tests/test_host.py re-derives them with exact fractions); for a
-// float-valued |v| the same thresholds are 10, 100, 1000, 10000 (the float just below 10^k prints 9...9.99....).
+// kDigitT[k-1] = the smallest double >= 10^k - 5e-7 (= kTextT[6][k]); for a float-valued |v| the same thresholds are
+// 10, 100, 1000, 10000 (the float just below 10^k prints 9...9.99....).
 __device__ __constant__ double kDigitT[4] = { 0x1.3ffffef390860p+3, 0x1.8fffffde7210cp+6, 0x1.f3fffffbce422p+9, 0x1.387fffffbce43p+13 };
 
 // (slow-path helpers return by value: a reference to the caller's flag word or arrays would pin them in local memory)
-__device__ __noinline__ uint2 fmt_len_slow_eval(double v) { uint32_t fl = 0; const uint32_t len = fmt_prepare(v, fl).len; return make_uint2(len, fl); }
-__device__ __forceinline__ uint32_t fmt_len_slow(double v, uint32_t& fl) { const uint2 r = fmt_len_slow_eval(v); fl |= r.y; return r.x; }
-__device__ __noinline__ int fmt_write_slow(uint8_t* dst, double v, uint32_t& fl) { const Num t = fmt_prepare(v, fl); return fmt_write(dst, t); }
+__device__ __noinline__ uint2 pcd_len_slow_eval(double v) { uint32_t fl = 0; const uint32_t len = pcd_prepare(v, fl).len; return make_uint2(len, fl); }
+__device__ __forceinline__ uint32_t pcd_len_slow(double v, uint32_t& fl) { const uint2 r = pcd_len_slow_eval(v); fl |= r.y; return r.x; }
 
 // text length of "%.6f" % v, without any digit: four compares
 __device__ __forceinline__ uint32_t fmt_len(double v, uint32_t& fl) {
     const double a = fabs(v);
-    if (!(a < kDigitT[3])) return fmt_len_slow(v, fl);              // >= 10^4, inf, nan
+    if (!(a < kDigitT[3])) return pcd_len_slow(v, fl);              // >= 10^4, inf, nan
     return ((uint32_t)__double2hiint(v) >> 31) + 8u + (a >= kDigitT[0]) + (a >= kDigitT[1]) + (a >= kDigitT[2]);
 }
 __device__ __forceinline__ uint32_t fmt_len(float v, uint32_t& fl) {
     const float a = fabsf(v);
-    if (!(a < 10000.0f)) return fmt_len_slow((double)v, fl);
+    if (!(a < 10000.0f)) return pcd_len_slow((double)v, fl);
     return (__float_as_uint(v) >> 31) + 8u + (a >= 10.0f) + (a >= 100.0f) + (a >= 1000.0f);
 }
 
 // ---- rows ------------------------------------------------------------------------------------------------------------
 template <bool F64>
-__device__ __forceinline__ void load_row(const void* pts, int64_t i, double (&v)[4]) {
-    if constexpr (F64) { const double* s = reinterpret_cast<const double*>(pts) + 4 * i; ldg256(s, v[0], v[1], v[2], v[3]); }
-    else { const float4 f = __ldg(reinterpret_cast<const float4*>(pts) + i); v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w; }
+__device__ __forceinline__ double load_cell(const void* rows, int64_t idx) {
+    if constexpr (F64) return __ldg(reinterpret_cast<const double*>(rows) + idx);
+    else return (double)__ldg(reinterpret_cast<const float*>(rows) + idx);
 }
 // the row in its own type (float4 rows are formatted from the floats: no conversion, f32 compares)
 template <bool F64> struct RowT { using T = double; };
@@ -213,7 +212,7 @@ __device__ __forceinline__ uint32_t swar4(uint32_t x) {
 // One number ready for the stream: the lead (sign + integer digits, ll = 1..5 bytes) and the fixed 8-byte tail ".dddddd<sep>".
 //   T0 = [ll, d, d, d] (ll rides in byte 0, where the '.' goes),  T1 = [d, d, d, sep]
 //   ll <= 4: L0 holds the ll lead bytes;  ll == 5: "-dddd", L0 holds the four digits;
-//   ll & kPieceSlow: the general formatter prints it (|v| >= 10^4, nan, inf): L0 = text length incl. separator, T1 = the last
+//   ll & kPieceSlow: the number core prints it (|v| >= 10^4, nan, inf): L0 = text length incl. separator, T1 = the last
 //   four bytes of the text (what the next thread's first word needs)
 struct Piece { uint32_t L0, T0, T1; };
 constexpr uint32_t kPieceSlow = 0x80u;
@@ -237,7 +236,7 @@ __device__ __forceinline__ void piece_finish(Piece& p, uint32_t ip, uint32_t q, 
 }
 __device__ __noinline__ uint3 piece_slow_eval(double v, uint32_t sepw) {     // {T1, text length incl. separator, status flags}
     uint32_t fl = 0;
-    const Num t = fmt_prepare(v, fl);
+    const Num t = pcd_prepare(v, fl);
     uint32_t t1;
     if (t.kind) t1 = (t.kind == 1 ? 0x006e616eu : 0x00666e69u) | (sepw << 24);            // "nan" / "inf" + separator
     else t1 = __byte_perm(swar4(t.fq % 10000u), sepw, 0x4321);
@@ -259,20 +258,12 @@ __device__ __forceinline__ bool piece_fast(Piece& p, float v, uint32_t sepw) {
     piece_finish(p, ip, __double2uint_rn(__dmul_rn((double)fr, 1.0e6)), __float_as_uint(v) >> 31, sepw);
     return !(a < 10000.0f);
 }
-// f64: hi + lo = fr * 10^6 exactly (FMA error term).  RNE(hi) is the answer unless hi sits exactly on a tie k + 0.5 (the only
-// place where the sign of lo can change the decision, since k + 0.5 is itself a double and rounding is monotonic)
+// f64: the core's rounding of the exact fraction (the FMA error term decides only on a tie)
 __device__ __forceinline__ bool piece_fast(Piece& p, double v, uint32_t sepw) {
     const double a = fabs(v);
     const uint32_t ip = __double2uint_rz(a);
     const double fr = __dsub_rn(a, __uint2double_rn(ip));
-    const double hi = __dmul_rn(fr, 1.0e6);
-    uint32_t q = __double2uint_rn(hi);
-    if (fabs(__dsub_rn(hi, __uint2double_rn(q))) == 0.5) {
-        const double lo = __fma_rn(fr, 1.0e6, -hi);
-        const uint32_t dn = __double2uint_rz(hi);
-        if (lo > 0.0) q = dn + 1u; else if (lo < 0.0) q = dn;
-    }
-    piece_finish(p, ip, q, (uint32_t)__double2hiint(v) >> 31, sepw);
+    piece_finish(p, ip, round_frac(fr, 1.0e6), (uint32_t)__double2hiint(v) >> 31, sepw);
     return !(a < kDigitT[3]);
 }
 __device__ __forceinline__ bool is_slow(float v) { return !(fabsf(v) < 10000.0f); }
@@ -312,6 +303,7 @@ struct LineStream {
     __device__ __forceinline__ void start(uint32_t img_s, uint32_t pos, uint32_t prev_t1) {
         addr = img_s + (pos & ~3u); sh = 8u * (pos & 3u); a0 = __funnelshift_l(prev_t1, 0u, sh);
     }
+    template <int MODE = 0>                                              // (MODE: see emit_u8; unused here)
     __device__ __forceinline__ void put(uint32_t chunk, uint32_t k) {   // the k (1..4) low bytes of chunk, the others 0
         const uint32_t w0 = a0 | (chunk << sh);
         const uint32_t hi = __funnelshift_l(chunk, 0u, sh);               // the bytes that did not fit (0 when sh == 0)
@@ -319,6 +311,12 @@ struct LineStream {
         const bool full = nsh >= 32u;
         if (full) sts(addr, w0);
         addr += full ? 4u : 0u; a0 = full ? hi : w0; sh = nsh & 31u;
+    }
+    template <int MODE = 0>
+    __device__ __forceinline__ void put4(uint32_t w) {                  // 4 bytes: one whole word leaves
+        sts(addr, a0 | (w << sh));
+        a0 = __funnelshift_l(w, 0u, sh);
+        addr += 4u;
     }
     __device__ __forceinline__ void put8(uint32_t lo, uint32_t hi) {    // 8 bytes: two whole words leave
         sts(addr, a0 | (lo << sh));
@@ -328,22 +326,102 @@ struct LineStream {
     }
     __device__ __forceinline__ void flush() { if (sh) sts(addr, a0); }   // only where no later thread completes the word
 };
+// Word stream of one row into the (zero-filled) tile image.  Rows of the generic writer are heterogeneous (any mix of column
+// widths), so the word a row shares with its predecessor is not handed over in registers as in the PCD writer: the row's FIRST
+// completed word and its last partial word are OR-ed into the image (shared-memory atomics commute), every word in between is
+// a plain store.
+struct TextStream {
+    uint32_t addr, sh, a0; bool first;
+    __device__ __forceinline__ void start(uint32_t img_s, uint32_t pos) { addr = img_s + (pos & ~3u); sh = 8u * (pos & 3u); a0 = 0u; first = true; }
+    // MODE 0: plain store; 1: OR (the word may be the one shared with the previous row); 2: decide at run time (generic formats)
+    template <int MODE>
+    __device__ __forceinline__ void out(uint32_t w) {
+        if (MODE == 1 || (MODE == 2 && first)) { asm volatile("red.shared.or.b32 [%0], %1;" :: "r"(addr), "r"(w) : "memory"); first = false; }
+        else asm volatile("st.shared.u32 [%0], %1;" :: "r"(addr), "r"(w) : "memory");
+        addr += 4u;
+    }
+    template <int MODE>
+    __device__ __forceinline__ void put(uint32_t chunk, uint32_t k) {   // the k (1..4) low bytes of chunk, the others 0
+        const uint32_t w0 = a0 | (chunk << sh);
+        const uint32_t hi = __funnelshift_l(chunk, 0u, sh);
+        const uint32_t nsh = sh + 8u * k;
+        if (nsh >= 32u) { out<MODE>(w0); a0 = hi; } else a0 = w0;
+        sh = nsh & 31u;
+    }
+    template <int MODE>
+    __device__ __forceinline__ void put4(uint32_t w) { out<MODE>(a0 | (w << sh)); a0 = __funnelshift_l(w, 0u, sh); }
+    __device__ __forceinline__ void finish() { if (sh) asm volatile("red.shared.or.b32 [%0], %1;" :: "r"(addr), "r"(a0) : "memory"); }
+};
+// The digit emitters write into either word stream: MODE is TextStream's store mode, a LineStream stores every word plainly.
+// x < 10^8 printed with nd (1..8) digits / with all 8 digits
+template <int MODE, class Stream>
+__device__ __forceinline__ void emit_u8(Stream& ts, uint32_t x, uint32_t nd) {
+    if (nd > 4u) {
+        const uint32_t h = (uint32_t)(((uint64_t)x * 3518437209ull) >> 45);       // x / 10^4, exact for 32-bit x
+        ts.template put<MODE>(swar4(h) >> (8u * (8u - nd)), nd - 4u);
+        ts.template put4<MODE>(swar4(x - h * 10000u));
+    } else ts.template put<MODE>(swar4(x) >> (8u * (4u - nd)), nd);
+}
+template <int MODE, class Stream>
+__device__ __forceinline__ void emit_u8_full(Stream& ts, uint32_t x) {
+    const uint32_t h = (uint32_t)(((uint64_t)x * 3518437209ull) >> 45);
+    ts.template put4<MODE>(swar4(h));
+    ts.template put4<MODE>(swar4(x - h * 10000u));
+}
+// one number + separator: sign, integer digits in groups of four (SWAR), fraction, separator
+template <int MODE, class Stream>
+__device__ __forceinline__ void emit_number(Stream& ts, const Num& t, int d, uint32_t sep) {
+    if (t.kind) {                                                      // "nan" | "inf" | "-inf"
+        if (t.kind == 2 && t.neg) ts.template put<MODE>(0x2du, 1u);
+        ts.template put<MODE>(t.kind == 1 ? 0x006e616eu : 0x00666e69u, 3u);
+        ts.template put<MODE>(sep, 1u);
+        return;
+    }
+    if (t.neg) ts.template put<MODE>(0x2du, 1u);
+    const uint32_t nd = t.len - (t.neg ? 1u : 0u) - (d ? 1u + (uint32_t)d : 0u);
+    if (t.ip < 100000000ull) emit_u8<MODE>(ts, (uint32_t)t.ip, nd);
+    else if (t.ip < 10000000000000000ull) {
+        const uint64_t h = t.ip / 100000000ull;
+        emit_u8<MODE>(ts, (uint32_t)h, nd - 8u);
+        emit_u8_full<MODE>(ts, (uint32_t)(t.ip - h * 100000000ull));
+    } else {
+        const uint64_t h = t.ip / 10000000000000000ull, r = t.ip - h * 10000000000000000ull, m = r / 100000000ull;
+        emit_u8<MODE>(ts, (uint32_t)h, nd - 16u);
+        emit_u8_full<MODE>(ts, (uint32_t)m);
+        emit_u8_full<MODE>(ts, (uint32_t)(r - m * 100000000ull));
+    }
+    if (d) {
+        // the d fraction digits = the last d characters of the 9-digit zero-padded fq
+        const uint32_t top = t.fq / 100000000u, r8 = t.fq - top * 100000000u;
+        const uint32_t h = (uint32_t)(((uint64_t)r8 * 3518437209ull) >> 45);
+        const uint64_t ab = (uint64_t)swar4(h) | ((uint64_t)swar4(r8 - h * 10000u) << 32);      // 8 digits, most significant in byte 0
+        if (d == 6) {                                                  // ".dddddd<sep>": two whole words
+            const uint64_t x = ab >> 16;
+            ts.template put4<MODE>(0x2eu | ((uint32_t)x << 8));
+            ts.template put4<MODE>(((uint32_t)x >> 24) | ((uint32_t)(x >> 32) << 8) | (sep << 24));
+            return;
+        }
+        ts.template put<MODE>(0x2eu, 1u);
+        if (d == 9) ts.template put<MODE>(0x30u + top, 1u);
+        const uint32_t dd = d == 9 ? 8u : (uint32_t)d;
+        const uint64_t x = ab >> (8u * (8u - dd));
+        if (dd > 4u) { ts.template put4<MODE>((uint32_t)x); ts.template put<MODE>((uint32_t)(x >> 32), dd - 4u); }
+        else ts.template put<MODE>((uint32_t)x, dd);
+    }
+    ts.template put<MODE>(sep, 1u);
+}
+
 template <bool F64>
 __device__ __noinline__ uint3 stream_slow(uint32_t addr, uint32_t sh, uint32_t a0, const void* pts, int64_t row, int c, uint32_t sep) {
     LineStream ws{addr, sh, a0};
-    double v[4];
-    load_row<F64>(pts, row, v);                                          // (re-read: nothing of a slow number is kept in registers)
-    uint8_t tmp[kNumMax + 3];
-    uint32_t fl = 0;
-    const int len = fmt_write_slow(tmp, v[c], fl);
-    for (int k = 0; k < len; ++k) ws.put(tmp[k], 1u);
-    ws.put(sep, 1u);
+    uint32_t fl = 0;                                                     // (piece_slow has flagged it already)
+    emit_number<0>(ws, pcd_prepare(load_cell<F64>(pts, 4 * row + c), fl), 6, sep);   // (re-read: nothing of a slow number is kept in registers)
     return make_uint3(ws.addr, ws.sh, ws.a0);
 }
 template <bool F64>
 __device__ __forceinline__ void stream_piece(LineStream& ws, const Piece& p, const void* pts, int64_t row, int c, uint32_t sep) {
     const uint32_t ll = piece_ll(p);
-    if (ll > 4u) {                                                       // rare: "-dddd" or the general formatter
+    if (ll > 4u) {                                                       // rare: "-dddd" or the number core
         if (ll & kPieceSlow) { const uint3 r = stream_slow<F64>(ws.addr, ws.sh, ws.a0, pts, row, c, sep); ws.addr = r.x; ws.sh = r.y; ws.a0 = r.z; return; }
         ws.put(0x2du, 1u); ws.put(p.L0, 4u);
     } else ws.put(p.L0, ll);
@@ -529,97 +607,18 @@ __global__ void __launch_bounds__(256) k_pcd_row_off(const void* __restrict__ pt
 }
 
 // ---- generic delimited text rows: CS:1643-1716 (_export_pcd '%.6f %.6f %.6f %.0f %.0f', _export_xyz, _export_csv) ----
-// "%.{d}f" with d = 0..9 per column and the full integer range a timestamp column needs (ns since the
-// epoch ~ 1.7e18): the value is split exactly into its integer part I (< 2^64) and the fraction
-// Q = round_half_even(frac * 10^d) (carry into I when Q reaches 10^d), all in exact FP64 steps.
+// "%.{d}f" with d = 0..9 per column and the full integer range a timestamp column needs (ns since the epoch ~ 1.7e18):
+// every number through the core's fmtg_prepare, except the compiled formats' fast '%.6f' numbers (piece_fast).
 constexpr int kTextCols   = 6;                      // LMC_TEXT_MAX_COLS
 
 struct TextFmt { int32_t n_cols, row_stride; int32_t col[kTextCols]; int32_t dec[kTextCols]; uint8_t sep; };
 
-__device__ __constant__ uint32_t kPow10[10] = { 1u, 10u, 100u, 1000u, 10000u, 100000u, 1000000u, 10000000u, 100000000u, 1000000000u };
-
-struct TextNum { uint64_t ip; uint32_t fq; uint32_t len; uint8_t kind; bool neg; };   // kind 0 finite, 1 nan, 2 inf
-
-__device__ __constant__ double kPow10d[10] = { 1.0, 10.0, 100.0, 1.0e3, 1.0e4, 1.0e5, 1.0e6, 1.0e7, 1.0e8, 1.0e9 };
-
-// Digit count of the ROUNDED integer part of "%.{d}f" % a without making a digit: the printed value reaches 10^k exactly when
-// a >= 10^k - 0.5 * 10^-d (a tie there goes to the even neighbour, and 10^(k+d) is even), so the count is found by comparing with
-// kTextT[d][k] = the smallest double >= that real number (generated with exact fractions; tests/test_host.py re-derives the table).
-// Which k to compare with follows from the binary exponent: 2^e <= a < 2^(e+1) has floor(e * log10 2) + 1 or + 2 digits.
-__device__ const double kTextT[10][20] = {
-    { 0.0, 0x1.3000000000000p+3, 0x1.8e00000000000p+6, 0x1.f3c0000000000p+9, 0x1.387c000000000p+13, 0x1.869f800000000p+16, 0x1.e847f00000000p+19, 0x1.312cff0000000p+23, 0x1.7d783fe000000p+26, 0x1.dcd64ffc00000p+29, 0x1.2a05f1ffc0000p+33, 0x1.74876e7ff8000p+36, 0x1.d1a94a1fff000p+39, 0x1.2309ce53fff00p+43, 0x1.6bcc41e8fffe0p+46, 0x1.c6bf52633fffcp+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3e66666666667p+3, 0x1.8fccccccccccdp+6, 0x1.f3f999999999ap+9, 0x1.387f99999999ap+13, 0x1.869ff33333334p+16, 0x1.e847fe6666667p+19, 0x1.312cffe666667p+23, 0x1.7d783ffcccccdp+26, 0x1.dcd64fff9999ap+29, 0x1.2a05f1fff999ap+33, 0x1.74876e7fff334p+36, 0x1.d1a94a1fffe67p+39, 0x1.2309ce53fffe7p+43, 0x1.6bcc41e8ffffdp+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3fd70a3d70a3ep+3, 0x1.8ffae147ae148p+6, 0x1.f3ff5c28f5c29p+9, 0x1.387ff5c28f5c3p+13, 0x1.869ffeb851eb9p+16, 0x1.e847ffd70a3d8p+19, 0x1.312cfffd70a3ep+23, 0x1.7d783fffae148p+26, 0x1.dcd64ffff5c29p+29, 0x1.2a05f1ffff5c3p+33, 0x1.74876e7fffeb9p+36, 0x1.d1a94a1ffffd8p+39, 0x1.2309ce53ffffep+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3ffbe76c8b43ap+3, 0x1.8fff7ced91688p+6, 0x1.f3ffef9db22d1p+9, 0x1.387ffef9db22ep+13, 0x1.869fffdf3b646p+16, 0x1.e847fffbe76c9p+19, 0x1.312cffffbe76dp+23, 0x1.7d783ffff7ceep+26, 0x1.dcd64ffffef9ep+29, 0x1.2a05f1ffffefap+33, 0x1.74876e7ffffe0p+36, 0x1.d1a94a1fffffcp+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3fff972474539p+3, 0x1.8ffff2e48e8a8p+6, 0x1.f3fffe5c91d15p+9, 0x1.387fffe5c91d2p+13, 0x1.869ffffcb923bp+16, 0x1.e847ffff97248p+19, 0x1.312cfffff9725p+23, 0x1.7d783fffff2e5p+26, 0x1.dcd64fffffe5dp+29, 0x1.2a05f1fffffe6p+33, 0x1.74876e7fffffdp+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3ffff583a53b9p+3, 0x1.8ffffeb074a78p+6, 0x1.f3ffffd60e94fp+9, 0x1.387ffffd60e95p+13, 0x1.869fffffac1d3p+16, 0x1.e847fffff583bp+19, 0x1.312cffffff584p+23, 0x1.7d783fffffeb1p+26, 0x1.dcd64ffffffd7p+29, 0x1.2a05f1ffffffep+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3ffffef390860p+3, 0x1.8fffffde7210cp+6, 0x1.f3fffffbce422p+9, 0x1.387fffffbce43p+13, 0x1.869ffffff79c9p+16, 0x1.e847fffffef3ap+19, 0x1.312cffffffef4p+23, 0x1.7d783ffffffdfp+26, 0x1.dcd64fffffffcp+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3fffffe5280d7p+3, 0x1.8ffffffca501bp+6, 0x1.f3ffffff94a04p+9, 0x1.387ffffff94a1p+13, 0x1.869fffffff295p+16, 0x1.e847ffffffe53p+19, 0x1.312cfffffffe6p+23, 0x1.7d783fffffffdp+26, 0x1.dcd6500000000p+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3ffffffd50ce3p+3, 0x1.8fffffffaa19dp+6, 0x1.f3fffffff5434p+9, 0x1.387fffffff544p+13, 0x1.869fffffffea9p+16, 0x1.e847fffffffd6p+19, 0x1.312cffffffffep+23, 0x1.7d78400000000p+26, 0x1.dcd6500000000p+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-    { 0.0, 0x1.3fffffffbb47ep+3, 0x1.8ffffffff7690p+6, 0x1.f3fffffffeed2p+9, 0x1.387fffffffeeep+13, 0x1.869ffffffffdep+16, 0x1.e847ffffffffcp+19, 0x1.312d000000000p+23, 0x1.7d78400000000p+26, 0x1.dcd6500000000p+29, 0x1.2a05f20000000p+33, 0x1.74876e8000000p+36, 0x1.d1a94a2000000p+39, 0x1.2309ce5400000p+43, 0x1.6bcc41e900000p+46, 0x1.c6bf526340000p+49, 0x1.1c37937e08000p+53, 0x1.6345785d8a000p+56, 0x1.bc16d674ec800p+59, 0x1.158e460913d00p+63 },
-};
-__device__ __forceinline__ uint32_t text_nd(double a, int d) {        // 0 <= a < 2^64
-    const int e = (int)(((uint32_t)__double2hiint(a) >> 20) & 0x7ffu) - 1023;
-    const int k0 = e > 0 ? (e * 1233) >> 12 : 0;
-    return (uint32_t)k0 + 1u + (a >= __ldg(&kTextT[d][k0 + 1]) ? 1u : 0u);
-}
-
-// Same exact-FP64 scheme as fmt_prepare: ip = trunc(|v|) (exact below 2^64), fr = |v| - ip (exact),
-// hi + lo = fr * 10^d exactly (10^d has <= 21 significant bits), q = floor(hi), tie test on (hi - q) - 0.5
-// with lo as the tie breaker; ties go to the even last printed digit (ip's when d == 0).
-__device__ __forceinline__ TextNum fmtg_prepare(double v, int d, uint32_t& fl) {
-    TextNum t;
-    const uint64_t bits = (uint64_t)__double_as_longlong(v);
-    t.neg = bits >> 63;
-    t.ip = 0; t.fq = 0; t.kind = 0;
-    const double a = fabs(v);
-    if (d == 0 && a < 18446744073709551616.0) {      // '%.0f': one round-to-nearest-even conversion IS the answer (a < 2^64 - 1024)
-        t.ip = __double2ull_rn(a);
-        t.len = (t.neg ? 1u : 0u) + text_nd(a, 0);
-        return t;
-    }
-    if (a < 18446744073709551616.0) {                // 2^64
-        uint64_t ip = __double2ull_rz(a);
-        const double fr = __dsub_rn(a, __ull2double_rn(ip));
-        const double p10 = kPow10d[d];
-        const double hi = __dmul_rn(fr, p10);
-        // RNE(hi) is the answer unless hi sits exactly on a tie k + 0.5 -- the only place where the FMA error term lo = fr * 10^d - hi
-        // can change the decision (k + 0.5 is itself a double and rounding is monotonic); an exact tie goes to the even last
-        // printed digit (ip's when d == 0)
-        uint32_t q = __double2uint_rn(hi);
-        if (fabs(__dsub_rn(hi, __uint2double_rn(q))) == 0.5) {
-            const double lo = __fma_rn(fr, p10, -hi);
-            const uint32_t dn = __double2uint_rz(hi);
-            if (lo > 0.0) q = dn + 1u;
-            else if (lo < 0.0) q = dn;
-            else q = dn + ((d ? (dn & 1u) : (uint32_t)(ip & 1ull)) ? 1u : 0u);
-        }
-        if (q >= kPow10[d]) { q -= kPow10[d]; ip += 1; }
-        t.ip = ip; t.fq = q;
-        t.len = (t.neg ? 1u : 0u) + text_nd(a, d) + (d ? 1u + (uint32_t)d : 0u);
-        return t;
-    } else if (a != a) {
-        t.kind = 1; t.len = 3u; return t;
-    } else if (isinf(a)) {
-        t.kind = 2; t.len = t.neg ? 4u : 3u; return t;
-    } else {
-        fl |= LMC_FLAG_OVERFLOW; t.ip = 0xffffffffffffffffull;
-    }
-    t.len = (t.neg ? 1u : 0u) + 20u + (d ? 1u + (uint32_t)d : 0u);     // finite >= 2^64: saturated to 2^64 - 1 (20 digits), flagged
-    return t;
-}
 // text length of "%.{d}f" % v: no digits, one table compare
 __device__ __noinline__ uint2 text_len_slow_eval(double v, int d) { uint32_t fl = 0; const uint32_t len = fmtg_prepare(v, d, fl).len; return make_uint2(len, fl); }
 __device__ __forceinline__ uint32_t text_len(double v, int d, uint32_t& fl) {
     const double a = fabs(v);
     if (!(a < 18446744073709551616.0)) { const uint2 r = text_len_slow_eval(v, d); fl |= r.y; return r.x; }     // nan, inf, >= 2^64
     return ((uint32_t)__double2hiint(v) >> 31) + text_nd(a, d) + (d ? 1u + (uint32_t)d : 0u);
-}
-
-template <bool F64>
-__device__ __forceinline__ double load_cell(const void* rows, int64_t idx) {
-    if constexpr (F64) return __ldg(reinterpret_cast<const double*>(rows) + idx);
-    else return (double)__ldg(reinterpret_cast<const float*>(rows) + idx);
 }
 
 // The format is a launch parameter (TextFmt), but every runtime test on it sits inside the per-number code: the three formats the
@@ -655,90 +654,6 @@ __global__ void __launch_bounds__(kPcdTile) k_text_len(const void* __restrict__ 
     }
 }
 
-// Word stream of one row into the (zero-filled) tile image.  Rows of the generic writer are heterogeneous (any mix of column
-// widths), so the word a row shares with its predecessor is not handed over in registers as in the PCD writer: the row's FIRST
-// completed word and its last partial word are OR-ed into the image (shared-memory atomics commute), every word in between is
-// a plain store.
-struct TextStream {
-    uint32_t addr, sh, a0; bool first;
-    __device__ __forceinline__ void start(uint32_t img_s, uint32_t pos) { addr = img_s + (pos & ~3u); sh = 8u * (pos & 3u); a0 = 0u; first = true; }
-    // MODE 0: plain store; 1: OR (the word may be the one shared with the previous row); 2: decide at run time (generic formats)
-    template <int MODE>
-    __device__ __forceinline__ void out(uint32_t w) {
-        if (MODE == 1 || (MODE == 2 && first)) { asm volatile("red.shared.or.b32 [%0], %1;" :: "r"(addr), "r"(w) : "memory"); first = false; }
-        else asm volatile("st.shared.u32 [%0], %1;" :: "r"(addr), "r"(w) : "memory");
-        addr += 4u;
-    }
-    template <int MODE>
-    __device__ __forceinline__ void put(uint32_t chunk, uint32_t k) {   // the k (1..4) low bytes of chunk, the others 0
-        const uint32_t w0 = a0 | (chunk << sh);
-        const uint32_t hi = __funnelshift_l(chunk, 0u, sh);
-        const uint32_t nsh = sh + 8u * k;
-        if (nsh >= 32u) { out<MODE>(w0); a0 = hi; } else a0 = w0;
-        sh = nsh & 31u;
-    }
-    template <int MODE>
-    __device__ __forceinline__ void put4(uint32_t w) { out<MODE>(a0 | (w << sh)); a0 = __funnelshift_l(w, 0u, sh); }
-    __device__ __forceinline__ void finish() { if (sh) asm volatile("red.shared.or.b32 [%0], %1;" :: "r"(addr), "r"(a0) : "memory"); }
-};
-// x < 10^8 printed with nd (1..8) digits / with all 8 digits
-template <int MODE>
-__device__ __forceinline__ void emit_u8(TextStream& ts, uint32_t x, uint32_t nd) {
-    if (nd > 4u) {
-        const uint32_t h = (uint32_t)(((uint64_t)x * 3518437209ull) >> 45);       // x / 10^4, exact for 32-bit x
-        ts.put<MODE>(swar4(h) >> (8u * (8u - nd)), nd - 4u);
-        ts.put4<MODE>(swar4(x - h * 10000u));
-    } else ts.put<MODE>(swar4(x) >> (8u * (4u - nd)), nd);
-}
-template <int MODE>
-__device__ __forceinline__ void emit_u8_full(TextStream& ts, uint32_t x) {
-    const uint32_t h = (uint32_t)(((uint64_t)x * 3518437209ull) >> 45);
-    ts.put4<MODE>(swar4(h));
-    ts.put4<MODE>(swar4(x - h * 10000u));
-}
-// one number + separator: sign, integer digits in groups of four (SWAR), fraction, separator
-template <int MODE>
-__device__ __forceinline__ void emit_number(TextStream& ts, const TextNum& t, int d, uint32_t sep) {
-    if (t.kind) {                                                      // "nan" | "inf" | "-inf"
-        if (t.kind == 2 && t.neg) ts.put<MODE>(0x2du, 1u);
-        ts.put<MODE>(t.kind == 1 ? 0x006e616eu : 0x00666e69u, 3u);
-        ts.put<MODE>(sep, 1u);
-        return;
-    }
-    if (t.neg) ts.put<MODE>(0x2du, 1u);
-    const uint32_t nd = t.len - (t.neg ? 1u : 0u) - (d ? 1u + (uint32_t)d : 0u);
-    if (t.ip < 100000000ull) emit_u8<MODE>(ts, (uint32_t)t.ip, nd);
-    else if (t.ip < 10000000000000000ull) {
-        const uint64_t h = t.ip / 100000000ull;
-        emit_u8<MODE>(ts, (uint32_t)h, nd - 8u);
-        emit_u8_full<MODE>(ts, (uint32_t)(t.ip - h * 100000000ull));
-    } else {
-        const uint64_t h = t.ip / 10000000000000000ull, r = t.ip - h * 10000000000000000ull, m = r / 100000000ull;
-        emit_u8<MODE>(ts, (uint32_t)h, nd - 16u);
-        emit_u8_full<MODE>(ts, (uint32_t)m);
-        emit_u8_full<MODE>(ts, (uint32_t)(r - m * 100000000ull));
-    }
-    if (d) {
-        // the d fraction digits = the last d characters of the 9-digit zero-padded fq
-        const uint32_t top = t.fq / 100000000u, r8 = t.fq - top * 100000000u;
-        const uint32_t h = (uint32_t)(((uint64_t)r8 * 3518437209ull) >> 45);
-        const uint64_t ab = (uint64_t)swar4(h) | ((uint64_t)swar4(r8 - h * 10000u) << 32);      // 8 digits, most significant in byte 0
-        if (d == 6) {                                                  // ".dddddd<sep>": two whole words
-            const uint64_t x = ab >> 16;
-            ts.put4<MODE>(0x2eu | ((uint32_t)x << 8));
-            ts.put4<MODE>(((uint32_t)x >> 24) | ((uint32_t)(x >> 32) << 8) | (sep << 24));
-            return;
-        }
-        ts.put<MODE>(0x2eu, 1u);
-        if (d == 9) ts.put<MODE>(0x30u + top, 1u);
-        const uint32_t dd = d == 9 ? 8u : (uint32_t)d;
-        const uint64_t x = ab >> (8u * (8u - dd));
-        if (dd > 4u) { ts.put4<MODE>((uint32_t)x); ts.put<MODE>((uint32_t)(x >> 32), dd - 4u); }
-        else ts.put<MODE>((uint32_t)x, dd);
-    }
-    ts.put<MODE>(sep, 1u);
-}
-
 // write pass: one row per thread, 256 rows per tile; exact (ip, fq) per number by fmtg_prepare, digits by SWAR groups, word stream
 template <bool F64, int NC, uint32_t DP>
 __global__ void __launch_bounds__(kPcdTile) k_text_write(const void* __restrict__ rows, int64_t n, const __grid_constant__ TextFmt F,
@@ -754,7 +669,7 @@ __global__ void __launch_bounds__(kPcdTile) k_text_write(const void* __restrict_
     // zero the part of the image this tile can reach (row edges are OR-ed in)
     const int img_words = (int)((phase + (tile_off[blockIdx.x + 1] - dst0) + 3 + 15) / 16) * 4;
     for (int k = tid * 4; k < img_words; k += kPcdTile * 4) *reinterpret_cast<uint4*>(s_img + 4 * k) = make_uint4(0, 0, 0, 0);
-    TextNum t[kTextCols];
+    Num t[kTextCols];
     [[maybe_unused]] Piece pc[kTextCols];
     [[maybe_unused]] bool slow6 = false;                             // compiled formats: some '%.6f' column of the row is not a fast number
     uint32_t len = 0, fl = 0;

@@ -10,7 +10,9 @@ reference's NumPy path.
 """
 import hashlib
 import json
+import math
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -813,9 +815,18 @@ def test_pcd_ascii_large_random(f64):
     got = body.cpu().numpy().tobytes()
     want = "".join("%.6f %.6f %.6f %.6f\n" % tuple(r) for r in pts.astype(np.float64)).encode()
     assert int(status.item()) == 0 and got == want
-    big = np.array([[1e13, 0, 0, 0]] * 3)
-    _, status = ops.pcd_ascii_body(dev(big))
-    assert int(status.item()) & C.FLAG_OVERFLOW
+    # a finite |v| >= 9.2e12 prints saturated and sets the overflow flag, in the size pass, the row offsets and the text alike
+    big = [9.2e12, -1e13, 2.0 ** 52, 1e300, -sys.float_info.max] if f64 else [9.2e12, -1e13, 2.0 ** 52, 3.4e38, -3.4e38]
+    sat = lambda x: ("-" if x < 0 else "") + "9199999999999.999999"          # noqa: E731
+    for v in big:
+        rows = np.array([[v, 0.5, -v, v]] * 3, np.float64 if f64 else np.float32)
+        line = ("%s 0.500000 %s %s\n" % (sat(v), sat(-v), sat(v))).encode()
+        body, tile_off, status = ops._pcd_format(dev(rows))
+        assert body.cpu().numpy().tobytes() == 3 * line and int(tile_off[-1].item()) == 3 * len(line), v
+        assert int(status.item()) == C.FLAG_OVERFLOW, v
+        text, boff, status = ops.pcd_ascii_frames(dev(rows), dev(np.array([0, 1, 3], np.int64)))
+        assert text.cpu().numpy().tobytes() == 3 * line and boff.cpu().numpy().tolist() == [0, len(line), 3 * len(line)], v
+        assert int(status.item()) == C.FLAG_OVERFLOW, v
 
 
 @pytest.mark.parametrize("f64", [True, False], ids=["f64", "f32"])
@@ -868,6 +879,29 @@ def test_pcd_ascii_tile_edges_and_slow_numbers(f64):
         assert t[0] == 0 and (np.diff(t) >= 0).all() and len(t) == (n + 255) // 256 + 1
         if n > 256:
             assert t[1] == len("".join("%.6f %.6f %.6f %.6f\n" % tuple(r) for r in pts[:256].astype(np.float64)))
+    # slow numbers over the whole range printed without a flag, [1e4, 9.2e12) of both signs, mixed into every column and as
+    # whole rows: random magnitudes, exact binary ties (k + 0.5) / 2^j above 2^43 (j = 6: a tie of the 6th decimal) and the
+    # largest double below the cap
+    n = 3 * 512 + 77
+    big = 10.0 ** rng.uniform(4, math.log10(9.2e12), (n, 4))
+    j = rng.integers(0, 9, (n, 4))
+    k = rng.integers(2 ** 43, 9.2e12 - 1, (n, 4)) * 2 ** j + rng.integers(0, 2 ** j)
+    tie = rng.random((n, 4)) < 0.4
+    big[tie] = (k[tie] + 0.5) / 2.0 ** j[tie]
+    big = np.minimum(big, math.nextafter(9.2e12, 0.0))
+    big[100] = big[511] = math.nextafter(9.2e12, 0.0)
+    big = np.where(rng.random((n, 4)) < 0.5, -big, big)
+    pts = rng.uniform(-1, 1, (n, 4)) * 10.0 ** rng.integers(-3, 4, (n, 4))
+    pick = rng.random((n, 4)) < 0.5
+    pick[200:260] = pick[511:514] = True
+    pts[pick] = big[pick]
+    if not f64:
+        pts = pts.astype(np.float32)
+        pts = np.clip(pts, -np.nextafter(np.float32(9.2e12), np.float32(0)), np.nextafter(np.float32(9.2e12), np.float32(0)))
+    want = "".join("%.6f %.6f %.6f %.6f\n" % tuple(r) for r in pts.astype(np.float64)).encode()
+    body, tile_off, status = ops._pcd_format(dev(pts))
+    assert body.cpu().numpy().tobytes() == want
+    assert int(status.item()) == 0 and int(tile_off[-1].item()) == len(want)
 
 
 def test_save_results_files_are_save_pcd_files(golden, tmp_path):

@@ -400,20 +400,23 @@ def test_exporter_merge_frames():
     assert exporter.PCD_HEADER.format(n=3).count("3") == 2 and exporter.CSV_HEADER == "x,y,z,intensity,timestamp\n"
 
 
+def _text_digit_table(src):
+    m = re.search(r"kTextT\[10\]\[20\]\s*=\s*\{(.*?)\n\};", src, re.S)
+    rows = re.findall(r"\{([^{}]*)\}", m.group(1))
+    return [[float.fromhex(t.strip()) if "x" in t else float(t) for t in r.split(",")] for r in rows]
+
+
 def test_pcd_digit_count_thresholds_are_exact():
     """csrc/lmc_pcd.cu: the length of '%.6f' is decided by comparing |v| with kDigitT[k-1] = the smallest double >= 10^k - 5e-7
-    (the real threshold is never a double, so the comparison is exact).  Re-derive the four constants with exact fractions
-    and check the boundary doubles against CPython's formatting."""
+    (the real threshold is never a double, so the comparison is exact).  The four constants are the '%.6f' row of the text
+    writer's kTextT (whose exact derivation is checked below); check the boundary doubles against CPython's formatting."""
     import math
-    from fractions import Fraction
     src = open(os.path.join(ROOT, "livox_motion_compensation_sim_b200", "csrc", "lmc_pcd.cu")).read()
     m = re.search(r"kDigitT\[4\]\s*=\s*\{([^}]*)\}", src)
     consts = [float.fromhex(t.strip()) for t in m.group(1).split(",")]
-    assert len(consts) == 4
+    assert consts == _text_digit_table(src)[6][1:5]
     for k, c in enumerate(consts, start=1):
-        thr = Fraction(10) ** k - Fraction(5, 10 ** 7)
         below = math.nextafter(c, 0.0)
-        assert Fraction(below) < thr < Fraction(c)
         assert "%.6f" % c == "1" + "0" * k + ".000000" and "%.6f" % below == "9" * k + ".999999"
         assert len("%.6f" % -c) == k + 9 and len("%.6f" % -below) == k + 8
 
@@ -425,9 +428,7 @@ def test_text_digit_count_table_is_exact():
     import math
     from fractions import Fraction
     src = open(os.path.join(ROOT, "livox_motion_compensation_sim_b200", "csrc", "lmc_pcd.cu")).read()
-    m = re.search(r"kTextT\[10\]\[20\]\s*=\s*\{(.*?)\n\};", src, re.S)
-    rows = re.findall(r"\{([^{}]*)\}", m.group(1))
-    T = [[float.fromhex(t.strip()) if "x" in t else float(t) for t in r.split(",")] for r in rows]
+    T = _text_digit_table(src)
     assert len(T) == 10 and all(len(r) == 20 for r in T)
     for d in range(10):
         for k in range(1, 20):
