@@ -179,6 +179,38 @@ int lmc_deskew_slerp_f32(const float* pts_n4, const uint32_t* ts_off, const int6
                          int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream);
 
 /*
+ * Pose at a time: Mode C's pose at each of n_query int64 ns times, with Mode C's bracket, end clamps and alpha
+ * (definition: oracle/lmc_oracle_local.c::orc_slerp_pose_at).  pose_out (n_query, 12) f64 is laid out like lmc_align_rigid_*'s
+ * pose_Rt: R(t) row-major, then pos(t).  lmc_align_rigid_* with these rows is Mode A at the interpolated pose.
+ * 1 <= n_samples < 2^31; seg and pose_out 16-byte aligned.
+ */
+int lmc_slerp_pose_at(const int64_t* sample_ts, const double* seg, int64_t n_samples,
+                      const int64_t* query_ts, int64_t n_query, double* pose_out, void* stream);
+
+/*
+ * Sensor-frame deskew: every point of frame f in the sensor frame of the frame's reference pose (R_r, x_r) = ref_pose[f]
+ * (normally lmc_slerp_pose_at at the frame's start or end time), rotation and translation removed
+ * (definition: oracle/lmc_oracle_local.c::orc_deskew_slerp_local_f64):
+ *   w   = R(ts) p + (pos(ts) - x_r)       Mode C's pose at the point's time, the offset formed before the lerp
+ *   out = R_r^T w ;  out[3] = p[3]
+ * The world position is never rounded to the point layout, so map / UTM-scale positions cost no precision in the f32
+ * layout.  Arguments, layouts, shards and exports as lmc_deskew_slerp_* (no hold_idx); ref_pose (n_frames, 12) f64,
+ * 16-byte aligned, Mode A's row layout.  LMC_LVX2_OF_OUTPUT records are the second simulator's LVX2 points with
+ * translation compensated.  Refused (LMC_ERR_INVALID, nothing written): n_peers > 0 or multicast pointers (a merged
+ * cloud of points in per-frame sensor frames means nothing), ref_pose NULL, n_samples < 1 or >= 2^31.
+ */
+int lmc_deskew_slerp_local_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off,
+                               const int64_t* frame_start, const int64_t* sample_ts, const double* seg,
+                               int64_t n_samples, const double* ref_pose, double* out_n4,
+                               int64_t n_points, int32_t n_frames,
+                               int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream);
+int lmc_deskew_slerp_local_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off,
+                               const int64_t* frame_start, const int64_t* sample_ts, const double* seg,
+                               int64_t n_samples, const double* ref_pose, float* out_n4,
+                               int64_t n_points, int32_t n_frames,
+                               int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream);
+
+/*
  * (a4)/(a5)/(a9)/(a10) stand-alone quantisers (no transform): LivoxLVXWriter._write_point_data_type2
  * LMC:252-272, the LVX2 packer CS:365-374 and the LAS integer packing behind LMC:957-961 /
  * CS:1683-1686.  `ex` selects outputs and modes exactly as in the fused calls; for lvx_mode both

@@ -58,6 +58,9 @@ _SIGNATURES = {
     "lmc_deskew_slerp_f64": ([vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
     "lmc_deskew_slerp_f32": ([vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
     "lmc_build_slerp_table": ([vp, vp, vp, i64, vp, vp], ctypes.c_int),
+    "lmc_slerp_pose_at": ([vp, vp, i64, vp, i64, vp, vp], ctypes.c_int),
+    "lmc_deskew_slerp_local_f64": ([vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
+    "lmc_deskew_slerp_local_f32": ([vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
     "lmc_quantize_f64": ([vp, i64, vp, vp], ctypes.c_int),
     "lmc_quantize_f32": ([vp, i64, vp, vp], ctypes.c_int),
     "lmc_lvx_v11_build_f64": ([vp, vp, vp, vp, vp, vp, i64, i32, i64, vp, vp], ctypes.c_int),

@@ -29,6 +29,8 @@ cudaError_t launch_lvx_v11(bool f64, const void* pts, const int64_t* frame_off, 
                            const int64_t* frame_id, uint8_t* out, int32_t n_frames, int32_t f_begin, int32_t f_end, int64_t max_frame_points,
                            uint32_t* status, cudaStream_t st);
 cudaError_t launch_slerp_table(const double* quat, const double* pos, const int64_t* ts, int64_t S, double* seg, cudaStream_t st);
+cudaError_t launch_slerp_pose_at(const int64_t* sample_ts, const double* seg, int64_t S, const int64_t* query_ts, int64_t n_query,
+                                 double* pose, cudaStream_t st);
 cudaError_t launch_homog(bool f64, const void* in, const double* T_host, int32_t order, void* out, int64_t n, cudaStream_t st);
 cudaError_t launch_text_size(bool f64, const void* rows, int64_t n, int32_t n_cols, int32_t row_stride, const int32_t* col, const int32_t* dec,
                              uint8_t sep, int64_t* tile_off, cudaStream_t st);
@@ -250,6 +252,46 @@ int lmc_deskew_slerp_f32(const float* pts_n4, const uint32_t* ts_off, const int6
                          float* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
                          const lmc_export* ex, void* stream) {
     LMC_SLERP_BODY(false, ts_off, true)
+}
+
+int lmc_slerp_pose_at(const int64_t* sample_ts, const double* seg, int64_t n_samples, const int64_t* query_ts, int64_t n_query,
+                      double* pose_out, void* stream) {
+    int rc = check_device();
+    if (rc != LMC_OK) return rc;
+    if (n_samples < 1 || n_samples >= (1LL << 31) || n_query < 0) return fail(LMC_ERR_INVALID, "need 1 <= n_samples < 2^31, n_query >= 0");
+    if (n_query == 0) return LMC_OK;
+    if (!sample_ts || !seg || !query_ts || !pose_out) return fail(LMC_ERR_INVALID, "NULL argument");
+    if ((reinterpret_cast<uintptr_t>(seg) | reinterpret_cast<uintptr_t>(pose_out)) & 15u) return fail(LMC_ERR_ALIGN, "seg / pose_out must be 16-byte aligned");
+    cudaError_t e = lmc::launch_slerp_pose_at(sample_ts, seg, n_samples, query_ts, n_query, pose_out, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_slerp_pose_at");
+}
+
+#define LMC_SLERP_LOCAL_BODY(F64, TS, NEED_FS)                                                           \
+    lmc::Params P = base_params(pts_n4, out_n4, n_points, n_frames, p_begin, p_end);                     \
+    if (n_samples < 1 || n_samples >= (1LL << 31) || !sample_ts || !seg)                                 \
+        return fail(LMC_ERR_INVALID, "need a sample table of 1 .. 2^31 - 1 rows");                       \
+    if (!ref_pose) return fail(LMC_ERR_INVALID, "ref_pose is NULL");                                     \
+    if (ex && (ex->n_peers > 0 || ex->mc_out || ex->mc_lvx14))                                           \
+        return fail(LMC_ERR_INVALID, "sensor-frame deskew has no merged-cloud assembly (each frame is in its own sensor frame)"); \
+    if (!TS) return fail(LMC_ERR_INVALID, "timestamps are NULL");                                        \
+    if (NEED_FS && !frame_start) return fail(LMC_ERR_INVALID, "frame_start is NULL");                    \
+    if ((reinterpret_cast<uintptr_t>(TS) | reinterpret_cast<uintptr_t>(seg) | reinterpret_cast<uintptr_t>(ref_pose)) & 15u) \
+        return fail(LMC_ERR_ALIGN, "timestamps / seg / ref_pose must be 16-byte aligned");               \
+    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = TS; P.pose_Rt = ref_pose;               \
+    P.samp_ts = sample_ts; P.samp_tab = seg; P.n_samp = n_samples;                                       \
+    return run(F64, lmc::kSlerpLocal, P, ex, stream);
+
+int lmc_deskew_slerp_local_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off, const int64_t* frame_start,
+                               const int64_t* sample_ts, const double* seg, int64_t n_samples, const double* ref_pose,
+                               double* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
+                               const lmc_export* ex, void* stream) {
+    LMC_SLERP_LOCAL_BODY(true, ts, false)
+}
+int lmc_deskew_slerp_local_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off, const int64_t* frame_start,
+                               const int64_t* sample_ts, const double* seg, int64_t n_samples, const double* ref_pose,
+                               float* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
+                               const lmc_export* ex, void* stream) {
+    LMC_SLERP_LOCAL_BODY(false, ts_off, true)
 }
 
 int lmc_quantize_f64(const double* pts_n4, int64_t n_points, const lmc_export* ex, void* stream) {

@@ -269,6 +269,26 @@ __device__ __forceinline__ void gyro_rotate_small(double ax, double ay, double a
     o.w = p.w;
 }
 
+// Mode C's Rodrigues step: p rotated by alpha * theta_k about the unit axis n_k (before R_k is applied); the same operations
+// as slerp_apply's first half (kept separate there: routing Mode C through this function perturbs its register allocation)
+template <bool SMALL>
+__device__ __forceinline__ void slerp_rotate(const double (&s)[kSegStride], double alpha, double px, double py, double pz,
+                                             double& x1, double& y1, double& z1) {
+    const double th = __dmul_rn(alpha, s[15]);
+    double sn, v;
+    if (SMALL) sin_vercos_small(th, sn, v); else sin_vercos(th, sn, v);
+    const double nx = s[12], ny = s[13], nz = s[14];
+    const double c1x = __fma_rn(ny, pz, -__dmul_rn(nz, py));
+    const double c1y = __fma_rn(nz, px, -__dmul_rn(nx, pz));
+    const double c1z = __fma_rn(nx, py, -__dmul_rn(ny, px));
+    const double c2x = __fma_rn(ny, c1z, -__dmul_rn(nz, c1y));
+    const double c2y = __fma_rn(nz, c1x, -__dmul_rn(nx, c1z));
+    const double c2z = __fma_rn(nx, c1y, -__dmul_rn(ny, c1x));
+    x1 = __fma_rn(v, c2x, __fma_rn(sn, c1x, px));
+    y1 = __fma_rn(v, c2y, __fma_rn(sn, c1y, py));
+    z1 = __fma_rn(v, c2z, __fma_rn(sn, c1z, pz));
+}
+
 // Mode C per-point evaluation (definition: oracle/lmc_oracle.c::orc_deskew_slerp_f64)
 template <bool SMALL = false>
 __device__ __forceinline__ void slerp_apply(const double (&s)[kSegStride], double alpha, const Pt& p, Pt& o) {
@@ -289,6 +309,27 @@ __device__ __forceinline__ void slerp_apply(const double (&s)[kSegStride], doubl
     o.y = __dadd_rn(dot_gemm(s[3], x1, s[4], y1, s[5], z1), __fma_rn(alpha, s[17], s[10]));
     o.z = __dadd_rn(dot_gemm(s[6], x1, s[7], y1, s[8], z1), __fma_rn(alpha, s[18], s[11]));
     o.w = p.w;
+}
+
+// Sensor-frame deskew (definition: oracle/lmc_oracle_local.c::orc_deskew_slerp_local_f64): Mode C's world point, formed as an
+// offset from the reference position x_r before the lerp (world-scale magnitudes never enter the result), then R_r^T.
+// ref = the frame's reference pose, R_r row-major | x_r.
+template <bool SMALL = false>
+__device__ __forceinline__ void slerp_local_apply(const double (&s)[kSegStride], double alpha, const double (&ref)[12], const Pt& p, Pt& o) {
+    double x1, y1, z1;
+    slerp_rotate<SMALL>(s, alpha, p.x, p.y, p.z, x1, y1, z1);
+    const double w0 = __dadd_rn(dot_gemm(s[0], x1, s[1], y1, s[2], z1), __fma_rn(alpha, s[16], __dsub_rn(s[9], ref[9])));
+    const double w1 = __dadd_rn(dot_gemm(s[3], x1, s[4], y1, s[5], z1), __fma_rn(alpha, s[17], __dsub_rn(s[10], ref[10])));
+    const double w2 = __dadd_rn(dot_gemm(s[6], x1, s[7], y1, s[8], z1), __fma_rn(alpha, s[18], __dsub_rn(s[11], ref[11])));
+    o.x = dot_gemm(ref[0], w0, ref[3], w1, ref[6], w2);
+    o.y = dot_gemm(ref[1], w0, ref[4], w1, ref[7], w2);
+    o.z = dot_gemm(ref[2], w0, ref[5], w1, ref[8], w2);
+    o.w = p.w;
+}
+__device__ __forceinline__ void load_pose12(const double* src, double (&m)[12]) {
+    const double2* pr = reinterpret_cast<const double2*>(src);
+#pragma unroll
+    for (int q = 0; q < 6; ++q) { const double2 v = __ldg(pr + q); m[2 * q] = v.x; m[2 * q + 1] = v.y; }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -556,6 +597,21 @@ __device__ __forceinline__ Pt point_eval(const Params& P, int32_t f, bool single
         for (int q = 0; q < kSegStride / 2; ++q) { const double2 v = __ldg(sr + q); row[2 * q] = v.x; row[2 * q + 1] = v.y; }
         alpha = __dmul_rn(alpha, row[19]);
         slerp_apply(row, alpha, in, out);
+    } else if constexpr (MODE == kSlerpLocal) {
+        const int64_t S = P.n_samp;
+        const int64_t t = F64 ? tsraw : tsraw + fs;
+        const Bracket b = bracket_of(P.samp_ts, S, t, t0, rate);
+        int64_t k = b.k; double alpha = 0.0;
+        if (k < 0) k = 0;
+        else if (k >= S - 1) k = S - 1;
+        else alpha = (double)(t - b.tb);
+        double row[kSegStride], ref[12];
+        const double2* sr = reinterpret_cast<const double2*>(P.samp_tab + kSegStride * k);
+#pragma unroll
+        for (int q = 0; q < kSegStride / 2; ++q) { const double2 v = __ldg(sr + q); row[2 * q] = v.x; row[2 * q + 1] = v.y; }
+        load_pose12(P.pose_Rt + 12 * (int64_t)f, ref);
+        alpha = __dmul_rn(alpha, row[19]);
+        slerp_local_apply(row, alpha, ref, in, out);
     }
     return out;
 }
@@ -575,13 +631,13 @@ __device__ __noinline__ Pt point_eval_slow(const Params& P, int32_t f, bool sing
 // ------------------------------------------------------------------------------------------
 template <bool F64, int MODE>
 struct PointCtx {
-    double  tab[MODE == kSlerp ? kSegStride : 12];
+    double  tab[kSlerpFamily<MODE> ? kSegStride : 12];
     int32_t key = -1;            // frame (Mode A) or sample index (Mode C) held in tab
     int64_t t0 = 0;              // Mode B/C: first sample time and mean sample rate for the bracket guess
     double  rate = 0.0;
 
     __device__ __forceinline__ void init(const Params& P) {
-        if constexpr (MODE == kGyro || MODE == kSlerp) {
+        if constexpr (MODE == kGyro || kSlerpFamily<MODE>) {
             if (P.n_samp > 0) {
                 t0 = __ldg(P.samp_ts);
                 const int64_t span = __ldg(P.samp_ts + P.n_samp - 1) - t0;
@@ -615,7 +671,7 @@ struct PointCtx {
                 return;
             }
         }
-        if constexpr (MODE == kSlerp) {
+        if constexpr (kSlerpFamily<MODE>) {
             const int64_t S = P.n_samp;
             if (LEAN || (P.hold_idx == nullptr && S >= 2 && S < 0x7fffffffLL)) {
                 const int64_t ta = F64 ? tsraw[0] : tsraw[0] + fs[0];
@@ -662,8 +718,16 @@ struct PointCtx {
                     for (int q = 12; q < kSegStride; ++q) row[q] = tab[q];
                     const double a0 = __dmul_rn((double)da, row[19]);
                     const double a1 = __dmul_rn((double)db, row[19]);
-                    slerp_apply<true>(row, a0, in[0], out[0]);
-                    slerp_apply<true>(row, a1, in[1], out[1]);
+                    if constexpr (MODE == kSlerp) {
+                        slerp_apply<true>(row, a0, in[0], out[0]);
+                        slerp_apply<true>(row, a1, in[1], out[1]);
+                    } else {                                          // the frame's reference pose row: L1, like R_k / pos_k
+                        double ref[12];
+                        load_pose12(P.pose_Rt + 12 * (int64_t)f[0], ref);
+                        slerp_local_apply<true>(row, a0, ref, in[0], out[0]);
+                        if (f[1] != f[0]) load_pose12(P.pose_Rt + 12 * (int64_t)f[1], ref);      // (a frame boundary inside the pair: rare)
+                        slerp_local_apply<true>(row, a1, ref, in[1], out[1]);
+                    }
                     return;
                 }
             }

@@ -41,7 +41,7 @@ __device__ __forceinline__ void tile_body(const Params& P, int64_t base, int64_t
         in[j][0] = in[j][1] = Pt{ 0.0, 0.0, 0.0, 0.0 };
         load_pair<F64, FULL>(P.pts, p, va, vb, in[j][0], in[j][1]);
         tsv[j][0] = tsv[j][1] = 0;
-        if constexpr (MODE == kGyro || MODE == kSlerp) {
+        if constexpr (MODE == kGyro || kSlerpFamily<MODE>) {
             if (P.ts != nullptr) {
                 if constexpr (F64) {
                     const int64_t* t = reinterpret_cast<const int64_t*>(P.ts) + p;
@@ -81,7 +81,7 @@ __device__ __forceinline__ void tile_body(const Params& P, int64_t base, int64_t
             if constexpr (MODE != kQuantOnly) {
                 if (FULL || valid[j][h]) {
                     f[h] = frame_of(P, s_tm, base + 2 * (tid + j * kThreads) + h, single[h]);
-                    if constexpr (MODE == kGyro || MODE == kSlerp) { if (P.frame_start != nullptr) fs[h] = frame_start_of(P, s_tm, f[h]); }
+                    if constexpr (MODE == kGyro || kSlerpFamily<MODE>) { if (P.frame_start != nullptr) fs[h] = frame_start_of(P, s_tm, f[h]); }
                 }
             }
         }
@@ -126,6 +126,21 @@ __global__ void __launch_bounds__(kThreads, 2) k_fused(const __grid_constant__ P
     if (lim_lo >= lim_hi) return;
     if (lim_lo == base && lim_hi == base + kTile) tile_body<F64, MODE, true>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
     else                                          tile_body<F64, MODE, false>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
+}
+// sensor-frame deskew (kSlerpLocal) under its own name: k_fused's body.  (Not shared through an inline function: routing
+// k_fused itself through one changes the register allocation of its float4 instantiations.)
+template <bool F64>
+__global__ void __launch_bounds__(kThreads, 2) k_local_fused(const __grid_constant__ Params P)
+{
+    __shared__ __align__(16) uint32_t s_lvx[kTilePairs * 7];
+    __shared__ TileMeta s_tm;
+    const int64_t tile0 = (P.p_begin / kTile) * kTile;
+    const int64_t base  = tile0 + (int64_t)blockIdx.x * kTile;
+    const int64_t lim_lo = base > P.p_begin ? base : P.p_begin;
+    const int64_t lim_hi = base + kTile < P.p_end ? base + kTile : P.p_end;
+    if (lim_lo >= lim_hi) return;
+    if (lim_lo == base && lim_hi == base + kTile) tile_body<F64, kSlerpLocal, true>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
+    else                                          tile_body<F64, kSlerpLocal, false>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
 }
 
 // (a1) LMC:802-812: one thread per frame
@@ -203,6 +218,42 @@ __global__ void k_slerp_table(const double* __restrict__ quat, const double* __r
     for (int j = 0; j < kSegStride / 2; ++j) dst[j] = make_double2(row[2 * j], row[2 * j + 1]);
 }
 
+// Pose at a time (definition: oracle/lmc_oracle_local.c::orc_slerp_pose_at), one thread per query: Mode C's bracket, clamps and
+// alpha, then column j of R(t) = R_k (Rodrigues step of e_j) and pos(t) = pos_k + alpha dpos_k -- 12 doubles laid out as a
+// Mode A pose row.
+__global__ void k_slerp_pose_at(const int64_t* __restrict__ sample_ts, const double* __restrict__ seg, int64_t S,
+                                const int64_t* __restrict__ query_ts, int64_t n_query, double* __restrict__ pose)
+{
+    const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_query) return;
+    const int64_t t0 = __ldg(sample_ts), span = __ldg(sample_ts + S - 1) - t0;
+    const double rate = span > 0 ? (double)(S - 1) / (double)span : 0.0;
+    const int64_t t = __ldg(query_ts + q);
+    const Bracket b = bracket_of(sample_ts, S, t, t0, rate);
+    int64_t k = b.k; double alpha = 0.0;
+    if (k < 0) k = 0;
+    else if (k >= S - 1) k = S - 1;
+    else alpha = (double)(t - b.tb);
+    double row[kSegStride];
+    const double2* sr = reinterpret_cast<const double2*>(seg + kSegStride * k);
+#pragma unroll
+    for (int j = 0; j < kSegStride / 2; ++j) { const double2 v = __ldg(sr + j); row[2 * j] = v.x; row[2 * j + 1] = v.y; }
+    alpha = __dmul_rn(alpha, row[19]);
+    double M[12];
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+        double x1, y1, z1;
+        slerp_rotate<false>(row, alpha, j == 0 ? 1.0 : 0.0, j == 1 ? 1.0 : 0.0, j == 2 ? 1.0 : 0.0, x1, y1, z1);
+#pragma unroll
+        for (int r = 0; r < 3; ++r) M[3 * r + j] = dot_gemm(row[3 * r], x1, row[3 * r + 1], y1, row[3 * r + 2], z1);
+    }
+#pragma unroll
+    for (int r = 0; r < 3; ++r) M[9 + r] = __fma_rn(alpha, row[16 + r], row[9 + r]);
+    double2* dst = reinterpret_cast<double2*>(pose + 12 * q);
+#pragma unroll
+    for (int j = 0; j < 6; ++j) dst[j] = make_double2(M[2 * j], M[2 * j + 1]);
+}
+
 // ---- launchers -------------------------------------------------------------------------------
 template <bool F64, int MODE>
 static cudaError_t launch_fused(const Params& P, cudaStream_t st) {
@@ -210,7 +261,8 @@ static cudaError_t launch_fused(const Params& P, cudaStream_t st) {
     const int64_t tile0 = (P.p_begin / kTile) * kTile;
     const int64_t tiles = (P.p_end - tile0 + kTile - 1) / kTile;
     if (tiles > 0x7fffffffLL) return cudaErrorInvalidValue;
-    k_fused<F64, MODE><<<(unsigned)tiles, kThreads, 0, st>>>(P);
+    if constexpr (MODE == kSlerpLocal) k_local_fused<F64><<<(unsigned)tiles, kThreads, 0, st>>>(P);
+    else                               k_fused<F64, MODE><<<(unsigned)tiles, kThreads, 0, st>>>(P);
     return cudaGetLastError();
 }
 
@@ -224,6 +276,15 @@ cudaError_t launch_pose_lookup(const double* traj_t, int64_t n_t, const double* 
                                int32_t n_frames, double* pose_Rt, int32_t* pose_idx, cudaStream_t st) {
     if (n_frames <= 0) return cudaSuccess;
     k_pose_lookup<<<(n_frames + 127) / 128, 128, 0, st>>>(traj_t, n_t, traj_Rt, frame_t, n_frames, pose_Rt, pose_idx);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_slerp_pose_at(const int64_t* sample_ts, const double* seg, int64_t S, const int64_t* query_ts, int64_t n_query,
+                                 double* pose, cudaStream_t st) {
+    if (n_query <= 0) return cudaSuccess;
+    const int64_t blocks = (n_query + 127) / 128;
+    if (blocks > 0x7fffffffLL) return cudaErrorInvalidValue;
+    k_slerp_pose_at<<<(unsigned)blocks, 128, 0, st>>>(sample_ts, seg, S, query_ts, n_query, pose);
     return cudaGetLastError();
 }
 

@@ -7,7 +7,11 @@
 
 namespace lmc {
 
-enum Mode : int { kRigid = 0, kGyro = 1, kSlerp = 2, kQuantOnly = 3 };
+// kSlerpLocal: Mode C's per-point pose, then into the sensor frame of the frame's reference pose (pose_Rt, one row per
+// frame): every point of a frame in the sensor frame of one instant, rotation and translation removed
+enum Mode : int { kRigid = 0, kGyro = 1, kSlerp = 2, kQuantOnly = 3, kSlerpLocal = 4 };
+constexpr bool slerp_mode(int mode) { return mode == kSlerp || mode == kSlerpLocal; }
+template <int MODE> inline constexpr bool kSlerpFamily = slerp_mode(MODE);      // (the same, usable in device code)
 
 // One launch = one Params block in constant/param space.
 struct Params {
@@ -16,7 +20,7 @@ struct Params {
     const void*     ts;           // int64[N] (f64 layout) | uint32[N] ns offsets (f32 layout)
     const int64_t*  frame_off;    // CSR, n_frames + 1
     const int64_t*  frame_start;  // int64[n_frames] ns
-    const double*   pose_Rt;      // Mode A: (n_frames, 12)
+    const double*   pose_Rt;      // Mode A: (n_frames, 12) | kSlerpLocal: reference pose per frame, same layout
     const int64_t*  samp_ts;      // Mode B: imu_ts | Mode C: sample_ts
     const double*   samp_tab;     // Mode B: imu_gyro (S,3) | Mode C: seg (S,20)
     const int32_t*  hold_idx;     // Mode C hold-next (optional)
@@ -44,7 +48,8 @@ struct Params {
 
 // k_stream tile shape (measured on B200, see profiles/): 15 consumer warps + 1 producer warp (512 threads -> 128 registers
 // each).  Mode C on float4 points amortises its per-tile bookkeeping best with 3 point pairs per thread (over a 3-stage
-// ring); everything else runs 2 pairs (f32) / 1 pair (f64) per thread.
+// ring); everything else runs 2 pairs (f32) / 1 pair (f64) per thread.  (Sensor-frame deskew holds a reference pose row
+// besides Mode C's: with 3 pairs its LVX2 variant spills twice what Mode C's lean variants do, with 2 it spills less.)
 constexpr int kCW = 15;
 constexpr int stream_pairs_per_thread(bool f64, int mode) { return f64 ? 1 : (mode == kSlerp ? 3 : 2); }
 constexpr int stream_tile_points(bool f64, int mode) { return kCW * 32 * 2 * stream_pairs_per_thread(f64, mode); }   // 960 / 1920 / 2880
@@ -53,7 +58,7 @@ constexpr int stream_tile_points(bool f64, int mode) { return kCW * 32 * 2 * str
 // (kExGeneric).  Lean variants also assume what plan_point_launch has verified: LVX records are type-2-of-input without
 // tag bytes, timestamps / frame starts are present where the mode needs them, no hold_idx, 2 <= n_samp < 2^31 - 1.
 // kExLvx2 (with kExLvx): the records are CS:365-374 on the COMPENSATED point (+ optional tag bytes) instead of LMC:252-272 on
-// the raw one -- the second simulator's product, lean for Mode B.
+// the raw one -- the second simulator's product, lean for Mode B and for sensor-frame deskew.
 // kExMc (with kExOut | kExLvx): fused merged-cloud assembly through the NVSwitch multicast mapping of the symmetric buffers --
 // every result of a full tile leaves as ONE multimem.st (the switch replicates it into every rank's copy, this rank's
 // included) instead of a local store plus one store per peer; ragged edge tiles fall back to local + per-peer stores.
@@ -82,6 +87,8 @@ inline Plan refuse_call(const char* msg) {
 // path: lmc_set_path (0 direct, 1 auto, 2 streaming); sm_count: the current device's.  P is a validated, non-empty call.
 inline Plan plan_point_launch(bool f64, int mode, const Params& P, int path, int sm_count) {
     Plan pl;
+    if (mode == kSlerpLocal && (P.n_peers > 0 || P.mc_out || P.mc_lvx))
+        return refuse_call("sensor-frame deskew has no merged-cloud assembly (each frame is in its own sensor frame)");
     const int64_t tp = stream_tile_points(f64, mode);
     pl.tile0 = (P.p_begin / tp) * tp;
     pl.n_tiles = (P.p_end - pl.tile0 + tp - 1) / tp;
@@ -104,6 +111,11 @@ inline Plan plan_point_launch(bool f64, int mode, const Params& P, int path, int
     const bool merge_shape = !f64 && mode != kGyro && mask == (kExOut | kExLvx) && !lvx2;
     const bool pb = !mc && peers && merge_shape;
     const bool timed = P.ts && P.n_samp >= 2 && P.n_samp < 0x7fffffffLL;
+    if (mode == kSlerpLocal) {                              // lean: the aligned cloud, alone or with LVX2 records of it
+        const bool lean_local = timed && (f64 || P.frame_start) && (mask == kExOut || (mask == (kExOut | kExLvx) && lvx2));
+        if (lean_local) pl.ex = lvx2 ? (kExOut | kExLvx | kExLvx2) : kExOut;
+        return pl;
+    }
     bool lean = (!peers || mc || pb) && (!lvx2 || mode == kGyro) && (!(mask & kExLas) || (P.las_x && P.las_int));
     if (mode == kSlerp) lean = lean && !P.hold_idx && timed && (f64 || P.frame_start);
     if (mode == kGyro)  lean = lean && timed && P.frame_start;
@@ -122,10 +134,11 @@ template <class Fn>
 auto dispatch_layout_mode(bool f64, int mode, Fn&& fn) {
     using T = std::true_type;
     using F = std::false_type;
-    switch (mode) {                                         // (mode is one of the four Modes: default = kQuantOnly)
+    switch (mode) {                                         // (mode is one of the five Modes: default = kQuantOnly)
     case kRigid: return f64 ? fn(T{}, std::integral_constant<int, kRigid>{}) : fn(F{}, std::integral_constant<int, kRigid>{});
     case kGyro:  return f64 ? fn(T{}, std::integral_constant<int, kGyro>{})  : fn(F{}, std::integral_constant<int, kGyro>{});
     case kSlerp: return f64 ? fn(T{}, std::integral_constant<int, kSlerp>{}) : fn(F{}, std::integral_constant<int, kSlerp>{});
+    case kSlerpLocal: return f64 ? fn(T{}, std::integral_constant<int, kSlerpLocal>{}) : fn(F{}, std::integral_constant<int, kSlerpLocal>{});
     default:     return f64 ? fn(T{}, std::integral_constant<int, kQuantOnly>{}) : fn(F{}, std::integral_constant<int, kQuantOnly>{});
     }
 }

@@ -35,7 +35,7 @@ template <bool F64, int MODE> struct StreamCfg {
     static constexpr int TAG_STAGE = TP;
     static constexpr int STAGE     = PTS_STAGE + TS_STAGE + TAG_STAGE;
     static constexpr int LVX_SLAB  = PPT * 64 * 14;              // bytes per consumer warp
-    static constexpr int ROWS      = (MODE == kSlerp && !F64) ? 12 : 0;   // pose rows staged per tile (Mode C, float4 layout): a 2880-point tile of a 10 us / 200 Hz stream touches 7
+    static constexpr int ROWS      = (kSlerpFamily<MODE> && !F64) ? 12 : 0;   // pose rows staged per tile (Mode C, float4 layout): a 2880-point tile of a 10 us / 200 Hz stream touches 7
     static constexpr int ROW_STAGE = ROWS * kSegStride * 8;
     static constexpr int SMEM      = STAGES * (STAGE + ROW_STAGE) + kCW * LVX_SLAB + STAGES * (int)sizeof(TileMeta) + STAGES * 64 + 2 * STAGES * 8 + 128;
     static_assert(SMEM <= 227 * 1024, "stage ring does not fit the 227 KB of shared memory a CTA can have");
@@ -98,8 +98,8 @@ __device__ __forceinline__ void consume_tile(const Params& P, const TileInfo& ti
     const bool do_out = GEN ? P.out != nullptr : bool(EX & kExOut);
     const bool do_lvx = GEN ? P.lvx14 != nullptr : bool(EX & kExLvx);
     const bool do_las = GEN ? (P.las_x != nullptr || P.las_int != nullptr) : bool(EX & kExLas);
-    const bool has_ts = (MODE == kGyro || MODE == kSlerp) && (GEN ? P.ts != nullptr : true);
-    const bool has_fs = (MODE == kGyro || MODE == kSlerp) && (GEN ? P.frame_start != nullptr : (MODE == kGyro || !F64));
+    const bool has_ts = (MODE == kGyro || kSlerpFamily<MODE>) && (GEN ? P.ts != nullptr : true);
+    const bool has_fs = (MODE == kGyro || kSlerpFamily<MODE>) && (GEN ? P.frame_start != nullptr : (MODE == kGyro || !F64));
     constexpr bool LVX2 = !GEN && (EX & kExLvx2);                // lean, records of the output
     const bool has_tag = LVX2 ? P.tag != nullptr : (GEN && do_lvx && P.tag != nullptr && P.lvx_mode == LMC_LVX2_OF_OUTPUT);
     const int64_t base = ti.base;
@@ -176,7 +176,7 @@ __device__ __forceinline__ void consume_tile(const Params& P, const TileInfo& ti
             }
         }
         // with staged pose rows the stage is still being read by ctx.pair() below: release it after the last pair's math
-        constexpr bool ROWS_STAGED = FULL && !GEN && MODE == kSlerp && !F64;   // (f64 tiles are one pair per thread: holding the stage through the math costs more than the row reads)
+        constexpr bool ROWS_STAGED = FULL && !GEN && kSlerpFamily<MODE> && !F64;   // (f64 tiles are one pair per thread: holding the stage through the math costs more than the row reads)
         constexpr bool PB_FULL = PB && FULL;                 // the stage is the staging buffer of the bulk stores: released after they have read it
         if (j == PPT - 1 && !ROWS_STAGED && !PB_FULL) {      // everything this warp needs from the stage is in registers
             __syncwarp();
@@ -317,7 +317,7 @@ __device__ __forceinline__ void consume_tile(const Params& P, const TileInfo& ti
 }
 
 template <bool F64, int MODE, int EX>
-__global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles)
+__device__ __forceinline__ void stream_body(const Params& P, int64_t tile0, int64_t n_tiles)
 {
     using Cfg = StreamCfg<F64, MODE>;
     constexpr bool GEN = EX == kExGeneric;
@@ -342,7 +342,7 @@ __global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_const
     __syncthreads();
     const uint32_t full0 = smem_u32(s_full), empty0 = smem_u32(s_empty);       // barrier s lives at +8*s
 
-    const bool has_ts = (MODE == kGyro || MODE == kSlerp) && (GEN ? P.ts != nullptr : true);
+    const bool has_ts = (MODE == kGyro || kSlerpFamily<MODE>) && (GEN ? P.ts != nullptr : true);
     const bool has_tag = (GEN || (EX & kExLvx2)) && P.lvx14 != nullptr && P.tag != nullptr && P.lvx_mode == LMC_LVX2_OF_OUTPUT;
 
     if (warp == kCW) {
@@ -351,7 +351,7 @@ __global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_const
         int64_t hint = -1;
         int64_t base = tile0 + t_begin * Cfg::TP;
         [[maybe_unused]] int64_t p_t0 = 0; [[maybe_unused]] double p_rate = 0.0;   // same bracket guess as PointCtx::init
-        if constexpr (MODE == kSlerp && !GEN && !F64) {
+        if constexpr (kSlerpFamily<MODE> && !GEN && !F64) {
             p_t0 = __ldg(P.samp_ts);
             const int64_t span = __ldg(P.samp_ts + P.n_samp - 1) - p_t0;
             p_rate = span > 0 ? (double)(P.n_samp - 1) / (double)span : 0.0;
@@ -384,7 +384,7 @@ __global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_const
                 }
                 uint32_t row_bytes = 0;
                 const double* row_src = nullptr;
-                if constexpr (MODE == kSlerp && !GEN && !F64) {
+                if constexpr (kSlerpFamily<MODE> && !GEN && !F64) {
                     // the pose rows this tile reads, from the times of its first and last point (exact for time-ordered
                     // points; anything outside the staged window is simply read from global memory by the consumer)
                     if (full && !s_meta[s].overflow && (reinterpret_cast<uintptr_t>(P.samp_tab) & 15u) == 0) {
@@ -441,18 +441,30 @@ __global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_const
         if (fl != 0 && P.status != nullptr) atomicOr(P.status, fl);
     }
 }
+template <bool F64, int MODE, int EX>
+__global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles) {
+    stream_body<F64, MODE, EX>(P, tile0, n_tiles);
+}
+// sensor-frame deskew (kSlerpLocal) under its own name
+template <bool F64, int EX>
+__global__ void __launch_bounds__(kStreamThreads, 1) k_local_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles) {
+    stream_body<F64, kSlerpLocal, EX>(P, tile0, n_tiles);
+}
 
 // ---- launcher ----------------------------------------------------------------------------------
 template <bool F64, int MODE, int EX>
 static cudaError_t launch_stream_ex(const Params& P, const Plan& pl, int dev, cudaStream_t st) {
     using Cfg = StreamCfg<F64, MODE>;
+    void (*kern)(const Params, int64_t, int64_t);
+    if constexpr (MODE == kSlerpLocal) kern = k_local_stream<F64, EX>;
+    else                               kern = k_stream<F64, MODE, EX>;
     static thread_local int attr_dev = -1;
     if (attr_dev != dev) {
-        cudaError_t e = cudaFuncSetAttribute(k_stream<F64, MODE, EX>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
         if (e != cudaSuccess) return e;
         attr_dev = dev;
     }
-    k_stream<F64, MODE, EX><<<pl.grid, kStreamThreads, Cfg::SMEM, st>>>(P, pl.tile0, pl.n_tiles);
+    kern<<<pl.grid, kStreamThreads, Cfg::SMEM, st>>>(P, pl.tile0, pl.n_tiles);
     return cudaGetLastError();
 }
 
@@ -461,7 +473,10 @@ cudaError_t launch_stream(bool f64, int mode, const Params& P, const Plan& pl, i
     return dispatch_layout_mode(f64, mode, [&](auto f64_c, auto mode_c) -> cudaError_t {
         constexpr bool F64 = decltype(f64_c)::value;
         constexpr int MODE = decltype(mode_c)::value;
-        if constexpr (MODE != kQuantOnly) {
+        if constexpr (MODE == kSlerpLocal) {
+            if (pl.ex == kExOut)                    return launch_stream_ex<F64, MODE, kExOut>(P, pl, dev, st);
+            if (pl.ex == (kExOut | kExLvx | kExLvx2)) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExLvx2>(P, pl, dev, st);
+        } else if constexpr (MODE != kQuantOnly) {
             switch (pl.ex) {
             case kExOut:           return launch_stream_ex<F64, MODE, kExOut>(P, pl, dev, st);
             case kExOut | kExLvx:  return launch_stream_ex<F64, MODE, kExOut | kExLvx>(P, pl, dev, st);

@@ -224,6 +224,41 @@ def deskew_slerp(pts: torch.Tensor, ts: Optional[torch.Tensor], frame_off: torch
 
 
 @_on_tensor_device
+def slerp_pose_at(sample_ts: torch.Tensor, seg: torch.Tensor, query_ts: torch.Tensor) -> torch.Tensor:
+    """Mode C's pose at each int64 ns query time (same bracket, end clamps and alpha as deskew_slerp): (n, 12) f64 rows
+    [R row-major | pos], the pose_Rt layout of align_rigid -- align_rigid with them is Mode A at the interpolated pose."""
+    n = query_ts.shape[0]
+    pose = torch.empty((n, 12), dtype=torch.float64, device=query_ts.device)
+    C.check(C.lib().lmc_slerp_pose_at(_req(sample_ts, torch.int64, "sample_ts"), _req(seg, torch.float64, "seg", (22,)), sample_ts.shape[0],
+                                      _req(query_ts, torch.int64, "query_ts"), n, pose.data_ptr(), _stream_ptr()))
+    return pose
+
+
+@_on_tensor_device
+def deskew_slerp_local(pts: torch.Tensor, ts: torch.Tensor, frame_off: torch.Tensor, frame_start: Optional[torch.Tensor],
+                       sample_ts: torch.Tensor, seg: torch.Tensor, ref_pose: torch.Tensor, *, out: Optional[torch.Tensor] = None,
+                       export: Optional[ExportSpec] = None, p_range=None, want_out: bool = True):
+    """Sensor-frame deskew: every point of frame f in the sensor frame of ref_pose[f] ((F, 12) f64, normally
+    slerp_pose_at of the frame's start or end time), rotation and translation removed.  Arguments as deskew_slerp (no
+    hold_idx); the world position is kept in f64 registers, so the f32 layout loses nothing at map-scale positions."""
+    f64 = _layout(pts)
+    n, F = pts.shape[0], frame_off.shape[0] - 1
+    if ref_pose.shape[0] != F:
+        raise ValueError("ref_pose must have one row per frame")
+    if out is None and want_out:
+        out = torch.empty_like(pts)
+    ex, bufs = _make_export(export, n, pts.device)
+    b, e = _range(n, p_range)
+    fn = C.lib().lmc_deskew_slerp_local_f64 if f64 else C.lib().lmc_deskew_slerp_local_f32
+    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(ts, torch.int64 if f64 else torch.uint32, "ts"),
+               _req(frame_off, torch.int64, "frame_off"), _req(frame_start, torch.int64, "frame_start"),
+               _req(sample_ts, torch.int64, "sample_ts"), _req(seg, torch.float64, "seg", (22,)), sample_ts.shape[0],
+               _req(ref_pose, torch.float64, "ref_pose", (12,)), _req(out, pts.dtype, "out", (4,)), n, F, b, e,
+               None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
+    return out, bufs
+
+
+@_on_tensor_device
 def quantize(pts: torch.Tensor, export: ExportSpec) -> ExportBuffers:
     """(a4)/(a5)/(a9)/(a10) stand-alone quantisers over an (N,4) point array."""
     f64 = _layout(pts)

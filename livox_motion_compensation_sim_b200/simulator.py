@@ -257,14 +257,9 @@ class LiDARMotionSimulator:
         self.last_merged, self.last_frame_off, self.last_export = merged, off, bufs
         return FR.split_frames(merged, off)
 
-    @_trace.traced("LiDARMotionSimulator.deskew_scans")
-    def deskew_scans(self, raw_scans: List[dict], trajectory: Dict, export: Optional[ops.ExportSpec] = None,
-                     _device_raw=None) -> List[np.ndarray]:
-        """Per-point deskew + alignment (north_star Mode C; the reference has no such step -- parity is against the
-        builder's SciPy Slerp + lerp oracle).  Pose samples = the trajectory's GPS positions / IMU orientations at
-        their own times (LMC:396-428); a point's time is ``scan['point_times']`` (int64 ns) when the scan dict has
-        it, else frame time + i * (frame period / n_f) (SURVEY 8d M-C3).  Points outside the sample span hold the
-        end pose.  Returns the per-frame world clouds; merged buffer kept as in align_scans."""
+    def _deskew_inputs(self, raw_scans: List[dict], trajectory: Dict, _device_raw=None):
+        """The per-point times and the pose-segment table both deskews need: (flat points on the device, frame offsets,
+        frame starts, int64 ns point times, sample times, seg) -- None for the device arrays when there are no points."""
         from scipy.spatial.transform import Rotation
         if _device_raw is not None:                                 # scans still resident on the device (run_simulation)
             flat_d, off = _device_raw
@@ -273,8 +268,7 @@ class LiDARMotionSimulator:
             flat_d = None
         n = int(off[-1])
         if n == 0:
-            self.last_merged, self.last_frame_off, self.last_export = np.zeros((0, 4)), off, None
-            return FR.split_frames(self.last_merged, off)
+            return None, off, None, None, None, None
         if flat_d is None:
             flat_d = self._to_dev(flat)
         period_ns = int(round(1e9 / float(self.config['lidar_fps'])))
@@ -288,8 +282,56 @@ class LiDARMotionSimulator:
         s_ts = np.round(np.asarray(trajectory['time'], np.float64) * 1e9).astype(np.int64)
         quat = Rotation.from_euler('xyz', np.asarray(trajectory['orientation_imu'], np.float64)).as_quat()
         seg = ops.build_slerp_table(self._to_dev(quat), self._to_dev(np.asarray(trajectory['position_gps'], np.float64)), self._to_dev(s_ts))
-        out, bufs = ops.deskew_slerp(flat_d, self._to_dev(ts), self._to_dev(off), self._to_dev(fstart), self._to_dev(s_ts), seg,
+        return flat_d, off, fstart, ts, self._to_dev(s_ts), seg
+
+    @_trace.traced("LiDARMotionSimulator.deskew_scans")
+    def deskew_scans(self, raw_scans: List[dict], trajectory: Dict, export: Optional[ops.ExportSpec] = None,
+                     _device_raw=None) -> List[np.ndarray]:
+        """Per-point deskew + alignment (north_star Mode C; the reference has no such step -- parity is against the
+        builder's SciPy Slerp + lerp oracle).  Pose samples = the trajectory's GPS positions / IMU orientations at
+        their own times (LMC:396-428); a point's time is ``scan['point_times']`` (int64 ns) when the scan dict has
+        it, else frame time + i * (frame period / n_f) (SURVEY 8d M-C3).  Points outside the sample span hold the
+        end pose.  Returns the per-frame world clouds; merged buffer kept as in align_scans."""
+        flat_d, off, fstart, ts, s_ts_d, seg = self._deskew_inputs(raw_scans, trajectory, _device_raw)
+        if flat_d is None:
+            self.last_merged, self.last_frame_off, self.last_export = np.zeros((0, 4)), off, None
+            return FR.split_frames(self.last_merged, off)
+        out, bufs = ops.deskew_slerp(flat_d, self._to_dev(ts), self._to_dev(off), self._to_dev(fstart), s_ts_d, seg,
                                      export=export)
+        self.last_merged, self.last_frame_off, self.last_export = self._to_host(out), off, bufs
+        return FR.split_frames(self.last_merged, off)
+
+    @_trace.traced("LiDARMotionSimulator.deskew_scans_local")
+    def deskew_scans_local(self, raw_scans: List[dict], trajectory: Dict, reference='end',
+                           export: Optional[ops.ExportSpec] = None) -> List[np.ndarray]:
+        """Per-point deskew into the sensor frame of one instant per frame: rotation and translation removed, the
+        product scan registration, odometry and LVX recording expect.  Point times and pose samples as deskew_scans.
+        reference: 'start' (the frame's start time, the MotionCompensator convention), 'end' (the time of the frame's
+        last point; frame start for an empty frame) or an int64 ns array with one entry per frame.  The reference pose
+        is Mode C's pose at that time (ops.slerp_pose_at).  Returns the per-frame sensor-frame clouds; the merged buffer
+        and the export buffers are kept as in align_scans."""
+        bad_ref = ValueError("reference must be 'start', 'end' or an int64 ns array with one entry per frame")
+        if isinstance(reference, str) and reference not in ('start', 'end'):
+            raise bad_ref
+        flat_d, off, fstart, ts, s_ts_d, seg = self._deskew_inputs(raw_scans, trajectory)
+        if flat_d is None:
+            self.last_merged, self.last_frame_off, self.last_export = np.zeros((0, 4)), off, None
+            return FR.split_frames(self.last_merged, off)
+        if isinstance(reference, str):
+            if reference == 'start':
+                ref_ts = fstart
+            else:
+                ref_ts = fstart.copy()
+                full = np.flatnonzero(np.diff(off) > 0)
+                ref_ts[full] = ts[off[full + 1] - 1]
+        else:
+            ref_ts = np.asarray(reference)
+            if ref_ts.shape != (len(raw_scans),) or not np.issubdtype(ref_ts.dtype, np.integer):
+                raise bad_ref
+            ref_ts = ref_ts.astype(np.int64)
+        ref_pose = ops.slerp_pose_at(s_ts_d, seg, self._to_dev(ref_ts))
+        out, bufs = ops.deskew_slerp_local(flat_d, self._to_dev(ts), self._to_dev(off), self._to_dev(fstart), s_ts_d, seg, ref_pose,
+                                           export=export)
         self.last_merged, self.last_frame_off, self.last_export = self._to_host(out), off, bufs
         return FR.split_frames(self.last_merged, off)
 
