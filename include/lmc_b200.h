@@ -211,6 +211,29 @@ int lmc_deskew_slerp_local_f32(const float* pts_n4, const uint32_t* ts_off, cons
                                int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream);
 
 /*
+ * Distortion, the exact inverse of Mode C: every world point W into the sensor frame of Mode C's pose at the point's own
+ * time -- what a sensor moving along the sample table records of a static world
+ * (definition: oracle/lmc_oracle_distort.c::orc_distort_slerp_f64):
+ *   (k, alpha) = Mode C's bracket, end clamps and alpha at ts
+ *   d   = (W - pos_k) - alpha dpos_k       the offset formed before the lerp: world-scale positions never enter the result
+ *   out = rot_{-alpha theta_k}(R_k^T d) ;  out[3] = W[3]        (= R(ts)^T (W - pos(ts)))
+ * lmc_deskew_slerp_* of the output gives W back.  Arguments, layouts, shards and exports as lmc_deskew_slerp_local_*
+ * (no ref_pose); input world points, output raw sensor-frame points (LMC_LVX_TYPE2_OF_INPUT records are of the world
+ * points, LMC_LVX2_OF_OUTPUT records of the raw ones).  Refused (LMC_ERR_INVALID, nothing written): n_peers > 0 or
+ * multicast pointers, n_samples < 1 or >= 2^31.
+ */
+int lmc_distort_slerp_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off,
+                          const int64_t* frame_start, const int64_t* sample_ts, const double* seg,
+                          int64_t n_samples, double* out_n4,
+                          int64_t n_points, int32_t n_frames,
+                          int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream);
+int lmc_distort_slerp_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off,
+                          const int64_t* frame_start, const int64_t* sample_ts, const double* seg,
+                          int64_t n_samples, float* out_n4,
+                          int64_t n_points, int32_t n_frames,
+                          int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream);
+
+/*
  * (a4)/(a5)/(a9)/(a10) stand-alone quantisers (no transform): LivoxLVXWriter._write_point_data_type2
  * LMC:252-272, the LVX2 packer CS:365-374 and the LAS integer packing behind LMC:957-961 /
  * CS:1683-1686.  `ex` selects outputs and modes exactly as in the fused calls; for lvx_mode both
@@ -428,6 +451,9 @@ int lmc_las_pf3_header(int64_t n_points, const double scale[3], const double off
  *          frame_off = cumsum(kept); noise = np.random.normal(0, std, (sum kept, 3)) or NULL)
  *   lmc_scan_emit  -> raw_out (sum kept, 4): rotated xyz (+ noise) and the environment intensity,
  *                     frame-major, ready for lmc_align_rigid_f64.
+ *   lmc_scan_emit_index -> env_idx_out (sum kept) int64: the environment row of every point lmc_scan_emit would emit,
+ *                     in its slot (same compaction and subsample), for a caller that observes the points from other
+ *                     poses (lmc_distort_slerp_f64: each point from the pose at its own time).
  * pos_f3 / R_f9: per-frame sensor position and SciPy rotation matrix (row-major) of the sensor pose.
  */
 #define LMC_SCAN_TILE 256
@@ -441,6 +467,9 @@ int lmc_scan_emit(const double* env_m4, int64_t n_env, const double* pos_f3, con
                   double range_max_sq, const uint8_t* flags, const int32_t* tile_off, const int32_t* n_visible,
                   const int64_t* frame_off, int32_t max_points, const double* noise_n3, double* raw_out_n4,
                   void* stream);
+int lmc_scan_emit_index(const double* env_m4, int64_t n_env, const double* pos_f3, const double* R_f9, int32_t n_frames,
+                        double range_max_sq, const uint8_t* flags, const int32_t* tile_off, const int32_t* n_visible,
+                        const int64_t* frame_off, int32_t max_points, int64_t* env_idx_out, void* stream);
 
 #ifdef __cplusplus
 }

@@ -61,6 +61,8 @@ _SIGNATURES = {
     "lmc_slerp_pose_at": ([vp, vp, i64, vp, i64, vp, vp], ctypes.c_int),
     "lmc_deskew_slerp_local_f64": ([vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
     "lmc_deskew_slerp_local_f32": ([vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
+    "lmc_distort_slerp_f64": ([vp, vp, vp, vp, vp, vp, i64, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
+    "lmc_distort_slerp_f32": ([vp, vp, vp, vp, vp, vp, i64, vp, i64, i32, i64, i64, vp, vp], ctypes.c_int),
     "lmc_quantize_f64": ([vp, i64, vp, vp], ctypes.c_int),
     "lmc_quantize_f32": ([vp, i64, vp, vp], ctypes.c_int),
     "lmc_lvx_v11_build_f64": ([vp, vp, vp, vp, vp, vp, i64, i32, i64, vp, vp], ctypes.c_int),
@@ -92,6 +94,7 @@ _SIGNATURES = {
     "lmc_scan_mark": ([vp, i64, vp, vp, i32, f64, f64, f64, f64, f64, vp, vp, vp, vp, vp], ctypes.c_int),
     "lmc_scan_recount": ([vp, i64, i32, vp, vp, vp], ctypes.c_int),
     "lmc_scan_emit": ([vp, i64, vp, vp, i32, f64, vp, vp, vp, vp, i32, vp, vp, vp], ctypes.c_int),
+    "lmc_scan_emit_index": ([vp, i64, vp, vp, i32, f64, vp, vp, vp, vp, i32, vp, vp], ctypes.c_int),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

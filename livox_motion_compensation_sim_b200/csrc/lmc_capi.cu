@@ -23,7 +23,7 @@ cudaError_t launch_scan_mark(const double* env, int64_t M, const double* pos, co
 cudaError_t launch_scan_recount(const uint8_t* flags, int64_t M, int32_t F, int32_t* tile_off, int32_t* n_visible, cudaStream_t st);
 cudaError_t launch_scan_emit(const double* env, int64_t M, const double* pos, const double* R, int32_t F, double rmax2, const uint8_t* flags,
                              const int32_t* tile_off, const int32_t* n_visible, const int64_t* frame_off, int32_t max_points,
-                             const double* noise, double* out, cudaStream_t st);
+                             const double* noise, double* out, int64_t* idx_out, cudaStream_t st);
 cudaError_t launch_las_pf3(bool f64, const LasParams& L, int parts, cudaStream_t st);
 cudaError_t launch_lvx_v11(bool f64, const void* pts, const int64_t* frame_off, const int64_t* frame_pos, const double* frame_time,
                            const int64_t* frame_id, uint8_t* out, int32_t n_frames, int32_t f_begin, int32_t f_end, int64_t max_frame_points,
@@ -292,6 +292,31 @@ int lmc_deskew_slerp_local_f32(const float* pts_n4, const uint32_t* ts_off, cons
                                float* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
                                const lmc_export* ex, void* stream) {
     LMC_SLERP_LOCAL_BODY(false, ts_off, true)
+}
+
+#define LMC_DISTORT_BODY(F64, TS, NEED_FS)                                                               \
+    lmc::Params P = base_params(pts_n4, out_n4, n_points, n_frames, p_begin, p_end);                     \
+    if (n_samples < 1 || n_samples >= (1LL << 31) || !sample_ts || !seg)                                 \
+        return fail(LMC_ERR_INVALID, "need a sample table of 1 .. 2^31 - 1 rows");                       \
+    if (ex && (ex->n_peers > 0 || ex->mc_out || ex->mc_lvx14))                                           \
+        return fail(LMC_ERR_INVALID, "distortion has no merged-cloud assembly (each point is in its own sensor frame)"); \
+    if (!TS) return fail(LMC_ERR_INVALID, "timestamps are NULL");                                        \
+    if (NEED_FS && !frame_start) return fail(LMC_ERR_INVALID, "frame_start is NULL");                    \
+    if ((reinterpret_cast<uintptr_t>(TS) | reinterpret_cast<uintptr_t>(seg)) & 15u)                      \
+        return fail(LMC_ERR_ALIGN, "timestamps / seg must be 16-byte aligned");                          \
+    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = TS;                                     \
+    P.samp_ts = sample_ts; P.samp_tab = seg; P.n_samp = n_samples;                                       \
+    return run(F64, lmc::kSlerpDistort, P, ex, stream);
+
+int lmc_distort_slerp_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off, const int64_t* frame_start,
+                          const int64_t* sample_ts, const double* seg, int64_t n_samples, double* out_n4,
+                          int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
+    LMC_DISTORT_BODY(true, ts, false)
+}
+int lmc_distort_slerp_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off, const int64_t* frame_start,
+                          const int64_t* sample_ts, const double* seg, int64_t n_samples, float* out_n4,
+                          int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
+    LMC_DISTORT_BODY(false, ts_off, true)
 }
 
 int lmc_quantize_f64(const double* pts_n4, int64_t n_points, const lmc_export* ex, void* stream) {
@@ -588,8 +613,20 @@ int lmc_scan_emit(const double* env_m4, int64_t n_env, const double* pos_f3, con
     if (!env_m4 || !pos_f3 || !R_f9 || !flags || !tile_off || !n_visible || !frame_off || !raw_out_n4) return fail(LMC_ERR_INVALID, "NULL argument");
     if (!aligned32(env_m4) || !aligned32(raw_out_n4)) return fail(LMC_ERR_ALIGN, "environment / output must be 32-byte aligned");
     cudaError_t e = lmc::launch_scan_emit(env_m4, n_env, pos_f3, R_f9, n_frames, range_max_sq, flags, tile_off, n_visible, frame_off, max_points,
-                                          noise_n3, raw_out_n4, static_cast<cudaStream_t>(stream));
+                                          noise_n3, raw_out_n4, nullptr, static_cast<cudaStream_t>(stream));
     return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_scan_emit");
+}
+int lmc_scan_emit_index(const double* env_m4, int64_t n_env, const double* pos_f3, const double* R_f9, int32_t n_frames,
+                        double range_max_sq, const uint8_t* flags, const int32_t* tile_off, const int32_t* n_visible,
+                        const int64_t* frame_off, int32_t max_points, int64_t* env_idx_out, void* stream) {
+    int rc = check_device();
+    if (rc != LMC_OK) return rc;
+    if (n_env < 0 || n_frames < 0 || max_points < 1) return fail(LMC_ERR_INVALID, "bad size / max_points");
+    if (n_frames == 0 || n_env == 0) return LMC_OK;
+    if (!env_m4 || !pos_f3 || !R_f9 || !flags || !tile_off || !n_visible || !frame_off || !env_idx_out) return fail(LMC_ERR_INVALID, "NULL argument");
+    cudaError_t e = lmc::launch_scan_emit(env_m4, n_env, pos_f3, R_f9, n_frames, range_max_sq, flags, tile_off, n_visible, frame_off, max_points,
+                                          nullptr, nullptr, env_idx_out, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_scan_emit (index)");
 }
 
 }  // extern "C"

@@ -326,6 +326,20 @@ __device__ __forceinline__ void slerp_local_apply(const double (&s)[kSegStride],
     o.z = dot_gemm(ref[2], w0, ref[5], w1, ref[8], w2);
     o.w = p.w;
 }
+// Distortion, the inverse of Mode C (definition: oracle/lmc_oracle_distort.c::orc_distort_slerp_f64): the world point into the
+// sensor frame of Mode C's pose at the point's time, R(t)^T (W - x(t)).  The offset from pos_k is formed before the lerp
+// (world-scale magnitudes never enter the result), R_k^T is applied, then the Rodrigues step by -alpha * theta_k.
+template <bool SMALL = false>
+__device__ __forceinline__ void distort_apply(const double (&s)[kSegStride], double alpha, const Pt& p, Pt& o) {
+    const double d0 = __fma_rn(-alpha, s[16], __dsub_rn(p.x, s[9]));
+    const double d1 = __fma_rn(-alpha, s[17], __dsub_rn(p.y, s[10]));
+    const double d2 = __fma_rn(-alpha, s[18], __dsub_rn(p.z, s[11]));
+    const double v0 = dot_gemm(s[0], d0, s[3], d1, s[6], d2);
+    const double v1 = dot_gemm(s[1], d0, s[4], d1, s[7], d2);
+    const double v2 = dot_gemm(s[2], d0, s[5], d1, s[8], d2);
+    slerp_rotate<SMALL>(s, -alpha, v0, v1, v2, o.x, o.y, o.z);
+    o.w = p.w;
+}
 __device__ __forceinline__ void load_pose12(const double* src, double (&m)[12]) {
     const double2* pr = reinterpret_cast<const double2*>(src);
 #pragma unroll
@@ -612,6 +626,20 @@ __device__ __forceinline__ Pt point_eval(const Params& P, int32_t f, bool single
         load_pose12(P.pose_Rt + 12 * (int64_t)f, ref);
         alpha = __dmul_rn(alpha, row[19]);
         slerp_local_apply(row, alpha, ref, in, out);
+    } else if constexpr (MODE == kSlerpDistort) {
+        const int64_t S = P.n_samp;
+        const int64_t t = F64 ? tsraw : tsraw + fs;
+        const Bracket b = bracket_of(P.samp_ts, S, t, t0, rate);
+        int64_t k = b.k; double alpha = 0.0;
+        if (k < 0) k = 0;
+        else if (k >= S - 1) k = S - 1;
+        else alpha = (double)(t - b.tb);
+        double row[kSegStride];
+        const double2* sr = reinterpret_cast<const double2*>(P.samp_tab + kSegStride * k);
+#pragma unroll
+        for (int q = 0; q < kSegStride / 2; ++q) { const double2 v = __ldg(sr + q); row[2 * q] = v.x; row[2 * q + 1] = v.y; }
+        alpha = __dmul_rn(alpha, row[19]);
+        distort_apply(row, alpha, in, out);
     }
     return out;
 }
@@ -721,6 +749,9 @@ struct PointCtx {
                     if constexpr (MODE == kSlerp) {
                         slerp_apply<true>(row, a0, in[0], out[0]);
                         slerp_apply<true>(row, a1, in[1], out[1]);
+                    } else if constexpr (MODE == kSlerpDistort) {
+                        distort_apply<true>(row, a0, in[0], out[0]);
+                        distort_apply<true>(row, a1, in[1], out[1]);
                     } else {                                          // the frame's reference pose row: L1, like R_k / pos_k
                         double ref[12];
                         load_pose12(P.pose_Rt + 12 * (int64_t)f[0], ref);

@@ -9,8 +9,10 @@ namespace lmc {
 
 // kSlerpLocal: Mode C's per-point pose, then into the sensor frame of the frame's reference pose (pose_Rt, one row per
 // frame): every point of a frame in the sensor frame of one instant, rotation and translation removed
-enum Mode : int { kRigid = 0, kGyro = 1, kSlerp = 2, kQuantOnly = 3, kSlerpLocal = 4 };
-constexpr bool slerp_mode(int mode) { return mode == kSlerp || mode == kSlerpLocal; }
+// kSlerpDistort: the inverse of Mode C -- a world point into the sensor frame of Mode C's pose at the point's own time
+// (what a moving sensor records of a static world)
+enum Mode : int { kRigid = 0, kGyro = 1, kSlerp = 2, kQuantOnly = 3, kSlerpLocal = 4, kSlerpDistort = 5 };
+constexpr bool slerp_mode(int mode) { return mode == kSlerp || mode == kSlerpLocal || mode == kSlerpDistort; }
 template <int MODE> inline constexpr bool kSlerpFamily = slerp_mode(MODE);      // (the same, usable in device code)
 
 // One launch = one Params block in constant/param space.
@@ -49,9 +51,10 @@ struct Params {
 // k_stream tile shape (measured on B200, see profiles/): 15 consumer warps + 1 producer warp (512 threads -> 128 registers
 // each).  Mode C on float4 points amortises its per-tile bookkeeping best with 3 point pairs per thread (over a 3-stage
 // ring); everything else runs 2 pairs (f32) / 1 pair (f64) per thread.  (Sensor-frame deskew holds a reference pose row
-// besides Mode C's: with 3 pairs its LVX2 variant spills twice what Mode C's lean variants do, with 2 it spills less.)
+// besides Mode C's: with 3 pairs its LVX2 variant spills twice what Mode C's lean variants do, with 2 it spills less.
+// Distortion holds exactly Mode C's registers and runs Mode C's shape.)
 constexpr int kCW = 15;
-constexpr int stream_pairs_per_thread(bool f64, int mode) { return f64 ? 1 : (mode == kSlerp ? 3 : 2); }
+constexpr int stream_pairs_per_thread(bool f64, int mode) { return f64 ? 1 : ((mode == kSlerp || mode == kSlerpDistort) ? 3 : 2); }
 constexpr int stream_tile_points(bool f64, int mode) { return kCW * 32 * 2 * stream_pairs_per_thread(f64, mode); }   // 960 / 1920 / 2880
 
 // k_stream export variants: the export configuration known at compile time ("lean" kernels) or tested at run time
@@ -89,6 +92,8 @@ inline Plan plan_point_launch(bool f64, int mode, const Params& P, int path, int
     Plan pl;
     if (mode == kSlerpLocal && (P.n_peers > 0 || P.mc_out || P.mc_lvx))
         return refuse_call("sensor-frame deskew has no merged-cloud assembly (each frame is in its own sensor frame)");
+    if (mode == kSlerpDistort && (P.n_peers > 0 || P.mc_out || P.mc_lvx))
+        return refuse_call("distortion has no merged-cloud assembly (each point is in its own sensor frame)");
     const int64_t tp = stream_tile_points(f64, mode);
     pl.tile0 = (P.p_begin / tp) * tp;
     pl.n_tiles = (P.p_end - pl.tile0 + tp - 1) / tp;
@@ -116,6 +121,10 @@ inline Plan plan_point_launch(bool f64, int mode, const Params& P, int path, int
         if (lean_local) pl.ex = lvx2 ? (kExOut | kExLvx | kExLvx2) : kExOut;
         return pl;
     }
+    if (mode == kSlerpDistort) {                            // lean: the raw cloud alone; any export is the generic kernel's
+        if (timed && (f64 || P.frame_start) && mask == kExOut) pl.ex = kExOut;
+        return pl;
+    }
     bool lean = (!peers || mc || pb) && (!lvx2 || mode == kGyro) && (!(mask & kExLas) || (P.las_x && P.las_int));
     if (mode == kSlerp) lean = lean && !P.hold_idx && timed && (f64 || P.frame_start);
     if (mode == kGyro)  lean = lean && timed && P.frame_start;
@@ -134,11 +143,12 @@ template <class Fn>
 auto dispatch_layout_mode(bool f64, int mode, Fn&& fn) {
     using T = std::true_type;
     using F = std::false_type;
-    switch (mode) {                                         // (mode is one of the five Modes: default = kQuantOnly)
+    switch (mode) {                                         // (mode is one of the six Modes: default = kQuantOnly)
     case kRigid: return f64 ? fn(T{}, std::integral_constant<int, kRigid>{}) : fn(F{}, std::integral_constant<int, kRigid>{});
     case kGyro:  return f64 ? fn(T{}, std::integral_constant<int, kGyro>{})  : fn(F{}, std::integral_constant<int, kGyro>{});
     case kSlerp: return f64 ? fn(T{}, std::integral_constant<int, kSlerp>{}) : fn(F{}, std::integral_constant<int, kSlerp>{});
     case kSlerpLocal: return f64 ? fn(T{}, std::integral_constant<int, kSlerpLocal>{}) : fn(F{}, std::integral_constant<int, kSlerpLocal>{});
+    case kSlerpDistort: return f64 ? fn(T{}, std::integral_constant<int, kSlerpDistort>{}) : fn(F{}, std::integral_constant<int, kSlerpDistort>{});
     default:     return f64 ? fn(T{}, std::integral_constant<int, kQuantOnly>{}) : fn(F{}, std::integral_constant<int, kQuantOnly>{});
     }
 }

@@ -18,7 +18,8 @@
 //   k_scan_mark     grid (tile, frame): visibility flag per (frame, env point) + per-tile counts
 //   k_scan_count    grid (tile, frame): per-tile counts again from (host-patched) flags
 //   k_scan_offsets  grid (frame): exclusive scan of the tile counts, visible total per frame
-//   k_scan_emit     grid (tile, frame): compaction rank -> subsample rule -> rotated xyz (+ noise), intensity
+//   k_scan_emit     grid (tile, frame): compaction rank -> subsample rule -> rotated xyz (+ noise), intensity; or (<true>) the
+//                   environment row index of every emitted point
 #include "lmc_device.cuh"
 
 namespace lmc {
@@ -110,11 +111,14 @@ __global__ void k_scan_offsets(int32_t* __restrict__ tile_off, int tiles, int32_
     n_visible[f] = acc;
 }
 
+// IDX = false: raw_out rows (rotated xyz + noise, intensity).  IDX = true: the environment row of every emitted point instead
+// (idx_out[o] = i), the same compaction and subsample -- for the caller that re-observes the points from other poses.
+template <bool IDX>
 __global__ void __launch_bounds__(kScanTile) k_scan_emit(const double* __restrict__ env, int64_t M, const double* __restrict__ pos_f3,
                                                          const double* __restrict__ R_f9, double rmax2, const uint8_t* __restrict__ flags,
                                                          const int32_t* __restrict__ tile_off, int tiles, const int32_t* __restrict__ n_visible,
                                                          const int64_t* __restrict__ frame_off, int32_t max_points,
-                                                         const double* __restrict__ noise, double* __restrict__ out) {
+                                                         const double* __restrict__ noise, double* __restrict__ out, int64_t* __restrict__ idx_out) {
     __shared__ int s_warp[kScanTile / 32];
     const int f = blockIdx.y;
     const int64_t i = (int64_t)blockIdx.x * kScanTile + threadIdx.x;
@@ -131,12 +135,16 @@ __global__ void __launch_bounds__(kScanTile) k_scan_emit(const double* __restric
         o = j / step;
     }
     o += frame_off[f];
-    const ScanGeom g = scan_geom(env, i, pos_f3 + 3 * f, R_f9 + 9 * f, rmax2);
-    double nx = 0.0, ny = 0.0, nz = 0.0;
-    if (noise != nullptr) { nx = noise[3 * o]; ny = noise[3 * o + 1]; nz = noise[3 * o + 2]; }
-    const double w = env[4 * i + 3];
-    if (noise != nullptr) stg256(out + 4 * o, __dadd_rn(g.x, nx), __dadd_rn(g.y, ny), __dadd_rn(g.z, nz), w);   // LMC:768 visible_points += noise
-    else                  stg256(out + 4 * o, g.x, g.y, g.z, w);
+    if constexpr (IDX) {
+        idx_out[o] = i;
+    } else {
+        const ScanGeom g = scan_geom(env, i, pos_f3 + 3 * f, R_f9 + 9 * f, rmax2);
+        double nx = 0.0, ny = 0.0, nz = 0.0;
+        if (noise != nullptr) { nx = noise[3 * o]; ny = noise[3 * o + 1]; nz = noise[3 * o + 2]; }
+        const double w = env[4 * i + 3];
+        if (noise != nullptr) stg256(out + 4 * o, __dadd_rn(g.x, nx), __dadd_rn(g.y, ny), __dadd_rn(g.z, nz), w);   // LMC:768 visible_points += noise
+        else                  stg256(out + 4 * o, g.x, g.y, g.z, w);
+    }
 }
 
 // grid.y carries the frame index (<= 65535 per launch): longer runs go in frame chunks
@@ -171,15 +179,21 @@ cudaError_t launch_scan_recount(const uint8_t* flags, int64_t M, int32_t F, int3
 
 cudaError_t launch_scan_emit(const double* env, int64_t M, const double* pos, const double* R, int32_t F, double rmax2, const uint8_t* flags,
                              const int32_t* tile_off, const int32_t* n_visible, const int64_t* frame_off, int32_t max_points,
-                             const double* noise, double* out, cudaStream_t st) {
+                             const double* noise, double* out, int64_t* idx_out, cudaStream_t st) {
     const int64_t tiles = (M + kScanTile - 1) / kScanTile;
     if (tiles == 0) return cudaSuccess;
     if (tiles > 0x7fffffffLL) return cudaErrorInvalidValue;
     for (int32_t f0 = 0; f0 < F; f0 += kScanMaxFramesPerLaunch) {
         const int nf = F - f0 < kScanMaxFramesPerLaunch ? F - f0 : kScanMaxFramesPerLaunch;
-        k_scan_emit<<<dim3((unsigned)tiles, (unsigned)nf), kScanTile, 0, st>>>(env, M, pos + 3 * (int64_t)f0, R + 9 * (int64_t)f0, rmax2, flags + (int64_t)f0 * M,
-                                                                              tile_off + (int64_t)f0 * (tiles + 1), (int)tiles, n_visible + f0, frame_off + f0,
-                                                                              max_points, noise, out);
+        const dim3 grid((unsigned)tiles, (unsigned)nf);
+        if (idx_out != nullptr)
+            k_scan_emit<true><<<grid, kScanTile, 0, st>>>(env, M, pos + 3 * (int64_t)f0, R + 9 * (int64_t)f0, rmax2, flags + (int64_t)f0 * M,
+                                                          tile_off + (int64_t)f0 * (tiles + 1), (int)tiles, n_visible + f0, frame_off + f0,
+                                                          max_points, nullptr, nullptr, idx_out);
+        else
+            k_scan_emit<false><<<grid, kScanTile, 0, st>>>(env, M, pos + 3 * (int64_t)f0, R + 9 * (int64_t)f0, rmax2, flags + (int64_t)f0 * M,
+                                                           tile_off + (int64_t)f0 * (tiles + 1), (int)tiles, n_visible + f0, frame_off + f0,
+                                                           max_points, noise, out, nullptr);
     }
     return cudaGetLastError();
 }

@@ -26,7 +26,7 @@ constexpr int kStreamThreads = 32 * (kCW + 1);           // + producer warp
 // tile shape: lmc_plan.h (the launch plan sizes the grid with the same tile)
 template <bool F64, int MODE> struct StreamCfg {
     static constexpr int PPT      = stream_pairs_per_thread(F64, MODE);   // point pairs per consumer thread per tile
-    static constexpr int STAGES   = (!F64 && MODE == kSlerp) ? 3 : 4;
+    static constexpr int STAGES   = (!F64 && (MODE == kSlerp || MODE == kSlerpDistort)) ? 3 : 4;
     static constexpr int TP       = stream_tile_points(F64, MODE);
     static constexpr int PT_BYTES = F64 ? 32 : 16;
     static constexpr int TS_BYTES = F64 ? 8 : 4;
@@ -450,14 +450,20 @@ template <bool F64, int EX>
 __global__ void __launch_bounds__(kStreamThreads, 1) k_local_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles) {
     stream_body<F64, kSlerpLocal, EX>(P, tile0, n_tiles);
 }
+// distortion (kSlerpDistort) under its own name
+template <bool F64, int EX>
+__global__ void __launch_bounds__(kStreamThreads, 1) k_distort_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles) {
+    stream_body<F64, kSlerpDistort, EX>(P, tile0, n_tiles);
+}
 
 // ---- launcher ----------------------------------------------------------------------------------
 template <bool F64, int MODE, int EX>
 static cudaError_t launch_stream_ex(const Params& P, const Plan& pl, int dev, cudaStream_t st) {
     using Cfg = StreamCfg<F64, MODE>;
     void (*kern)(const Params, int64_t, int64_t);
-    if constexpr (MODE == kSlerpLocal) kern = k_local_stream<F64, EX>;
-    else                               kern = k_stream<F64, MODE, EX>;
+    if constexpr (MODE == kSlerpLocal)        kern = k_local_stream<F64, EX>;
+    else if constexpr (MODE == kSlerpDistort) kern = k_distort_stream<F64, EX>;
+    else                                      kern = k_stream<F64, MODE, EX>;
     static thread_local int attr_dev = -1;
     if (attr_dev != dev) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
@@ -476,6 +482,8 @@ cudaError_t launch_stream(bool f64, int mode, const Params& P, const Plan& pl, i
         if constexpr (MODE == kSlerpLocal) {
             if (pl.ex == kExOut)                    return launch_stream_ex<F64, MODE, kExOut>(P, pl, dev, st);
             if (pl.ex == (kExOut | kExLvx | kExLvx2)) return launch_stream_ex<F64, MODE, kExOut | kExLvx | kExLvx2>(P, pl, dev, st);
+        } else if constexpr (MODE == kSlerpDistort) {
+            if (pl.ex == kExOut)                    return launch_stream_ex<F64, MODE, kExOut>(P, pl, dev, st);
         } else if constexpr (MODE != kQuantOnly) {
             switch (pl.ex) {
             case kExOut:           return launch_stream_ex<F64, MODE, kExOut>(P, pl, dev, st);

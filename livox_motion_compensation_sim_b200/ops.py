@@ -259,6 +259,27 @@ def deskew_slerp_local(pts: torch.Tensor, ts: torch.Tensor, frame_off: torch.Ten
 
 
 @_on_tensor_device
+def distort_slerp(pts: torch.Tensor, ts: torch.Tensor, frame_off: torch.Tensor, frame_start: Optional[torch.Tensor],
+                  sample_ts: torch.Tensor, seg: torch.Tensor, *, out: Optional[torch.Tensor] = None,
+                  export: Optional[ExportSpec] = None, p_range=None, want_out: bool = True):
+    """Distortion, the exact inverse of deskew_slerp: every WORLD point into the sensor frame of Mode C's pose at the
+    point's own time, R(t)^T (W - x(t)) -- what a sensor moving along the sample table records of a static world.
+    Arguments as deskew_slerp_local (no ref_pose); deskew_slerp of the result gives the world points back."""
+    f64 = _layout(pts)
+    n, F = pts.shape[0], frame_off.shape[0] - 1
+    if out is None and want_out:
+        out = torch.empty_like(pts)
+    ex, bufs = _make_export(export, n, pts.device)
+    b, e = _range(n, p_range)
+    fn = C.lib().lmc_distort_slerp_f64 if f64 else C.lib().lmc_distort_slerp_f32
+    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(ts, torch.int64 if f64 else torch.uint32, "ts"),
+               _req(frame_off, torch.int64, "frame_off"), _req(frame_start, torch.int64, "frame_start"),
+               _req(sample_ts, torch.int64, "sample_ts"), _req(seg, torch.float64, "seg", (22,)), sample_ts.shape[0],
+               _req(out, pts.dtype, "out", (4,)), n, F, b, e, None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
+    return out, bufs
+
+
+@_on_tensor_device
 def quantize(pts: torch.Tensor, export: ExportSpec) -> ExportBuffers:
     """(a4)/(a5)/(a9)/(a10) stand-alone quantisers over an (N,4) point array."""
     f64 = _layout(pts)
@@ -515,9 +536,15 @@ def _redecide_uncertain(env, pos, Rm, flags, fov_h, fov_v, range_min) -> int:
 @_on_tensor_device
 def scan_frames(env: torch.Tensor, pos: torch.Tensor, Rm: torch.Tensor, *, range_max: float, range_min: float,
                 fov_horizontal: float, fov_vertical: float, points_per_frame: int, noise_std: float, noise_fn=None,
-                max_flag_bytes: int = 1 << 30, edge_eps_deg: float = 1e-9):
+                max_flag_bytes: int = 1 << 30, edge_eps_deg: float = 1e-9, motion=None):
     """(N4) LMC:701-770 for every frame at once.  env (M,4) f64, pos (F,3), Rm (F,9) row-major SciPy matrices.
     Returns (raw (N,4) f64 device tensor, frame_off np.int64[F+1]).
+
+    motion = (sample_ts, seg, frame_start, period_ns) (device int64 sample times, the (S,22) table of build_slerp_table,
+    host int64[F] frame start times, the frame period in ns) simulates a moving sensor: which points a frame sees is
+    still decided at pos[f] / Rm[f], but point j of the m_f kept points of frame f is observed at time
+    frame_start[f] + (j * period_ns) // m_f from Mode C's pose there (distort_slerp), and the same noise is added in that
+    sensor frame.  Returns (raw, frame_off, point times np.int64[N], env row indices (N) int64 device tensor) then.
 
     noise_fn(n) must return the (n,3) host array the reference would draw -- by default
     ``np.random.normal(0, noise_std, (n, 3))`` from the GLOBAL legacy NumPy RNG (replayed bit-identically by
@@ -538,7 +565,13 @@ def scan_frames(env: torch.Tensor, pos: torch.Tensor, Rm: torch.Tensor, *, range
     L = C.lib()
     _req(env, torch.float64, "env", (4,)); _req(pos, torch.float64, "pos", (3,)); _req(Rm, torch.float64, "Rm", (9,))
     chunk = max(1, min(F, max_flag_bytes // max(M, 1)))
-    outs, kept_all = [], []
+    outs, kept_all, idx_all, ts_all = [], [], [], []
+    if motion is not None:
+        s_ts, seg, fstart, period_ns = motion
+        fstart = np.asarray(fstart, np.int64)
+        if fstart.shape != (F,):
+            raise ValueError("motion: frame_start needs one entry per frame")
+        _req(s_ts, torch.int64, "sample_ts"); _req(seg, torch.float64, "seg", (22,))
     for f0 in range(0, F, chunk):
         f1 = min(F, f0 + chunk)
         nf = f1 - f0
@@ -575,12 +608,33 @@ def scan_frames(env: torch.Tensor, pos: torch.Tensor, Rm: torch.Tensor, *, range
                 else:
                     noise_d = torch.from_numpy(np.ascontiguousarray(noise_fn(n_c), dtype=np.float64)).to(dev)
             fo = torch.from_numpy(off_c).to(dev)
-            C.check(L.lmc_scan_emit(env.data_ptr(), M, p_c.data_ptr(), r_c.data_ptr(), nf, rmax2, flags.data_ptr(), tile_off.data_ptr(),
-                                    n_vis.data_ptr(), fo.data_ptr(), maxp, _req(noise_d, torch.float64, "noise", (3,)), out.data_ptr(), _stream_ptr()))
+            if motion is None:
+                C.check(L.lmc_scan_emit(env.data_ptr(), M, p_c.data_ptr(), r_c.data_ptr(), nf, rmax2, flags.data_ptr(), tile_off.data_ptr(),
+                                        n_vis.data_ptr(), fo.data_ptr(), maxp, _req(noise_d, torch.float64, "noise", (3,)), out.data_ptr(), _stream_ptr()))
+            else:
+                idx = torch.empty(n_c, dtype=torch.int64, device=dev)
+                C.check(L.lmc_scan_emit_index(env.data_ptr(), M, p_c.data_ptr(), r_c.data_ptr(), nf, rmax2, flags.data_ptr(), tile_off.data_ptr(),
+                                              n_vis.data_ptr(), fo.data_ptr(), maxp, idx.data_ptr(), _stream_ptr()))
+                m = np.diff(off_c)
+                fidx = np.repeat(np.arange(nf), m)
+                j = np.arange(n_c, dtype=np.int64) - off_c[fidx]
+                ts_c = fstart[f0 + fidx] + (j * int(period_ns)) // m[fidx]       # the point-time convention of the deskews
+                distort_slerp(env[idx], torch.from_numpy(ts_c).to(dev), fo, None, s_ts, seg, out=out)
+                if noise_d is not None:
+                    out[:, :3] += noise_d                                        # LMC:768, in the sensor frame of the point's pose
+                idx_all.append(idx)
+                ts_all.append(ts_c)
+        elif motion is not None:
+            idx_all.append(torch.empty(0, dtype=torch.int64, device=dev))
+            ts_all.append(np.zeros(0, np.int64))
         outs.append(out)
         kept_all.append(kept)
     kept_all = np.concatenate(kept_all) if kept_all else np.zeros(0, np.int64)
     frame_off = np.zeros(F + 1, np.int64)
     np.cumsum(kept_all, out=frame_off[1:])
     raw = outs[0] if len(outs) == 1 else (torch.cat(outs, dim=0) if outs else torch.empty((0, 4), dtype=torch.float64, device=dev))
-    return raw, frame_off
+    if motion is None:
+        return raw, frame_off
+    env_idx = torch.cat(idx_all) if idx_all else torch.empty(0, dtype=torch.int64, device=dev)
+    point_ts = np.concatenate(ts_all) if ts_all else np.zeros(0, np.int64)
+    return raw, frame_off, point_ts, env_idx

@@ -59,6 +59,14 @@ class LiDARMotionSimulator:
             # 'hold_next' = the reference's per-frame pose (LMC:802-812); 'slerp' = per-point deskew: every point's
             # timestamp is bracketed in the trajectory samples, orientation SLERPed, position lerped (north_star Mode C)
             'pose_interpolation': 'hold_next',
+            # False (default): the device scanner sees every point of a frame from the frame's hold-next pose, as the
+            # reference does.  True: a moving sensor -- point j of a frame's m kept points is observed at frame time +
+            # j * period / m from the pose interpolated there (Mode C's pose: SLERP + lerp of the trajectory samples), so
+            # the raw scans carry the motion distortion the deskews remove; every raw scan dict gains 'point_times' (int64
+            # ns) and 'env_index' (its environment rows).  Which points a frame sees is still decided at the hold-next pose,
+            # so the point sets and the NumPy noise stream are the reference's.  Needs the device scanner (a frame_source
+            # without .scan).
+            'motion_distortion': False,
             # False (default): results are ordinary NumPy arrays -- D2H into one reusable pinned staging buffer, then a threaded
             # copy (lmc_host_copy); nothing stays page-locked behind the caller's back.
             # True: opt-in throughput knob -- results ARE page-locked blocks of torch's caching host allocator (no second copy:
@@ -142,18 +150,22 @@ class LiDARMotionSimulator:
 
     # ------------------------------------------------------------------ (N4) LMC:701-770
     @_trace.traced("LiDARMotionSimulator.scan_all")
-    def scan_all(self, environment, positions, eulers, keep_device: bool = False) -> List[np.ndarray]:
+    def scan_all(self, environment, positions, eulers, keep_device: bool = False, motion=None) -> List[np.ndarray]:
         """scan_environment for every frame in ONE device pass (range / FOV cull, compaction, subsample);
         the noise is drawn on the host from the global NumPy RNG exactly as LMC:767 does, so a seeded
-        run reproduces the reference's raw scans.  Returns the per-frame (n_f,4) arrays."""
+        run reproduces the reference's raw scans.  Returns the per-frame (n_f,4) arrays.
+        motion: ops.scan_frames' motion argument (each point observed from the pose at its own time); the point times and
+        environment rows are then kept in self.last_scan_motion = (point_times np.int64[N], env_index np.int64[N])."""
         from scipy.spatial.transform import Rotation
         positions = np.asarray(positions, np.float64).reshape(-1, 3)
         Rm = Rotation.from_euler('xyz', np.asarray(eulers, np.float64).reshape(-1, 3)).as_matrix().reshape(-1, 9)   # LMC:726
         c = self.config
-        raw, off = ops.scan_frames(self._to_dev(np.asarray(environment, np.float64)), self._to_dev(positions), self._to_dev(Rm),
-                                   range_max=c['range_max'], range_min=c['range_min'], fov_horizontal=c['fov_horizontal'],
-                                   fov_vertical=c['fov_vertical'], points_per_frame=c['points_per_frame'],
-                                   noise_std=c['lidar_range_noise'])
+        res = ops.scan_frames(self._to_dev(np.asarray(environment, np.float64)), self._to_dev(positions), self._to_dev(Rm),
+                              range_max=c['range_max'], range_min=c['range_min'], fov_horizontal=c['fov_horizontal'],
+                              fov_vertical=c['fov_vertical'], points_per_frame=c['points_per_frame'],
+                              noise_std=c['lidar_range_noise'], motion=motion)
+        raw, off = res[0], res[1]
+        self.last_scan_motion = (res[2], res[3].cpu().numpy()) if motion is not None else None
         self._dev_scan = (raw, off) if keep_device else None      # run_simulation aligns the device copy directly
         host = self._to_host(raw)
         return [host[off[i]:off[i + 1]] if off[i + 1] > off[i] else np.array([]).reshape(0, 4) for i in range(len(off) - 1)]
@@ -196,12 +208,19 @@ class LiDARMotionSimulator:
           .scan(i, t, sensor_pose)   -> (n,4) f64 raw sensor-frame points   (LMC:701-770); if absent,
                                         .environment is scanned on the device for all frames at once (N4)
           .environment               -> (M,4) f64 world cloud (needed when .scan is absent)
+        With config 'motion_distortion' the device scanner observes every point from the pose at its own time (see
+        default_config) and every raw scan dict carries 'point_times' and 'env_index'; alignment_error then measures what
+        the alignment leaves of that distortion.
         Returns the reference's results dict (LMC:852-858)."""
         if frame_source is None:
             raise NotImplementedError(
                 "trajectory / environment / scanner generators are outside the accelerated hot path "
                 "(SURVEY.md section 2 rows 8-11); pass a frame_source, or mix this class into the "
                 "reference's LiDARMotionSimulator as shown in INTEGRATION.md")
+        distort = bool(self.config.get('motion_distortion', False))
+        if distort and hasattr(frame_source, 'scan'):
+            raise ValueError("motion_distortion needs the device scanner: a frame_source with its own .scan has no environment "
+                             "rows to observe from other poses")
         trajectory = frame_source.trajectory
         lidar_times = FR.lidar_frame_times(self.config['duration'], self.config['lidar_fps'])
         _, pose_idx = self.lookup_frame_poses(trajectory, lidar_times)
@@ -209,8 +228,15 @@ class LiDARMotionSimulator:
         all_scans, motion_data = [], []
         device_scans = None
         if not hasattr(frame_source, 'scan'):           # no host scanner supplied: scan every frame on the device (N4)
+            motion = None
+            if distort:                                 # the pose samples the deskews read (_deskew_inputs), one table
+                s_ts_d, seg = self._slerp_samples(trajectory)
+                motion = (s_ts_d, seg, np.round(np.asarray(lidar_times, np.float64) * 1e9).astype(np.int64),
+                          int(round(1e9 / float(self.config['lidar_fps']))))
             device_scans = self.scan_all(frame_source.environment, trajectory['position_gps'][pose_idx],
-                                         trajectory['orientation_imu'][pose_idx], keep_device=True)
+                                         trajectory['orientation_imu'][pose_idx], keep_device=True, motion=motion)
+        scan_motion = getattr(self, 'last_scan_motion', None) if distort else None
+        scan_off = self._dev_scan[1] if scan_motion is not None else None
         for i, t in enumerate(lidar_times):
             k = int(pose_idx[i])
             sensor_pose = {'position': trajectory['position_gps'][k],
@@ -218,11 +244,14 @@ class LiDARMotionSimulator:
                            'velocity': trajectory['velocity'][k]}
             scan = device_scans[i] if device_scans is not None else frame_source.scan(i, t, sensor_pose)
             all_scans.append({'frame_id': i, 'timestamp': t, 'points_local': scan, 'sensor_pose': sensor_pose})
+            if scan_motion is not None:
+                a, b = int(scan_off[i]), int(scan_off[i + 1])
+                all_scans[-1]['point_times'], all_scans[-1]['env_index'] = scan_motion[0][a:b], scan_motion[1][a:b]
             motion_data.append(self._motion_row(i, t, sensor_pose))
         dev_scan = getattr(self, '_dev_scan', None) if device_scans is not None else None
         self._dev_scan = None
         if self.config.get('pose_interpolation', 'hold_next') == 'slerp':
-            aligned = self.deskew_scans(all_scans, trajectory, _device_raw=dev_scan)
+            aligned = self.deskew_scans(all_scans, trajectory, _device_raw=dev_scan, _samples=motion[:2] if distort else None)
         elif dev_scan is not None and self._np_dtype() == np.float64 and dev_scan[0].shape[0] > 0:
             # the scans are still resident: align them where they are (no flatten, no second upload)
             raw_d, off = dev_scan
@@ -257,10 +286,19 @@ class LiDARMotionSimulator:
         self.last_merged, self.last_frame_off, self.last_export = merged, off, bufs
         return FR.split_frames(merged, off)
 
-    def _deskew_inputs(self, raw_scans: List[dict], trajectory: Dict, _device_raw=None):
+    def _slerp_samples(self, trajectory: Dict):
+        """The pose samples of Mode C on the device: the trajectory's GPS positions / IMU orientations at their own times
+        -> (int64 ns sample times, the (S,22) pose-segment table)."""
+        from scipy.spatial.transform import Rotation
+        s_ts = np.round(np.asarray(trajectory['time'], np.float64) * 1e9).astype(np.int64)
+        quat = Rotation.from_euler('xyz', np.asarray(trajectory['orientation_imu'], np.float64)).as_quat()
+        s_ts_d = self._to_dev(s_ts)
+        seg = ops.build_slerp_table(self._to_dev(quat), self._to_dev(np.asarray(trajectory['position_gps'], np.float64)), s_ts_d)
+        return s_ts_d, seg
+
+    def _deskew_inputs(self, raw_scans: List[dict], trajectory: Dict, _device_raw=None, _samples=None):
         """The per-point times and the pose-segment table both deskews need: (flat points on the device, frame offsets,
         frame starts, int64 ns point times, sample times, seg) -- None for the device arrays when there are no points."""
-        from scipy.spatial.transform import Rotation
         if _device_raw is not None:                                 # scans still resident on the device (run_simulation)
             flat_d, off = _device_raw
         else:
@@ -279,20 +317,18 @@ class LiDARMotionSimulator:
             if m:
                 pt = s.get('point_times')
                 ts[off[i]:off[i + 1]] = pt if pt is not None else fstart[i] + (np.arange(m, dtype=np.int64) * period_ns) // m
-        s_ts = np.round(np.asarray(trajectory['time'], np.float64) * 1e9).astype(np.int64)
-        quat = Rotation.from_euler('xyz', np.asarray(trajectory['orientation_imu'], np.float64)).as_quat()
-        seg = ops.build_slerp_table(self._to_dev(quat), self._to_dev(np.asarray(trajectory['position_gps'], np.float64)), self._to_dev(s_ts))
-        return flat_d, off, fstart, ts, self._to_dev(s_ts), seg
+        s_ts_d, seg = self._slerp_samples(trajectory) if _samples is None else _samples
+        return flat_d, off, fstart, ts, s_ts_d, seg
 
     @_trace.traced("LiDARMotionSimulator.deskew_scans")
     def deskew_scans(self, raw_scans: List[dict], trajectory: Dict, export: Optional[ops.ExportSpec] = None,
-                     _device_raw=None) -> List[np.ndarray]:
+                     _device_raw=None, _samples=None) -> List[np.ndarray]:
         """Per-point deskew + alignment (north_star Mode C; the reference has no such step -- parity is against the
         builder's SciPy Slerp + lerp oracle).  Pose samples = the trajectory's GPS positions / IMU orientations at
         their own times (LMC:396-428); a point's time is ``scan['point_times']`` (int64 ns) when the scan dict has
         it, else frame time + i * (frame period / n_f) (SURVEY 8d M-C3).  Points outside the sample span hold the
         end pose.  Returns the per-frame world clouds; merged buffer kept as in align_scans."""
-        flat_d, off, fstart, ts, s_ts_d, seg = self._deskew_inputs(raw_scans, trajectory, _device_raw)
+        flat_d, off, fstart, ts, s_ts_d, seg = self._deskew_inputs(raw_scans, trajectory, _device_raw, _samples)
         if flat_d is None:
             self.last_merged, self.last_frame_off, self.last_export = np.zeros((0, 4)), off, None
             return FR.split_frames(self.last_merged, off)
@@ -334,6 +370,29 @@ class LiDARMotionSimulator:
                                            export=export)
         self.last_merged, self.last_frame_off, self.last_export = self._to_host(out), off, bufs
         return FR.split_frames(self.last_merged, off)
+
+    def alignment_error(self, results) -> Dict:
+        """How far the aligned clouds of a run are from the environment points they observed: |aligned_i - env[env_index_i]|
+        (Euclidean, metres) over every point, on the device.  Needs a run with 'motion_distortion' (the raw scans carry
+        'env_index').  Returns {'max_m', 'rms_m', 'per_frame_max_m'} (per-frame list; 0.0 for an empty frame)."""
+        scans = results['raw_scans']
+        if not scans or any(s.get('env_index') is None for s in scans):
+            raise ValueError("alignment_error needs the environment rows of the raw points: run with 'motion_distortion': True")
+        aligned = results['aligned_pointclouds']
+        off = FR.frame_offsets(aligned)
+        if not np.array_equal(off, FR.frame_offsets([s['env_index'] for s in scans])):
+            raise ValueError("aligned clouds and raw scans differ in their point counts")
+        n = int(off[-1])
+        if n == 0:
+            return {'max_m': 0.0, 'rms_m': 0.0, 'per_frame_max_m': [0.0] * len(scans)}
+        flat, _ = FR.flatten_frames([np.asarray(a).reshape(-1, 4) for a in aligned], np.float64)
+        idx = self._to_dev(np.concatenate([np.asarray(s['env_index'], np.int64) for s in scans]))
+        env = self._to_dev(np.asarray(results['environment'], np.float64))
+        err = torch.linalg.vector_norm(self._to_dev(flat)[:, :3] - env[idx, :3], dim=1)
+        fidx = self._to_dev(np.repeat(np.arange(len(scans)), np.diff(off)))
+        per = torch.zeros(len(scans), dtype=torch.float64, device=self.device).scatter_reduce(0, fidx, err, 'amax')
+        return {'max_m': float(err.max().item()), 'rms_m': float(torch.sqrt(torch.mean(err * err)).item()),
+                'per_frame_max_m': per.cpu().numpy().tolist()}
 
     # ------------------------------------------------------------------ (a3) LMC:886-899
     def _merge_flags(self, results):
