@@ -194,64 +194,82 @@ int lmc_build_slerp_table(const double* sample_quat_xyzw, const double* sample_p
     return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_slerp_table");
 }
 
-#define LMC_RIGID_BODY(F64)                                                                              \
-    lmc::Params P = base_params(pts_n4, out_n4, n_points, n_frames, p_begin, p_end);                     \
-    if (!pose_Rt) return fail(LMC_ERR_INVALID, "pose_Rt is NULL");                                       \
-    if (reinterpret_cast<uintptr_t>(pose_Rt) & 15u) return fail(LMC_ERR_ALIGN, "pose_Rt must be 16-byte aligned"); \
-    P.frame_off = frame_off; P.pose_Rt = pose_Rt;                                                        \
-    return run(F64, lmc::kRigid, P, ex, stream);
-
+static int align_rigid(bool f64, const void* pts, const int64_t* frame_off, const double* pose_Rt, void* out,
+                       int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
+    lmc::Params P = base_params(pts, out, n_points, n_frames, p_begin, p_end);
+    if (!pose_Rt) return fail(LMC_ERR_INVALID, "pose_Rt is NULL");
+    if (reinterpret_cast<uintptr_t>(pose_Rt) & 15u) return fail(LMC_ERR_ALIGN, "pose_Rt must be 16-byte aligned");
+    P.frame_off = frame_off; P.pose_Rt = pose_Rt;
+    return run(f64, lmc::kRigid, P, ex, stream);
+}
 int lmc_align_rigid_f64(const double* pts_n4, const int64_t* frame_off, const double* pose_Rt, double* out_n4,
                         int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
-    LMC_RIGID_BODY(true)
+    return align_rigid(true, pts_n4, frame_off, pose_Rt, out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 int lmc_align_rigid_f32(const float* pts_n4, const int64_t* frame_off, const double* pose_Rt, float* out_n4,
                         int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
-    LMC_RIGID_BODY(false)
+    return align_rigid(false, pts_n4, frame_off, pose_Rt, out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 
-#define LMC_GYRO_BODY(F64, TS)                                                                           \
-    lmc::Params P = base_params(pts_n4, out_n4, n_points, n_frames, p_begin, p_end);                     \
-    if (n_imu < 0) return fail(LMC_ERR_INVALID, "n_imu < 0");                                            \
-    if (!TS || !frame_start) return fail(LMC_ERR_INVALID, "timestamps / frame_start are NULL");          \
-    if (n_imu > 0 && (!imu_ts || !imu_gyro)) return fail(LMC_ERR_INVALID, "imu tables are NULL");        \
-    if (reinterpret_cast<uintptr_t>(TS) & 15u) return fail(LMC_ERR_ALIGN, "timestamps must be 16-byte aligned"); \
-    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = TS;                                     \
-    P.samp_ts = imu_ts; P.samp_tab = imu_gyro; P.n_samp = n_imu;                                         \
-    return run(F64, lmc::kGyro, P, ex, stream);
-
+static int deskew_gyro(bool f64, const void* pts, const void* ts, const int64_t* frame_off, const int64_t* frame_start,
+                       const int64_t* imu_ts, const double* imu_gyro, int64_t n_imu, void* out,
+                       int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
+    lmc::Params P = base_params(pts, out, n_points, n_frames, p_begin, p_end);
+    if (n_imu < 0) return fail(LMC_ERR_INVALID, "n_imu < 0");
+    if (!ts || !frame_start) return fail(LMC_ERR_INVALID, "timestamps / frame_start are NULL");
+    if (n_imu > 0 && (!imu_ts || !imu_gyro)) return fail(LMC_ERR_INVALID, "imu tables are NULL");
+    if (reinterpret_cast<uintptr_t>(ts) & 15u) return fail(LMC_ERR_ALIGN, "timestamps must be 16-byte aligned");
+    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = ts;
+    P.samp_ts = imu_ts; P.samp_tab = imu_gyro; P.n_samp = n_imu;
+    return run(f64, lmc::kGyro, P, ex, stream);
+}
 int lmc_deskew_gyro_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off, const int64_t* frame_start,
                         const int64_t* imu_ts, const double* imu_gyro, int64_t n_imu, double* out_n4,
                         int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
-    LMC_GYRO_BODY(true, ts)
+    return deskew_gyro(true, pts_n4, ts, frame_off, frame_start, imu_ts, imu_gyro, n_imu, out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 int lmc_deskew_gyro_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off, const int64_t* frame_start,
                         const int64_t* imu_ts, const double* imu_gyro, int64_t n_imu, float* out_n4,
                         int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
-    LMC_GYRO_BODY(false, ts_off)
+    return deskew_gyro(false, pts_n4, ts_off, frame_off, frame_start, imu_ts, imu_gyro, n_imu, out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 
-#define LMC_SLERP_BODY(F64, TS, NEED_FS)                                                                 \
-    lmc::Params P = base_params(pts_n4, out_n4, n_points, n_frames, p_begin, p_end);                     \
-    if (n_samples < 1 || !sample_ts || !seg) return fail(LMC_ERR_INVALID, "need a non-empty sample table"); \
-    if (!hold_idx && !TS) return fail(LMC_ERR_INVALID, "timestamps are NULL");                           \
-    if (!hold_idx && NEED_FS && !frame_start) return fail(LMC_ERR_INVALID, "frame_start is NULL");       \
-    if ((reinterpret_cast<uintptr_t>(TS) | reinterpret_cast<uintptr_t>(seg)) & 15u) return fail(LMC_ERR_ALIGN, "timestamps / seg must be 16-byte aligned"); \
-    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = TS;                                     \
-    P.samp_ts = sample_ts; P.samp_tab = seg; P.n_samp = n_samples; P.hold_idx = hold_idx;                \
-    return run(F64, lmc::kSlerp, P, ex, stream);
-
+// Mode C (kSlerp, with the optional hold_idx), sensor-frame deskew (kSlerpLocal, with ref_pose) and distortion (kSlerpDistort).
+// f32 points carry ns offsets from their frame's start, so they need frame_start.
+static int slerp_family(bool f64, int mode, const void* pts, const void* ts, const int64_t* frame_off, const int64_t* frame_start,
+                        const int64_t* sample_ts, const double* seg, int64_t n_samples, const int32_t* hold_idx, const double* ref_pose,
+                        void* out, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
+    lmc::Params P = base_params(pts, out, n_points, n_frames, p_begin, p_end);
+    if (mode == lmc::kSlerp) {
+        if (n_samples < 1 || !sample_ts || !seg) return fail(LMC_ERR_INVALID, "need a non-empty sample table");
+    } else {
+        if (n_samples < 1 || n_samples >= (1LL << 31) || !sample_ts || !seg)
+            return fail(LMC_ERR_INVALID, "need a sample table of 1 .. 2^31 - 1 rows");
+        if (mode == lmc::kSlerpLocal && !ref_pose) return fail(LMC_ERR_INVALID, "ref_pose is NULL");
+        // (refused here too, not only by the launch plan: an empty point range returns before the plan is made)
+        if (ex && (ex->n_peers > 0 || ex->mc_out || ex->mc_lvx14)) return fail(LMC_ERR_INVALID, "%s", lmc::no_merge_reason(mode));
+    }
+    if (!hold_idx && !ts) return fail(LMC_ERR_INVALID, "timestamps are NULL");
+    if (!hold_idx && !f64 && !frame_start) return fail(LMC_ERR_INVALID, "frame_start is NULL");
+    if ((reinterpret_cast<uintptr_t>(ts) | reinterpret_cast<uintptr_t>(seg) | reinterpret_cast<uintptr_t>(ref_pose)) & 15u)
+        return fail(LMC_ERR_ALIGN, mode == lmc::kSlerpLocal ? "timestamps / seg / ref_pose must be 16-byte aligned" : "timestamps / seg must be 16-byte aligned");
+    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = ts; P.pose_Rt = ref_pose;
+    P.samp_ts = sample_ts; P.samp_tab = seg; P.n_samp = n_samples; P.hold_idx = hold_idx;
+    return run(f64, mode, P, ex, stream);
+}
 int lmc_deskew_slerp_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off, const int64_t* frame_start,
                          const int64_t* sample_ts, const double* seg, int64_t n_samples, const int32_t* hold_idx,
                          double* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
                          const lmc_export* ex, void* stream) {
-    LMC_SLERP_BODY(true, ts, false)
+    return slerp_family(true, lmc::kSlerp, pts_n4, ts, frame_off, frame_start, sample_ts, seg, n_samples, hold_idx, nullptr,
+                        out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 int lmc_deskew_slerp_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off, const int64_t* frame_start,
                          const int64_t* sample_ts, const double* seg, int64_t n_samples, const int32_t* hold_idx,
                          float* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
                          const lmc_export* ex, void* stream) {
-    LMC_SLERP_BODY(false, ts_off, true)
+    return slerp_family(false, lmc::kSlerp, pts_n4, ts_off, frame_off, frame_start, sample_ts, seg, n_samples, hold_idx, nullptr,
+                        out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 
 int lmc_slerp_pose_at(const int64_t* sample_ts, const double* seg, int64_t n_samples, const int64_t* query_ts, int64_t n_query,
@@ -266,57 +284,32 @@ int lmc_slerp_pose_at(const int64_t* sample_ts, const double* seg, int64_t n_sam
     return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_slerp_pose_at");
 }
 
-#define LMC_SLERP_LOCAL_BODY(F64, TS, NEED_FS)                                                           \
-    lmc::Params P = base_params(pts_n4, out_n4, n_points, n_frames, p_begin, p_end);                     \
-    if (n_samples < 1 || n_samples >= (1LL << 31) || !sample_ts || !seg)                                 \
-        return fail(LMC_ERR_INVALID, "need a sample table of 1 .. 2^31 - 1 rows");                       \
-    if (!ref_pose) return fail(LMC_ERR_INVALID, "ref_pose is NULL");                                     \
-    if (ex && (ex->n_peers > 0 || ex->mc_out || ex->mc_lvx14))                                           \
-        return fail(LMC_ERR_INVALID, "sensor-frame deskew has no merged-cloud assembly (each frame is in its own sensor frame)"); \
-    if (!TS) return fail(LMC_ERR_INVALID, "timestamps are NULL");                                        \
-    if (NEED_FS && !frame_start) return fail(LMC_ERR_INVALID, "frame_start is NULL");                    \
-    if ((reinterpret_cast<uintptr_t>(TS) | reinterpret_cast<uintptr_t>(seg) | reinterpret_cast<uintptr_t>(ref_pose)) & 15u) \
-        return fail(LMC_ERR_ALIGN, "timestamps / seg / ref_pose must be 16-byte aligned");               \
-    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = TS; P.pose_Rt = ref_pose;               \
-    P.samp_ts = sample_ts; P.samp_tab = seg; P.n_samp = n_samples;                                       \
-    return run(F64, lmc::kSlerpLocal, P, ex, stream);
-
 int lmc_deskew_slerp_local_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off, const int64_t* frame_start,
                                const int64_t* sample_ts, const double* seg, int64_t n_samples, const double* ref_pose,
                                double* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
                                const lmc_export* ex, void* stream) {
-    LMC_SLERP_LOCAL_BODY(true, ts, false)
+    return slerp_family(true, lmc::kSlerpLocal, pts_n4, ts, frame_off, frame_start, sample_ts, seg, n_samples, nullptr, ref_pose,
+                        out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 int lmc_deskew_slerp_local_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off, const int64_t* frame_start,
                                const int64_t* sample_ts, const double* seg, int64_t n_samples, const double* ref_pose,
                                float* out_n4, int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end,
                                const lmc_export* ex, void* stream) {
-    LMC_SLERP_LOCAL_BODY(false, ts_off, true)
+    return slerp_family(false, lmc::kSlerpLocal, pts_n4, ts_off, frame_off, frame_start, sample_ts, seg, n_samples, nullptr, ref_pose,
+                        out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
-
-#define LMC_DISTORT_BODY(F64, TS, NEED_FS)                                                               \
-    lmc::Params P = base_params(pts_n4, out_n4, n_points, n_frames, p_begin, p_end);                     \
-    if (n_samples < 1 || n_samples >= (1LL << 31) || !sample_ts || !seg)                                 \
-        return fail(LMC_ERR_INVALID, "need a sample table of 1 .. 2^31 - 1 rows");                       \
-    if (ex && (ex->n_peers > 0 || ex->mc_out || ex->mc_lvx14))                                           \
-        return fail(LMC_ERR_INVALID, "distortion has no merged-cloud assembly (each point is in its own sensor frame)"); \
-    if (!TS) return fail(LMC_ERR_INVALID, "timestamps are NULL");                                        \
-    if (NEED_FS && !frame_start) return fail(LMC_ERR_INVALID, "frame_start is NULL");                    \
-    if ((reinterpret_cast<uintptr_t>(TS) | reinterpret_cast<uintptr_t>(seg)) & 15u)                      \
-        return fail(LMC_ERR_ALIGN, "timestamps / seg must be 16-byte aligned");                          \
-    P.frame_off = frame_off; P.frame_start = frame_start; P.ts = TS;                                     \
-    P.samp_ts = sample_ts; P.samp_tab = seg; P.n_samp = n_samples;                                       \
-    return run(F64, lmc::kSlerpDistort, P, ex, stream);
 
 int lmc_distort_slerp_f64(const double* pts_n4, const int64_t* ts, const int64_t* frame_off, const int64_t* frame_start,
                           const int64_t* sample_ts, const double* seg, int64_t n_samples, double* out_n4,
                           int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
-    LMC_DISTORT_BODY(true, ts, false)
+    return slerp_family(true, lmc::kSlerpDistort, pts_n4, ts, frame_off, frame_start, sample_ts, seg, n_samples, nullptr, nullptr,
+                        out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 int lmc_distort_slerp_f32(const float* pts_n4, const uint32_t* ts_off, const int64_t* frame_off, const int64_t* frame_start,
                           const int64_t* sample_ts, const double* seg, int64_t n_samples, float* out_n4,
                           int64_t n_points, int32_t n_frames, int64_t p_begin, int64_t p_end, const lmc_export* ex, void* stream) {
-    LMC_DISTORT_BODY(false, ts_off, true)
+    return slerp_family(false, lmc::kSlerpDistort, pts_n4, ts_off, frame_off, frame_start, sample_ts, seg, n_samples, nullptr, nullptr,
+                        out_n4, n_points, n_frames, p_begin, p_end, ex, stream);
 }
 
 int lmc_quantize_f64(const double* pts_n4, int64_t n_points, const lmc_export* ex, void* stream) {

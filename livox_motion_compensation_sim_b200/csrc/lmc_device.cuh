@@ -593,10 +593,10 @@ __device__ __forceinline__ Pt point_eval(const Params& P, int32_t f, bool single
         }
         const double dt = __dmul_rn((double)(t - fs), 1e-9);                                   // CS:1454
         gyro_rotate(__dmul_rn(g0, dt), __dmul_rn(g1, dt), __dmul_rn(g2, dt), in, out);
-    } else if constexpr (MODE == kSlerp) {
+    } else if constexpr (kSlerpFamily<MODE>) {
         const int64_t S = P.n_samp;
         int64_t k; double alpha = 0.0;
-        if (P.hold_idx != nullptr) k = __ldg(P.hold_idx + f);
+        if (MODE == kSlerp && P.hold_idx != nullptr) k = __ldg(P.hold_idx + f);
         else {
             const int64_t t = F64 ? tsraw : tsraw + fs;
             const Bracket b = bracket_of(P.samp_ts, S, t, t0, rate);
@@ -605,41 +605,15 @@ __device__ __forceinline__ Pt point_eval(const Params& P, int32_t f, bool single
             else if (k >= S - 1) k = S - 1;
             else alpha = (double)(t - b.tb);                           // times inv_dt_k below
         }
-        double row[kSegStride];
+        double row[kSegStride], ref[12];                           // ref: the frame's reference pose (kSlerpLocal)
         const double2* sr = reinterpret_cast<const double2*>(P.samp_tab + kSegStride * k);
 #pragma unroll
         for (int q = 0; q < kSegStride / 2; ++q) { const double2 v = __ldg(sr + q); row[2 * q] = v.x; row[2 * q + 1] = v.y; }
+        if constexpr (MODE == kSlerpLocal) load_pose12(P.pose_Rt + 12 * (int64_t)f, ref);
         alpha = __dmul_rn(alpha, row[19]);
-        slerp_apply(row, alpha, in, out);
-    } else if constexpr (MODE == kSlerpLocal) {
-        const int64_t S = P.n_samp;
-        const int64_t t = F64 ? tsraw : tsraw + fs;
-        const Bracket b = bracket_of(P.samp_ts, S, t, t0, rate);
-        int64_t k = b.k; double alpha = 0.0;
-        if (k < 0) k = 0;
-        else if (k >= S - 1) k = S - 1;
-        else alpha = (double)(t - b.tb);
-        double row[kSegStride], ref[12];
-        const double2* sr = reinterpret_cast<const double2*>(P.samp_tab + kSegStride * k);
-#pragma unroll
-        for (int q = 0; q < kSegStride / 2; ++q) { const double2 v = __ldg(sr + q); row[2 * q] = v.x; row[2 * q + 1] = v.y; }
-        load_pose12(P.pose_Rt + 12 * (int64_t)f, ref);
-        alpha = __dmul_rn(alpha, row[19]);
-        slerp_local_apply(row, alpha, ref, in, out);
-    } else if constexpr (MODE == kSlerpDistort) {
-        const int64_t S = P.n_samp;
-        const int64_t t = F64 ? tsraw : tsraw + fs;
-        const Bracket b = bracket_of(P.samp_ts, S, t, t0, rate);
-        int64_t k = b.k; double alpha = 0.0;
-        if (k < 0) k = 0;
-        else if (k >= S - 1) k = S - 1;
-        else alpha = (double)(t - b.tb);
-        double row[kSegStride];
-        const double2* sr = reinterpret_cast<const double2*>(P.samp_tab + kSegStride * k);
-#pragma unroll
-        for (int q = 0; q < kSegStride / 2; ++q) { const double2 v = __ldg(sr + q); row[2 * q] = v.x; row[2 * q + 1] = v.y; }
-        alpha = __dmul_rn(alpha, row[19]);
-        distort_apply(row, alpha, in, out);
+        if constexpr (MODE == kSlerp)           slerp_apply(row, alpha, in, out);
+        else if constexpr (MODE == kSlerpLocal) slerp_local_apply(row, alpha, ref, in, out);
+        else                                    distort_apply(row, alpha, in, out);
     }
     return out;
 }

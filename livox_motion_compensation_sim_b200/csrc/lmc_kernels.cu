@@ -127,35 +127,6 @@ __global__ void __launch_bounds__(kThreads, 2) k_fused(const __grid_constant__ P
     if (lim_lo == base && lim_hi == base + kTile) tile_body<F64, MODE, true>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
     else                                          tile_body<F64, MODE, false>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
 }
-// sensor-frame deskew (kSlerpLocal) under its own name: k_fused's body.  (Not shared through an inline function: routing
-// k_fused itself through one changes the register allocation of its float4 instantiations.)
-template <bool F64>
-__global__ void __launch_bounds__(kThreads, 2) k_local_fused(const __grid_constant__ Params P)
-{
-    __shared__ __align__(16) uint32_t s_lvx[kTilePairs * 7];
-    __shared__ TileMeta s_tm;
-    const int64_t tile0 = (P.p_begin / kTile) * kTile;
-    const int64_t base  = tile0 + (int64_t)blockIdx.x * kTile;
-    const int64_t lim_lo = base > P.p_begin ? base : P.p_begin;
-    const int64_t lim_hi = base + kTile < P.p_end ? base + kTile : P.p_end;
-    if (lim_lo >= lim_hi) return;
-    if (lim_lo == base && lim_hi == base + kTile) tile_body<F64, kSlerpLocal, true>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
-    else                                          tile_body<F64, kSlerpLocal, false>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
-}
-// distortion (kSlerpDistort) under its own name: k_fused's body, as k_local_fused
-template <bool F64>
-__global__ void __launch_bounds__(kThreads, 2) k_distort_fused(const __grid_constant__ Params P)
-{
-    __shared__ __align__(16) uint32_t s_lvx[kTilePairs * 7];
-    __shared__ TileMeta s_tm;
-    const int64_t tile0 = (P.p_begin / kTile) * kTile;
-    const int64_t base  = tile0 + (int64_t)blockIdx.x * kTile;
-    const int64_t lim_lo = base > P.p_begin ? base : P.p_begin;
-    const int64_t lim_hi = base + kTile < P.p_end ? base + kTile : P.p_end;
-    if (lim_lo >= lim_hi) return;
-    if (lim_lo == base && lim_hi == base + kTile) tile_body<F64, kSlerpDistort, true>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
-    else                                          tile_body<F64, kSlerpDistort, false>(P, base, lim_lo, lim_hi, s_lvx, s_tm);
-}
 
 // (a1) LMC:802-812: one thread per frame
 __global__ void k_pose_lookup(const double* __restrict__ traj_t, int64_t n_t, const double* __restrict__ traj_Rt,
@@ -275,9 +246,7 @@ static cudaError_t launch_fused(const Params& P, cudaStream_t st) {
     const int64_t tile0 = (P.p_begin / kTile) * kTile;
     const int64_t tiles = (P.p_end - tile0 + kTile - 1) / kTile;
     if (tiles > 0x7fffffffLL) return cudaErrorInvalidValue;
-    if constexpr (MODE == kSlerpLocal)        k_local_fused<F64><<<(unsigned)tiles, kThreads, 0, st>>>(P);
-    else if constexpr (MODE == kSlerpDistort) k_distort_fused<F64><<<(unsigned)tiles, kThreads, 0, st>>>(P);
-    else                                      k_fused<F64, MODE><<<(unsigned)tiles, kThreads, 0, st>>>(P);
+    k_fused<F64, MODE><<<(unsigned)tiles, kThreads, 0, st>>>(P);
     return cudaGetLastError();
 }
 

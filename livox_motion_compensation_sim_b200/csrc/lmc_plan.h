@@ -87,13 +87,17 @@ inline Plan refuse_call(const char* msg) {
     return pl;
 }
 
+// why a kSlerpLocal / kSlerpDistort call with peer or multicast pointers is refused
+inline const char* no_merge_reason(int mode) {
+    return mode == kSlerpLocal ? "sensor-frame deskew has no merged-cloud assembly (each frame is in its own sensor frame)"
+                               : "distortion has no merged-cloud assembly (each point is in its own sensor frame)";
+}
+
 // path: lmc_set_path (0 direct, 1 auto, 2 streaming); sm_count: the current device's.  P is a validated, non-empty call.
 inline Plan plan_point_launch(bool f64, int mode, const Params& P, int path, int sm_count) {
     Plan pl;
-    if (mode == kSlerpLocal && (P.n_peers > 0 || P.mc_out || P.mc_lvx))
-        return refuse_call("sensor-frame deskew has no merged-cloud assembly (each frame is in its own sensor frame)");
-    if (mode == kSlerpDistort && (P.n_peers > 0 || P.mc_out || P.mc_lvx))
-        return refuse_call("distortion has no merged-cloud assembly (each point is in its own sensor frame)");
+    if ((mode == kSlerpLocal || mode == kSlerpDistort) && (P.n_peers > 0 || P.mc_out || P.mc_lvx))
+        return refuse_call(no_merge_reason(mode));
     const int64_t tp = stream_tile_points(f64, mode);
     pl.tile0 = (P.p_begin / tp) * tp;
     pl.n_tiles = (P.p_end - pl.tile0 + tp - 1) / tp;

@@ -441,29 +441,17 @@ __device__ __forceinline__ void stream_body(const Params& P, int64_t tile0, int6
         if (fl != 0 && P.status != nullptr) atomicOr(P.status, fl);
     }
 }
+// (stream_body stays a separate inline function: folding it into k_stream changes the machine code of k_stream's instantiations)
 template <bool F64, int MODE, int EX>
 __global__ void __launch_bounds__(kStreamThreads, 1) k_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles) {
     stream_body<F64, MODE, EX>(P, tile0, n_tiles);
-}
-// sensor-frame deskew (kSlerpLocal) under its own name
-template <bool F64, int EX>
-__global__ void __launch_bounds__(kStreamThreads, 1) k_local_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles) {
-    stream_body<F64, kSlerpLocal, EX>(P, tile0, n_tiles);
-}
-// distortion (kSlerpDistort) under its own name
-template <bool F64, int EX>
-__global__ void __launch_bounds__(kStreamThreads, 1) k_distort_stream(const __grid_constant__ Params P, int64_t tile0, int64_t n_tiles) {
-    stream_body<F64, kSlerpDistort, EX>(P, tile0, n_tiles);
 }
 
 // ---- launcher ----------------------------------------------------------------------------------
 template <bool F64, int MODE, int EX>
 static cudaError_t launch_stream_ex(const Params& P, const Plan& pl, int dev, cudaStream_t st) {
     using Cfg = StreamCfg<F64, MODE>;
-    void (*kern)(const Params, int64_t, int64_t);
-    if constexpr (MODE == kSlerpLocal)        kern = k_local_stream<F64, EX>;
-    else if constexpr (MODE == kSlerpDistort) kern = k_distort_stream<F64, EX>;
-    else                                      kern = k_stream<F64, MODE, EX>;
+    void (*kern)(const Params, int64_t, int64_t) = k_stream<F64, MODE, EX>;
     static thread_local int attr_dev = -1;
     if (attr_dev != dev) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);

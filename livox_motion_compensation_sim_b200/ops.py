@@ -165,23 +165,38 @@ def pose_lookup_hold_next(traj_t: torch.Tensor, traj_Rt: torch.Tensor, frame_t: 
     return pose, idx
 
 
-@_on_tensor_device
-def align_rigid(pts: torch.Tensor, frame_off: torch.Tensor, pose_Rt: torch.Tensor, *, out: Optional[torch.Tensor] = None,
-                export: Optional[ExportSpec] = None, p_range=None, want_out: bool = True):
-    """(a2)+(a3) LMC:772-776 over all frames, frame-major (LMC:888). Returns (aligned, ExportBuffers|None)."""
+def _point_op(name, pts, frame_off, args, out, export, p_range, want_out, per_frame=None):
+    """The body of the aligned-cloud operators: lmc_<name>_f64 / _f32 (pts, *args(f64), out, n_points, n_frames, p_begin,
+    p_end, ex, stream), with out and the export buffers allocated here.  args(f64) checks and returns the operator's own
+    arguments between pts and out (timestamps follow the layout); per_frame = (name, tensor) needs one row per frame."""
     f64 = _layout(pts)
     n, F = pts.shape[0], frame_off.shape[0] - 1
-    if pose_Rt.shape[0] != F:
-        raise ValueError("pose_Rt must have one row per frame")
+    if per_frame is not None and per_frame[1].shape[0] != F:
+        raise ValueError(f"{per_frame[0]} must have one row per frame")
     if out is None and want_out:
         out = torch.empty_like(pts)
     ex, bufs = _make_export(export, n, pts.device)
     b, e = _range(n, p_range)
-    fn = C.lib().lmc_align_rigid_f64 if f64 else C.lib().lmc_align_rigid_f32
-    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(frame_off, torch.int64, "frame_off"),
-               _req(pose_Rt, torch.float64, "pose_Rt", (12,)), _req(out, pts.dtype, "out", (4,)),
-               n, F, b, e, None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
+    fn = getattr(C.lib(), f"lmc_{name}_{'f64' if f64 else 'f32'}")
+    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), *args(f64), _req(out, pts.dtype, "out", (4,)), n, F, b, e,
+               None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
     return out, bufs
+
+
+def _slerp_args(f64, ts, frame_off, frame_start, sample_ts, seg):
+    """The Mode C arguments of deskew_slerp, deskew_slerp_local and distort_slerp: ts ... n_samples."""
+    return (_req(ts, torch.int64 if f64 else torch.uint32, "ts"), _req(frame_off, torch.int64, "frame_off"),
+            _req(frame_start, torch.int64, "frame_start"), _req(sample_ts, torch.int64, "sample_ts"),
+            _req(seg, torch.float64, "seg", (22,)), sample_ts.shape[0])
+
+
+@_on_tensor_device
+def align_rigid(pts: torch.Tensor, frame_off: torch.Tensor, pose_Rt: torch.Tensor, *, out: Optional[torch.Tensor] = None,
+                export: Optional[ExportSpec] = None, p_range=None, want_out: bool = True):
+    """(a2)+(a3) LMC:772-776 over all frames, frame-major (LMC:888). Returns (aligned, ExportBuffers|None)."""
+    return _point_op("align_rigid", pts, frame_off,
+                     lambda f64: (_req(frame_off, torch.int64, "frame_off"), _req(pose_Rt, torch.float64, "pose_Rt", (12,))),
+                     out, export, p_range, want_out, per_frame=("pose_Rt", pose_Rt))
 
 
 @_on_tensor_device
@@ -189,18 +204,11 @@ def deskew_gyro(pts: torch.Tensor, ts: torch.Tensor, frame_off: torch.Tensor, fr
                 imu_ts: torch.Tensor, imu_gyro: torch.Tensor, *, out: Optional[torch.Tensor] = None,
                 export: Optional[ExportSpec] = None, p_range=None, want_out: bool = True):
     """(a6)-(a8) CS:1435-1536. f64 points take int64 ns timestamps, f32 points uint32 ns offsets."""
-    f64 = _layout(pts)
-    n, F = pts.shape[0], frame_off.shape[0] - 1
-    if out is None and want_out:
-        out = torch.empty_like(pts)
-    ex, bufs = _make_export(export, n, pts.device)
-    b, e = _range(n, p_range)
-    fn = C.lib().lmc_deskew_gyro_f64 if f64 else C.lib().lmc_deskew_gyro_f32
-    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(ts, torch.int64 if f64 else torch.uint32, "ts"),
-               _req(frame_off, torch.int64, "frame_off"), _req(frame_start, torch.int64, "frame_start"),
-               _req(imu_ts, torch.int64, "imu_ts"), _req(imu_gyro, torch.float64, "imu_gyro", (3,)), imu_ts.shape[0],
-               _req(out, pts.dtype, "out", (4,)), n, F, b, e, None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
-    return out, bufs
+    return _point_op("deskew_gyro", pts, frame_off,
+                     lambda f64: (_req(ts, torch.int64 if f64 else torch.uint32, "ts"), _req(frame_off, torch.int64, "frame_off"),
+                                  _req(frame_start, torch.int64, "frame_start"), _req(imu_ts, torch.int64, "imu_ts"),
+                                  _req(imu_gyro, torch.float64, "imu_gyro", (3,)), imu_ts.shape[0]),
+                     out, export, p_range, want_out)
 
 
 @_on_tensor_device
@@ -208,19 +216,9 @@ def deskew_slerp(pts: torch.Tensor, ts: Optional[torch.Tensor], frame_off: torch
                  sample_ts: torch.Tensor, seg: torch.Tensor, *, hold_idx: Optional[torch.Tensor] = None,
                  out: Optional[torch.Tensor] = None, export: Optional[ExportSpec] = None, p_range=None, want_out: bool = True):
     """Mode C: per-point bracket search + SLERP + lerp (+ optional hold-next = Mode A)."""
-    f64 = _layout(pts)
-    n, F = pts.shape[0], frame_off.shape[0] - 1
-    if out is None and want_out:
-        out = torch.empty_like(pts)
-    ex, bufs = _make_export(export, n, pts.device)
-    b, e = _range(n, p_range)
-    fn = C.lib().lmc_deskew_slerp_f64 if f64 else C.lib().lmc_deskew_slerp_f32
-    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(ts, torch.int64 if f64 else torch.uint32, "ts"),
-               _req(frame_off, torch.int64, "frame_off"), _req(frame_start, torch.int64, "frame_start"),
-               _req(sample_ts, torch.int64, "sample_ts"), _req(seg, torch.float64, "seg", (22,)), sample_ts.shape[0],
-               _req(hold_idx, torch.int32, "hold_idx"), _req(out, pts.dtype, "out", (4,)), n, F, b, e,
-               None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
-    return out, bufs
+    return _point_op("deskew_slerp", pts, frame_off,
+                     lambda f64: (*_slerp_args(f64, ts, frame_off, frame_start, sample_ts, seg), _req(hold_idx, torch.int32, "hold_idx")),
+                     out, export, p_range, want_out)
 
 
 @_on_tensor_device
@@ -241,21 +239,10 @@ def deskew_slerp_local(pts: torch.Tensor, ts: torch.Tensor, frame_off: torch.Ten
     """Sensor-frame deskew: every point of frame f in the sensor frame of ref_pose[f] ((F, 12) f64, normally
     slerp_pose_at of the frame's start or end time), rotation and translation removed.  Arguments as deskew_slerp (no
     hold_idx); the world position is kept in f64 registers, so the f32 layout loses nothing at map-scale positions."""
-    f64 = _layout(pts)
-    n, F = pts.shape[0], frame_off.shape[0] - 1
-    if ref_pose.shape[0] != F:
-        raise ValueError("ref_pose must have one row per frame")
-    if out is None and want_out:
-        out = torch.empty_like(pts)
-    ex, bufs = _make_export(export, n, pts.device)
-    b, e = _range(n, p_range)
-    fn = C.lib().lmc_deskew_slerp_local_f64 if f64 else C.lib().lmc_deskew_slerp_local_f32
-    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(ts, torch.int64 if f64 else torch.uint32, "ts"),
-               _req(frame_off, torch.int64, "frame_off"), _req(frame_start, torch.int64, "frame_start"),
-               _req(sample_ts, torch.int64, "sample_ts"), _req(seg, torch.float64, "seg", (22,)), sample_ts.shape[0],
-               _req(ref_pose, torch.float64, "ref_pose", (12,)), _req(out, pts.dtype, "out", (4,)), n, F, b, e,
-               None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
-    return out, bufs
+    return _point_op("deskew_slerp_local", pts, frame_off,
+                     lambda f64: (*_slerp_args(f64, ts, frame_off, frame_start, sample_ts, seg),
+                                  _req(ref_pose, torch.float64, "ref_pose", (12,))),
+                     out, export, p_range, want_out, per_frame=("ref_pose", ref_pose))
 
 
 @_on_tensor_device
@@ -265,18 +252,9 @@ def distort_slerp(pts: torch.Tensor, ts: torch.Tensor, frame_off: torch.Tensor, 
     """Distortion, the exact inverse of deskew_slerp: every WORLD point into the sensor frame of Mode C's pose at the
     point's own time, R(t)^T (W - x(t)) -- what a sensor moving along the sample table records of a static world.
     Arguments as deskew_slerp_local (no ref_pose); deskew_slerp of the result gives the world points back."""
-    f64 = _layout(pts)
-    n, F = pts.shape[0], frame_off.shape[0] - 1
-    if out is None and want_out:
-        out = torch.empty_like(pts)
-    ex, bufs = _make_export(export, n, pts.device)
-    b, e = _range(n, p_range)
-    fn = C.lib().lmc_distort_slerp_f64 if f64 else C.lib().lmc_distort_slerp_f32
-    C.check(fn(_req(pts, pts.dtype, "pts", (4,)), _req(ts, torch.int64 if f64 else torch.uint32, "ts"),
-               _req(frame_off, torch.int64, "frame_off"), _req(frame_start, torch.int64, "frame_start"),
-               _req(sample_ts, torch.int64, "sample_ts"), _req(seg, torch.float64, "seg", (22,)), sample_ts.shape[0],
-               _req(out, pts.dtype, "out", (4,)), n, F, b, e, None if ex is None else C.ctypes.byref(ex), _stream_ptr()))
-    return out, bufs
+    return _point_op("distort_slerp", pts, frame_off,
+                     lambda f64: _slerp_args(f64, ts, frame_off, frame_start, sample_ts, seg),
+                     out, export, p_range, want_out)
 
 
 @_on_tensor_device

@@ -1,8 +1,8 @@
 """Sensor-frame deskew (lmc_deskew_slerp_local_*) and the pose at a time (lmc_slerp_pose_at).
 
 CPU: the C oracle against an independent SciPy restatement (Slerp + np.interp, then R_ref^-1 (R(t) p + x(t) - x_ref)), the
-pose oracle against Slerp and the golden lerp, the launch plan's routing of the new mode, and the library's k_local_*
-instantiations against the kernels this file's GPU table names.
+pose oracle against Slerp and the golden lerp, the launch plan's routing of the new mode, and the library's k_fused /
+k_stream instantiations of the mode against the kernels this file's GPU table names.
 GPU: every new kernel against the oracle on a stream built as test_kernel_variants builds it (empty and one-point frames,
 tiles with 0 / 1 / many boundaries, clamps, an edge-value block), plus the properties that make the output a sensor-frame
 cloud: a stationary trajectory changes nothing, align_rigid at the reference pose gives Mode C's world cloud back, raw
@@ -172,7 +172,7 @@ def test_routing(plan):
 class Case:
     f64: bool
     path: int
-    kernel: tuple                  # ("local_fused", f64) or ("local_stream", f64, ex)
+    kernel: tuple                  # ("local_fused", f64): k_fused<F64, 4>; ("local_stream", f64, ex): k_stream<F64, 4, ex>
     out: bool = True
     lvx: Optional[str] = None      # None | "t2" | "lvx2" | "lvx2+tag"
     las: bool = False              # LAS x / y / z + intensity, decimal scales
@@ -207,15 +207,16 @@ def test_table_routes_to_its_kernels(plan):
 
 
 def test_table_covers_every_local_kernel():
-    """The library's k_local_* instantiations are exactly the kernels the GPU table names: a variant without a row fails."""
+    """The library's k_fused / k_stream instantiations of mode 4 are exactly the kernels the GPU table names: a variant
+    without a row fails."""
     from livox_motion_compensation_sim_b200 import _build
     path = os.environ.get("LMC_B200_LIB", _build.LIB_PATH)
     if not os.path.exists(path):
         pytest.skip(f"{path} is not built")
     exe = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
     text = subprocess.run([exe, "-symbols", path], capture_output=True, text=True, check=True, timeout=300).stdout
-    built = {("local_fused", f == "1") for f in re.findall(r"k_local_fusedILb([01])EEEv", text)}
-    built |= {("local_stream", f == "1", int(x)) for f, x in re.findall(r"k_local_streamILb([01])ELi(\d+)EEEv", text)}
+    built = {("local_fused", f == "1") for f in re.findall(rf"k_fusedILb([01])ELi{LOCAL}EE", text)}
+    built |= {("local_stream", f == "1", int(x)) for f, x in re.findall(rf"k_streamILb([01])ELi{LOCAL}ELi(\d+)EE", text)}
     assert built == {c.kernel for c in TABLE}
 
 

@@ -2,8 +2,8 @@
 simulator's motion-distorted scans built on it (lmc_scan_emit_index, ops.scan_frames(motion=...), 'motion_distortion').
 
 CPU: the C oracle against an independent SciPy restatement (Slerp + np.interp, then R(t)^-1 (W - x(t))) and against Mode C
-(deskewing the distorted points gives the world back), the launch plan's routing of the new mode, the library's k_distort_*
-instantiations against the kernels this file's GPU table names, and the simulator's argument checks.
+(deskewing the distorted points gives the world back), the launch plan's routing of the new mode, the library's k_fused /
+k_stream instantiations of the mode against the kernels this file's GPU table names, and the simulator's argument checks.
 GPU: every new kernel against the oracle on a stream built as test_kernel_variants builds it, the fast and the general route
 byte for byte, the refusals, the inverse properties (Mode C and sensor-frame deskew of distorted points), the scanner on a
 stationary trajectory, and the C3 golden run with and without motion distortion."""
@@ -125,7 +125,7 @@ def test_routing(plan):
 class Case:
     f64: bool
     path: int
-    kernel: tuple                  # ("distort_fused", f64) or ("distort_stream", f64, ex)
+    kernel: tuple                  # ("distort_fused", f64): k_fused<F64, 5>; ("distort_stream", f64, ex): k_stream<F64, 5, ex>
     out: bool = True
     lvx: Optional[str] = None      # None | "t2" | "lvx2" | "lvx2+tag"
     las: bool = False              # LAS x / y / z + intensity, decimal scales
@@ -159,15 +159,16 @@ def test_table_routes_to_its_kernels(plan):
 
 
 def test_table_covers_every_distort_kernel():
-    """The library's k_distort_* instantiations are exactly the kernels the GPU table names: a variant without a row fails."""
+    """The library's k_fused / k_stream instantiations of mode 5 are exactly the kernels the GPU table names: a variant
+    without a row fails."""
     from livox_motion_compensation_sim_b200 import _build
     path = os.environ.get("LMC_B200_LIB", _build.LIB_PATH)
     if not os.path.exists(path):
         pytest.skip(f"{path} is not built")
     exe = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
     text = subprocess.run([exe, "-symbols", path], capture_output=True, text=True, check=True, timeout=300).stdout
-    built = {("distort_fused", f == "1") for f in re.findall(r"k_distort_fusedILb([01])EEEv", text)}
-    built |= {("distort_stream", f == "1", int(x)) for f, x in re.findall(r"k_distort_streamILb([01])ELi(\d+)EEEv", text)}
+    built = {("distort_fused", f == "1") for f in re.findall(rf"k_fusedILb([01])ELi{DISTORT}EE", text)}
+    built |= {("distort_stream", f == "1", int(x)) for f, x in re.findall(rf"k_streamILb([01])ELi{DISTORT}ELi(\d+)EE", text)}
     assert built == {c.kernel for c in TABLE}
 
 
