@@ -455,8 +455,11 @@ int lmc_las_pf3_header(int64_t n_points, const double scale[3], const double off
  *                     in its slot (same compaction and subsample), for a caller that observes the points from other
  *                     poses (lmc_distort_slerp_f64: each point from the pose at its own time).
  * pos_f3 / R_f9: per-frame sensor position and SciPy rotation matrix (row-major) of the sensor pose.
+ * n_env <= LMC_SCAN_MAX_ENV: per-frame counts, ranks and tile_off are int32, so all four calls refuse a larger
+ * environment with LMC_ERR_INVALID before they write anything.
  */
 #define LMC_SCAN_TILE 256
+#define LMC_SCAN_MAX_ENV 2147483647LL
 int lmc_scan_mark(const double* env_m4, int64_t n_env, const double* pos_f3, const double* R_f9, int32_t n_frames,
                   double range_max_sq, double fov_h_half_deg, double fov_v_half_deg, double range_min,
                   double edge_eps_deg, uint8_t* flags, int32_t* tile_off, int32_t* n_visible,

@@ -580,6 +580,7 @@ int lmc_scan_mark(const double* env_m4, int64_t n_env, const double* pos_f3, con
     int rc = check_device();
     if (rc != LMC_OK) return rc;
     if (n_env < 0 || n_frames < 0 || !(edge_eps_deg >= 0.0)) return fail(LMC_ERR_INVALID, "negative size / edge_eps");
+    if (n_env > LMC_SCAN_MAX_ENV) return fail(LMC_ERR_INVALID, "n_env above LMC_SCAN_MAX_ENV");
     if (n_frames == 0) return LMC_OK;
     if (!pos_f3 || !R_f9 || !tile_off || !n_visible || (n_env > 0 && (!env_m4 || !flags))) return fail(LMC_ERR_INVALID, "NULL argument");
     if (!aligned32(env_m4)) return fail(LMC_ERR_ALIGN, "environment must be 32-byte aligned");
@@ -591,6 +592,7 @@ int lmc_scan_recount(const uint8_t* flags, int64_t n_env, int32_t n_frames, int3
     int rc = check_device();
     if (rc != LMC_OK) return rc;
     if (n_env < 0 || n_frames < 0) return fail(LMC_ERR_INVALID, "negative size");
+    if (n_env > LMC_SCAN_MAX_ENV) return fail(LMC_ERR_INVALID, "n_env above LMC_SCAN_MAX_ENV");
     if (n_frames == 0) return LMC_OK;
     if (!tile_off || !n_visible || (n_env > 0 && !flags)) return fail(LMC_ERR_INVALID, "NULL argument");
     cudaError_t e = lmc::launch_scan_recount(flags, n_env, n_frames, tile_off, n_visible, static_cast<cudaStream_t>(stream));
@@ -602,6 +604,7 @@ int lmc_scan_emit(const double* env_m4, int64_t n_env, const double* pos_f3, con
     int rc = check_device();
     if (rc != LMC_OK) return rc;
     if (n_env < 0 || n_frames < 0 || max_points < 1) return fail(LMC_ERR_INVALID, "bad size / max_points");
+    if (n_env > LMC_SCAN_MAX_ENV) return fail(LMC_ERR_INVALID, "n_env above LMC_SCAN_MAX_ENV");
     if (n_frames == 0 || n_env == 0) return LMC_OK;
     if (!env_m4 || !pos_f3 || !R_f9 || !flags || !tile_off || !n_visible || !frame_off || !raw_out_n4) return fail(LMC_ERR_INVALID, "NULL argument");
     if (!aligned32(env_m4) || !aligned32(raw_out_n4)) return fail(LMC_ERR_ALIGN, "environment / output must be 32-byte aligned");
@@ -615,6 +618,7 @@ int lmc_scan_emit_index(const double* env_m4, int64_t n_env, const double* pos_f
     int rc = check_device();
     if (rc != LMC_OK) return rc;
     if (n_env < 0 || n_frames < 0 || max_points < 1) return fail(LMC_ERR_INVALID, "bad size / max_points");
+    if (n_env > LMC_SCAN_MAX_ENV) return fail(LMC_ERR_INVALID, "n_env above LMC_SCAN_MAX_ENV");
     if (n_frames == 0 || n_env == 0) return LMC_OK;
     if (!env_m4 || !pos_f3 || !R_f9 || !flags || !tile_off || !n_visible || !frame_off || !env_idx_out) return fail(LMC_ERR_INVALID, "NULL argument");
     cudaError_t e = lmc::launch_scan_emit(env_m4, n_env, pos_f3, R_f9, n_frames, range_max_sq, flags, tile_off, n_visible, frame_off, max_points,

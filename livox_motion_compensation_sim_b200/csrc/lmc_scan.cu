@@ -7,7 +7,7 @@
 // the per-frame counts back, draws the identical stream in one call, and k_scan_emit adds it.
 //
 // Arithmetic in the reference's order: d2 = (dx*dx + dy*dy) + dz*dz (np.sum over 3 columns),
-// rotated = R^T t through dgemm (k = 0,1,2 FMA chain -- also for a single column, measured),
+// rotated = R^T t through dgemm (k = 0,1,2 FMA chain from +0.0 -- also for a single column, measured),
 // az = atan2(y,x)*180/pi, el = asin(clip(z / max(sqrt(d2),1e-6), -1, 1))*180/pi.  Coordinates are
 // bit-exact.  The FOV decisions could differ from NumPy's only for a point within a few ulp of the FOV
 // edge (device atan2/asin vs the host libm): k_scan_mark therefore marks every point whose |azimuth| or
@@ -37,9 +37,10 @@ __device__ __forceinline__ ScanGeom scan_geom(const double* __restrict__ env, in
     g.d2 = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));     // LMC:713
     g.in_range = g.d2 <= rmax2;                                                                // LMC:717
     // (R^T t)[r] = sum_k R[k][r] t[k]                                                         // LMC:726-728
-    g.x = __fma_rn(R[6], dz, __fma_rn(R[3], dy, __dmul_rn(R[0], dx)));
-    g.y = __fma_rn(R[7], dz, __fma_rn(R[4], dy, __dmul_rn(R[1], dx)));
-    g.z = __fma_rn(R[8], dz, __fma_rn(R[5], dy, __dmul_rn(R[2], dx)));
+    // accumulated from +0.0 as dgemm does: three -0.0 products then sum to +0.0, not -0.0 (atan2 would turn that into 180 deg)
+    g.x = __fma_rn(R[6], dz, __fma_rn(R[3], dy, __fma_rn(R[0], dx, 0.0)));
+    g.y = __fma_rn(R[7], dz, __fma_rn(R[4], dy, __fma_rn(R[1], dx, 0.0)));
+    g.z = __fma_rn(R[8], dz, __fma_rn(R[5], dy, __fma_rn(R[2], dx, 0.0)));
     return g;
 }
 

@@ -540,6 +540,8 @@ def scan_frames(env: torch.Tensor, pos: torch.Tensor, Rm: torch.Tensor, *, range
     dev = env.device
     rmax2 = float(range_max ** 2)                                   # LMC:714
     maxp = int(points_per_frame)
+    if maxp < 1:                                                    # (the kept counts below would silently be 0)
+        raise ValueError(f"points_per_frame must be >= 1, got {points_per_frame}")
     L = C.lib()
     _req(env, torch.float64, "env", (4,)); _req(pos, torch.float64, "pos", (3,)); _req(Rm, torch.float64, "Rm", (9,))
     chunk = max(1, min(F, max_flag_bytes // max(M, 1)))

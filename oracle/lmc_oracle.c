@@ -336,7 +336,7 @@ void orc_deskew_slerp_f64(const double* pts, const int64_t* ts, const int64_t* f
 /* ------------------------------------------------------------------------------------
  * (N4) scan_environment without the noise -- LMC:701-770
  *   d2 = sum((env - pos)**2, axis=1) ; range mask d2 <= range_max**2
- *   rotated = (R.T @ (env - pos).T).T            (dgemm, k = 0,1,2 FMA chain, also for one column)
+ *   rotated = (R.T @ (env - pos).T).T            (dgemm, k = 0,1,2 FMA chain from +0.0, also for one column)
  *   az = arctan2(y, x) * 180 / pi ; el = arcsin(clip(z / max(sqrt(d2), 1e-6), -1, 1)) * 180 / pi
  *   visible = |az| <= fov_h/2 & |el| <= fov_v/2 & range >= range_min   (env order kept)
  *   n_visible > max_points: step = n_visible // max_points; keep indices arange(0, n, step)[:max]
@@ -353,9 +353,10 @@ int64_t orc_scan_frame(const double* env, int64_t M, const double* pos, const do
         double dx = env[4 * i] - pos[0], dy = env[4 * i + 1] - pos[1], dz = env[4 * i + 2] - pos[2];
         double d2 = (dx * dx + dy * dy) + dz * dz;
         if (!(d2 <= rmax2)) continue;
-        double x = fma(R[6 + 0], dz, fma(R[3 + 0], dy, R[0] * dx));
-        double y = fma(R[6 + 1], dz, fma(R[3 + 1], dy, R[1] * dx));
-        double z = fma(R[6 + 2], dz, fma(R[3 + 2], dy, R[2] * dx));
+        /* from +0.0 like dgemm: three -0.0 products sum to +0.0 */
+        double x = fma(R[6 + 0], dz, fma(R[3 + 0], dy, fma(R[0], dx, 0.0)));
+        double y = fma(R[6 + 1], dz, fma(R[3 + 1], dy, fma(R[1], dx, 0.0)));
+        double z = fma(R[6 + 2], dz, fma(R[3 + 2], dy, fma(R[2], dx, 0.0)));
         double rng = sqrt(d2);
         double az = atan2(y, x) * 180.0 / pi;
         double sr = rng > 1e-6 ? rng : 1e-6;
