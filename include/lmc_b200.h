@@ -474,6 +474,39 @@ int lmc_scan_emit_index(const double* env_m4, int64_t n_env, const double* pos_f
                         double range_max_sq, const uint8_t* flags, const int32_t* tile_off, const int32_t* n_visible,
                         const int64_t* frame_off, int32_t max_points, int64_t* env_idx_out, void* stream);
 
+/*
+ * Voxel-grid map of an (n,4) cloud [x y z intensity]: one centroid and one point count per occupied voxel
+ * (definition: oracle/lmc_oracle_voxel.py).  leaf[3] > 0 and origin[3] are finite HOST values; all arithmetic is f64
+ * with explicit rounding, f32 points widened exactly.  Per point and axis:
+ *   u = (p - o) / L ; k = floor(u) in [-2^20, 2^20) ; q = min(trunc((u - k) 2^32), 2^32 - 1) ; q_I = rint(I 2^24), |I| < 256
+ * A point with a non-finite value is dropped with LMC_FLAG_NAN, one with k out of range or |I| >= 256 with
+ * LMC_FLAG_OVERFLOW.  Per voxel, with n points and the int64 sums S of q and q_I:
+ *   centroid = o + (k + (S / n) 2^-32) L ; intensity = (S_I / n) 2^-24      (every operation rounded to nearest;
+ *                                                                            the f32 layout rounds once at the end)
+ * The sums are integers, so the map is bit-identical under any thread schedule and any permutation of the input.
+ * Voxels are ranked by their first point (smallest point index): a frame-major cloud's map grows frame by frame.
+ * Two calls; the caller owns every buffer and reads V in between:
+ *   lmc_voxel_workspace_bytes(n)  bytes of scratch (a hash table of the power of two >= 2n slots, 16 bytes a slot, and
+ *                                 52 bytes a point); a negative LMC_ERR_* for n outside 0 .. 2^31 - 1
+ *   lmc_voxel_index_*             keys, table, ranks; V -> *n_voxels_dev (device int64), flags OR-ed into *status
+ *   lmc_voxel_reduce_*            out_n4 (V,4) centroids in the input's layout, counts int32[V], and, when point_voxel is
+ *                                 not NULL, int32[n] rank of every point's voxel (-1 for a dropped point)
+ * The same points, leaf, origin and workspace go to both calls.  Refused with LMC_ERR_INVALID before anything is
+ * written: n < 0 or n >= 2^31, a leaf that is not finite or <= 0, an origin that is not finite, a NULL required
+ * buffer, n_voxels outside 0 .. n.  Points, workspace and outputs must be 32-byte aligned (LMC_ERR_ALIGN).
+ */
+int64_t lmc_voxel_workspace_bytes(int64_t n_points);
+int lmc_voxel_index_f64(const double* pts_n4, int64_t n_points, const double leaf[3], const double origin[3],
+                        void* workspace, int64_t* n_voxels_dev, uint32_t* status, void* stream);
+int lmc_voxel_index_f32(const float* pts_n4, int64_t n_points, const double leaf[3], const double origin[3],
+                        void* workspace, int64_t* n_voxels_dev, uint32_t* status, void* stream);
+int lmc_voxel_reduce_f64(const double* pts_n4, int64_t n_points, const double leaf[3], const double origin[3],
+                         void* workspace, int64_t n_voxels, double* out_n4, int32_t* counts, int32_t* point_voxel,
+                         void* stream);
+int lmc_voxel_reduce_f32(const float* pts_n4, int64_t n_points, const double leaf[3], const double origin[3],
+                         void* workspace, int64_t n_voxels, float* out_n4, int32_t* counts, int32_t* point_voxel,
+                         void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -95,6 +95,11 @@ _SIGNATURES = {
     "lmc_scan_recount": ([vp, i64, i32, vp, vp, vp], ctypes.c_int),
     "lmc_scan_emit": ([vp, i64, vp, vp, i32, f64, vp, vp, vp, vp, i32, vp, vp, vp], ctypes.c_int),
     "lmc_scan_emit_index": ([vp, i64, vp, vp, i32, f64, vp, vp, vp, vp, i32, vp, vp], ctypes.c_int),
+    "lmc_voxel_workspace_bytes": ([i64], i64),
+    "lmc_voxel_index_f64": ([vp, i64, vp, vp, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_voxel_index_f32": ([vp, i64, vp, vp, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_voxel_reduce_f64": ([vp, i64, vp, vp, vp, i64, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_voxel_reduce_f32": ([vp, i64, vp, vp, vp, i64, vp, vp, vp, vp], ctypes.c_int),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

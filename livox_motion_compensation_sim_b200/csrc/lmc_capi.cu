@@ -39,6 +39,11 @@ cudaError_t launch_text_write(bool f64, const void* rows, int64_t n, int32_t n_c
 cudaError_t launch_lvx_cs(bool f64, const void* pts, const uint8_t* tag, const int64_t* frame_off, const uint64_t* frame_ts,
                           const uint8_t* prefix_host, int32_t prefix_len, int32_t format, uint8_t* out, int32_t n_frames,
                           int64_t max_frame_points, uint32_t* status, cudaStream_t st);
+size_t voxel_workspace_bytes(int64_t n);
+cudaError_t launch_voxel_index(bool f64, const void* pts, int64_t n, const double* leaf, const double* origin, void* ws,
+                               int64_t* n_voxels, uint32_t* status, cudaStream_t st);
+cudaError_t launch_voxel_reduce(bool f64, const void* pts, int64_t n, const double* leaf, const double* origin, void* ws,
+                                int64_t V, void* out, int32_t* counts, int32_t* point_voxel, cudaStream_t st);
 }
 
 namespace {
@@ -476,6 +481,58 @@ int lmc_pcd_ascii_row_offsets_f64(const double* pts_n4, int64_t n_points, const 
                                   int64_t* byte_off, void* stream) { return pcd_row_off(true, pts_n4, n_points, tile_off, rows, n_rows, byte_off, stream); }
 int lmc_pcd_ascii_row_offsets_f32(const float* pts_n4, int64_t n_points, const int64_t* tile_off, const int64_t* rows, int32_t n_rows,
                                   int64_t* byte_off, void* stream) { return pcd_row_off(false, pts_n4, n_points, tile_off, rows, n_rows, byte_off, stream); }
+
+// ---- voxel-grid map: lmc_voxel_index_* (table, ranks, V) then lmc_voxel_reduce_* (sums, centroids) -------------------
+int64_t lmc_voxel_workspace_bytes(int64_t n_points) {
+    if (n_points < 0 || n_points >= (1LL << 31)) return fail(LMC_ERR_INVALID, "n_points must be 0 .. 2^31 - 1");
+    return (int64_t)lmc::voxel_workspace_bytes(n_points);
+}
+static int voxel_check(const void* pts, int64_t n, const double* leaf, const double* origin, const void* ws) {
+    int rc = check_device();
+    if (rc != LMC_OK) return rc;
+    if (n < 0 || n >= (1LL << 31)) return fail(LMC_ERR_INVALID, "n_points must be 0 .. 2^31 - 1");
+    if (!leaf || !origin || !ws || (n > 0 && !pts)) return fail(LMC_ERR_INVALID, "NULL argument");
+    for (int c = 0; c < 3; ++c) {
+        if (!(leaf[c] > 0.0 && leaf[c] <= 1.7976931348623157e308)) return fail(LMC_ERR_INVALID, "leaf[%d] must be finite and > 0", c);
+        if (!(origin[c] >= -1.7976931348623157e308 && origin[c] <= 1.7976931348623157e308)) return fail(LMC_ERR_INVALID, "origin[%d] must be finite", c);
+    }
+    if (!aligned32(pts) || !aligned32(ws)) return fail(LMC_ERR_ALIGN, "points and workspace must be 32-byte aligned");
+    return LMC_OK;
+}
+static int voxel_index(bool f64, const void* pts, int64_t n, const double* leaf, const double* origin, void* ws, int64_t* n_voxels,
+                       uint32_t* status, void* stream) {
+    int rc = voxel_check(pts, n, leaf, origin, ws);
+    if (rc != LMC_OK) return rc;
+    if (!n_voxels || !status) return fail(LMC_ERR_INVALID, "NULL n_voxels_dev / status");
+    cudaError_t e = lmc::launch_voxel_index(f64, pts, n, leaf, origin, ws, n_voxels, status, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_voxel_insert / k_voxel_count / k_voxel_rank");
+}
+static int voxel_reduce(bool f64, const void* pts, int64_t n, const double* leaf, const double* origin, void* ws, int64_t V, void* out,
+                        int32_t* counts, int32_t* point_voxel, void* stream) {
+    int rc = voxel_check(pts, n, leaf, origin, ws);
+    if (rc != LMC_OK) return rc;
+    if (V < 0 || V > n) return fail(LMC_ERR_INVALID, "n_voxels must be 0 .. n_points");
+    if (V > 0 && (!out || !counts)) return fail(LMC_ERR_INVALID, "NULL out_n4 / counts");
+    if (!aligned32(out) || !aligned32(counts) || !aligned32(point_voxel)) return fail(LMC_ERR_ALIGN, "outputs must be 32-byte aligned");
+    cudaError_t e = lmc::launch_voxel_reduce(f64, pts, n, leaf, origin, ws, V, out, counts, point_voxel, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_voxel_accum / k_voxel_finalize");
+}
+int lmc_voxel_index_f64(const double* pts_n4, int64_t n_points, const double leaf[3], const double origin[3], void* workspace,
+                        int64_t* n_voxels_dev, uint32_t* status, void* stream) {
+    return voxel_index(true, pts_n4, n_points, leaf, origin, workspace, n_voxels_dev, status, stream);
+}
+int lmc_voxel_index_f32(const float* pts_n4, int64_t n_points, const double leaf[3], const double origin[3], void* workspace,
+                        int64_t* n_voxels_dev, uint32_t* status, void* stream) {
+    return voxel_index(false, pts_n4, n_points, leaf, origin, workspace, n_voxels_dev, status, stream);
+}
+int lmc_voxel_reduce_f64(const double* pts_n4, int64_t n_points, const double leaf[3], const double origin[3], void* workspace,
+                         int64_t n_voxels, double* out_n4, int32_t* counts, int32_t* point_voxel, void* stream) {
+    return voxel_reduce(true, pts_n4, n_points, leaf, origin, workspace, n_voxels, out_n4, counts, point_voxel, stream);
+}
+int lmc_voxel_reduce_f32(const float* pts_n4, int64_t n_points, const double leaf[3], const double origin[3], void* workspace,
+                         int64_t n_voxels, float* out_n4, int32_t* counts, int32_t* point_voxel, void* stream) {
+    return voxel_reduce(false, pts_n4, n_points, leaf, origin, workspace, n_voxels, out_n4, counts, point_voxel, stream);
+}
 
 // ---- host-side staging helpers (no device work): the reference hands over / expects lists of small per-frame
 // arrays; packing them into the pinned staging buffer (and unpacking results) is memory-bound host work that one

@@ -535,7 +535,7 @@ __global__ void __launch_bounds__(kScanChunk) k_pcd_scan_add(int64_t* __restrict
     const int64_t last = (c + 1) * kScanChunk < n_tiles ? (c + 1) * kScanChunk : n_tiles;
     if (k + 1 < last) tile_off[k + 1] += tile_off[c * kScanChunk];      // (entry `last` is already global)
 }
-static cudaError_t launch_tile_scan(int64_t* tile_off, int64_t tiles, cudaStream_t st) {
+cudaError_t launch_tile_scan(int64_t* tile_off, int64_t tiles, cudaStream_t st) {      // (also the voxel ranks, lmc_voxel.cu)
     if (tiles <= 0) return cudaMemsetAsync(tile_off, 0, sizeof(int64_t), st);
     const int64_t chunks = (tiles + kScanChunk - 1) / kScanChunk;
     k_pcd_scan_chunks<<<(unsigned)chunks, kScanChunk, 0, st>>>(tile_off, tiles);

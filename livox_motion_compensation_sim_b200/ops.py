@@ -483,6 +483,44 @@ def build_las_pf3(pts: torch.Tensor, *, scale=(0.01, 0.01, 0.01), offset=(0.0, 0
     return out, status
 
 
+def _grid3(v, name):
+    import numpy as np
+    a = np.broadcast_to(np.asarray(v, np.float64), (3,))
+    if not np.isfinite(a).all() or (name == "leaf" and not (a > 0).all()):
+        raise ValueError(f"{name} must be three finite values{' > 0' if name == 'leaf' else ''} (or one, broadcast)")
+    return (C.ctypes.c_double * 3)(*[float(x) for x in a])
+
+
+@_on_tensor_device
+def voxel_downsample(pts: torch.Tensor, leaf, origin=(0.0, 0.0, 0.0), *, point_voxel: bool = False):
+    """Voxel-grid map of an (N,4) cloud on the device: the centroid and the point count of every occupied voxel of the
+    grid with cell size `leaf` (three values or one) anchored at `origin`, voxels ranked by their first point (a
+    frame-major cloud's map grows frame by frame).  Exact integer sums: the result is bit-identical from run to run and
+    under any permutation of the input.  A point with a non-finite value, a key beyond 2^20 cells from the origin on an
+    axis or |intensity| >= 256 belongs to no voxel and sets C.FLAG_NAN / C.FLAG_OVERFLOW in status.
+    Returns (centroids (V,4) in pts' dtype, counts int32[V], point_voxel int32[N] (voxel rank, -1 dropped) or None,
+    status (1) int32)."""
+    f64 = _layout(pts)
+    n, dev = pts.shape[0], pts.device
+    L, O = _grid3(leaf, "leaf"), _grid3(origin, "origin")
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    pv = torch.empty(n, dtype=torch.int32, device=dev) if point_voxel else None
+    if n == 0:
+        return torch.empty((0, 4), dtype=pts.dtype, device=dev), torch.empty(0, dtype=torch.int32, device=dev), pv, status
+    lib = C.lib()
+    ws = torch.empty(int(lib.lmc_voxel_workspace_bytes(n)), dtype=torch.uint8, device=dev)
+    nv = torch.empty(1, dtype=torch.int64, device=dev)
+    ptr = _req(pts, pts.dtype, "pts", (4,))
+    C.check((lib.lmc_voxel_index_f64 if f64 else lib.lmc_voxel_index_f32)(ptr, n, L, O, ws.data_ptr(), nv.data_ptr(), status.data_ptr(),
+                                                                          _stream_ptr()))
+    V = int(nv.item())                                      # the one host sync: the outputs are sized by V
+    cent = torch.empty((V, 4), dtype=pts.dtype, device=dev)
+    counts = torch.empty(V, dtype=torch.int32, device=dev)
+    C.check((lib.lmc_voxel_reduce_f64 if f64 else lib.lmc_voxel_reduce_f32)(ptr, n, L, O, ws.data_ptr(), V, cent.data_ptr(), counts.data_ptr(),
+                                                                            _req(pv, torch.int32, "point_voxel"), _stream_ptr()))
+    return cent, counts, pv, status
+
+
 def _redecide_uncertain(env, pos, Rm, flags, fov_h, fov_v, range_min) -> int:
     """Host re-decision of the points k_scan_mark flagged uncertain (bit 1), with the NumPy calls of LMC:726-745."""
     import numpy as np
