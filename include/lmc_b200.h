@@ -507,6 +507,66 @@ int lmc_voxel_reduce_f32(const float* pts_n4, int64_t n_points, const double lea
                          void* workspace, int64_t n_voxels, float* out_n4, int32_t* counts, int32_t* point_voxel,
                          void* stream);
 
+/*
+ * A prior point map on the device, exact fixed-radius nearest neighbours in it, and per-frame pose refinement against
+ * it (definition: oracle/lmc_oracle_register.py).  The map is the voxel map's grid (leaf, origin, keys: the same f64
+ * expressions) over its points: rows sorted by voxel rank (f64, the original row index beside each), CSR voxel
+ * offsets, and a lookup table key -> rank (open addressing, the power of two >= 2V slots).  The caller builds the
+ * first three from lmc_voxel_index_* / lmc_voxel_reduce_* (ranks, counts, point_voxel) and a stable sort, then fills
+ * the table with lmc_map_build.  Every buffer is device memory and 32-byte aligned (LMC_ERR_ALIGN).
+ *
+ * Nearest (lmc_map_nearest_*): for a query w, its cell k = floor((w - origin) / leaf) and the 27 cells around it;
+ * d = w - m and d2 = (dx dx + dy dy) + dz dz, every operation rounded to nearest (no contraction); accepted when
+ * d2 <= r2 with r2 = max_dist^2 rounded once on the host; the result is the minimum over (d2, original index), so equal
+ * distances go to the smaller index.  max_dist <= min(leaf), so the 27 cells cover the ball.  A query with a
+ * non-finite coordinate or whose cell is outside the key range has no match (index -1, d2 = +inf); a non-finite query
+ * sets LMC_FLAG_NAN in *status.
+ *
+ * Register (lmc_register_frames_*): frame f's points p (sensor frame, rows frame_off[f] .. frame_off[f+1]) and its
+ * pose [R | t] (pose_Rt rows, align_rigid's layout).  Each of `iters` iterations, for every frame not yet done:
+ * a = R p, w = a + t, its nearest map point q as above, and over the inliers r = w - q the 17 sums n, Sa, S aa^T,
+ * Sr, S a x r, S |r|^2; then H = [[n I, -[Sa]x], [[Sa]x, S|a|^2 I - S aa^T]], g = [Sr; S a x r], delta = [tau; phi]
+ * = -H^-1 g by Cholesky, t <- t + tau, R <- Exp(phi) R (about the sensor position).  A frame with n < 6 or a Cholesky
+ * pivot <= 1e-12 trace(H) is DEGENERATE and keeps its pose from then on; one with |tau| <= tol_t and |phi| <= tol_r
+ * (after applying that update) is CONVERGED and stops.  Per frame: inliers (n) and rms_m (sqrt(S|r|^2 / n), NaN for
+ * n = 0) of its last iteration, the iterations it ran, flags.  No float atomics: results are bit-identical run to run
+ * (they depend on the order of the points, which fixes the summation order).
+ *
+ * Refused with LMC_ERR_INVALID before anything is written: NULL required buffers, negative sizes, more than 2^31 - 1
+ * points or map points, n_voxels outside 0 .. n_map_points, a leaf that is not finite and > 0 or an origin that is not
+ * finite, max_dist not finite and > 0 or > min(leaf), iters < 1, tol_t / tol_r not finite and >= 0, n_frames < 1 with
+ * points present.
+ */
+#define LMC_REG_CONVERGED       1
+#define LMC_REG_DEGENERATE      2
+
+typedef struct lmc_point_map {
+    const double*  pts_m4;        /* (n_points, 4) f64 rows sorted by voxel rank                      */
+    const int64_t* index;         /* (n_points) original row of each sorted row                       */
+    const int64_t* vox_off;       /* (n_voxels + 1) CSR offsets of the voxels' rows                    */
+    void*          table;         /* lmc_map_workspace_bytes(n_voxels) bytes: keys u64[cap] | rank u32 */
+    int64_t        n_points;
+    int64_t        n_voxels;
+    double         leaf[3];       /* host values, as the voxel map                                     */
+    double         origin[3];
+} lmc_point_map;
+
+int64_t lmc_map_workspace_bytes(int64_t n_voxels);
+int lmc_map_build(const lmc_point_map* map, void* stream);          /* fills map->table */
+int lmc_map_nearest_f64(const double* pts_n4, int64_t n_points, const lmc_point_map* map, double max_dist,
+                        int64_t* index_out, double* d2_out, uint32_t* status, void* stream);
+int lmc_map_nearest_f32(const float* pts_n4, int64_t n_points, const lmc_point_map* map, double max_dist,
+                        int64_t* index_out, double* d2_out, uint32_t* status, void* stream);
+int64_t lmc_register_workspace_bytes(int64_t n_points, int32_t n_frames);
+int lmc_register_frames_f64(const double* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames,
+                            const double* pose_Rt, const lmc_point_map* map, double max_dist, int32_t iters, double tol_t,
+                            double tol_r, void* workspace, double* pose_out, int32_t* inliers, double* rms_m,
+                            int32_t* iterations, int32_t* flags, uint32_t* status, void* stream);
+int lmc_register_frames_f32(const float* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames,
+                            const double* pose_Rt, const lmc_point_map* map, double max_dist, int32_t iters, double tol_t,
+                            double tol_r, void* workspace, double* pose_out, int32_t* inliers, double* rms_m,
+                            int32_t* iterations, int32_t* flags, uint32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -21,6 +21,7 @@ PCD_TILE = 256
 MAX_PEERS = 7
 LAS_HEADER_BYTES, LAS_RECORD_BYTES = 227, 34
 SCAN_TILE = 256
+REG_CONVERGED, REG_DEGENERATE = 1, 2
 
 vp, i64, i32, f64 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_double
 
@@ -35,6 +36,15 @@ class LmcExport(ctypes.Structure):
         ("status", vp),
         ("n_peers", i32), ("peer_out", vp * 7), ("peer_lvx14", vp * 7),
         ("mc_out", vp), ("mc_lvx14", vp),
+    ]
+
+
+class LmcPointMap(ctypes.Structure):
+    """struct lmc_point_map (include/lmc_b200.h)"""
+    _fields_ = [
+        ("pts_m4", vp), ("index", vp), ("vox_off", vp), ("table", vp),
+        ("n_points", i64), ("n_voxels", i64),
+        ("leaf", ctypes.c_double * 3), ("origin", ctypes.c_double * 3),
     ]
 
 
@@ -100,6 +110,13 @@ _SIGNATURES = {
     "lmc_voxel_index_f32": ([vp, i64, vp, vp, vp, vp, vp, vp], ctypes.c_int),
     "lmc_voxel_reduce_f64": ([vp, i64, vp, vp, vp, i64, vp, vp, vp, vp], ctypes.c_int),
     "lmc_voxel_reduce_f32": ([vp, i64, vp, vp, vp, i64, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_map_workspace_bytes": ([i64], i64),
+    "lmc_map_build": ([vp, vp], ctypes.c_int),
+    "lmc_map_nearest_f64": ([vp, i64, vp, f64, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_map_nearest_f32": ([vp, i64, vp, f64, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_register_workspace_bytes": ([i64, i32], i64),
+    "lmc_register_frames_f64": ([vp, i64, vp, i32, vp, vp, f64, i32, f64, f64, vp, vp, vp, vp, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_register_frames_f32": ([vp, i64, vp, i32, vp, vp, f64, i32, f64, f64, vp, vp, vp, vp, vp, vp, vp, vp], ctypes.c_int),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

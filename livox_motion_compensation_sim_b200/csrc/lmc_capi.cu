@@ -44,6 +44,19 @@ cudaError_t launch_voxel_index(bool f64, const void* pts, int64_t n, const doubl
                                int64_t* n_voxels, uint32_t* status, cudaStream_t st);
 cudaError_t launch_voxel_reduce(bool f64, const void* pts, int64_t n, const double* leaf, const double* origin, void* ws,
                                 int64_t V, void* out, int32_t* counts, int32_t* point_voxel, cudaStream_t st);
+size_t map_table_bytes(int64_t V);
+size_t register_workspace_bytes(int64_t n, int64_t F);
+int64_t register_max_chunks(int64_t n, int64_t F);
+cudaError_t launch_map_build(const double* pts, const int64_t* vox_off, int64_t V, const double* leaf, const double* origin,
+                             void* table, cudaStream_t st);
+cudaError_t launch_map_nearest(bool f64, const void* q, int64_t n, const double* pts, const int64_t* idx, const int64_t* vox_off,
+                               const void* table, int64_t V, const double* leaf, const double* origin, double r2,
+                               int64_t* idx_out, double* d2_out, uint32_t* status, cudaStream_t st);
+cudaError_t launch_register_frames(bool f64, const void* q, int64_t n, const int64_t* frame_off, int64_t F, const double* pose_in,
+                                   const double* pts, const int64_t* idx, const int64_t* vox_off, const void* table, int64_t V,
+                                   const double* leaf, const double* origin, double r2, int32_t iters, double tol_t, double tol_r,
+                                   void* ws, double* pose_out, int32_t* inliers, double* rms, int32_t* iterations, int32_t* flags,
+                                   uint32_t* status, cudaStream_t st);
 }
 
 namespace {
@@ -532,6 +545,107 @@ int lmc_voxel_reduce_f64(const double* pts_n4, int64_t n_points, const double le
 int lmc_voxel_reduce_f32(const float* pts_n4, int64_t n_points, const double leaf[3], const double origin[3], void* workspace,
                          int64_t n_voxels, float* out_n4, int32_t* counts, int32_t* point_voxel, void* stream) {
     return voxel_reduce(false, pts_n4, n_points, leaf, origin, workspace, n_voxels, out_n4, counts, point_voxel, stream);
+}
+
+// ---- point map: lmc_map_build (lookup table), lmc_map_nearest_* (fixed-radius nearest), lmc_register_frames_* -------
+static const int64_t kMax31 = (1LL << 31) - 1;
+static bool finite_d(double v) { return v >= -1.7976931348623157e308 && v <= 1.7976931348623157e308; }
+int64_t lmc_map_workspace_bytes(int64_t n_voxels) {
+    if (n_voxels < 0 || n_voxels > kMax31) return fail(LMC_ERR_INVALID, "n_voxels must be 0 .. 2^31 - 1");
+    return (int64_t)lmc::map_table_bytes(n_voxels);
+}
+static int map_check(const lmc_point_map* m) {
+    int rc = check_device();
+    if (rc != LMC_OK) return rc;
+    if (!m) return fail(LMC_ERR_INVALID, "NULL map");
+    if (m->n_points < 0 || m->n_points > kMax31) return fail(LMC_ERR_INVALID, "map n_points must be 0 .. 2^31 - 1");
+    if (m->n_voxels < 0 || m->n_voxels > m->n_points) return fail(LMC_ERR_INVALID, "map n_voxels must be 0 .. n_points");
+    if (!m->vox_off || !m->table || (m->n_points > 0 && (!m->pts_m4 || !m->index))) return fail(LMC_ERR_INVALID, "NULL map buffer");
+    for (int c = 0; c < 3; ++c) {
+        if (!(m->leaf[c] > 0.0 && finite_d(m->leaf[c]))) return fail(LMC_ERR_INVALID, "leaf[%d] must be finite and > 0", c);
+        if (!finite_d(m->origin[c])) return fail(LMC_ERR_INVALID, "origin[%d] must be finite", c);
+    }
+    if (!aligned32(m->pts_m4) || !aligned32(m->index) || !aligned32(m->vox_off) || !aligned32(m->table))
+        return fail(LMC_ERR_ALIGN, "map buffers must be 32-byte aligned");
+    return LMC_OK;
+}
+// r2 = max_dist^2 rounded once; max_dist <= min(leaf) keeps the ball inside the 27 cells around the query's
+static int gate_check(const lmc_point_map* m, double max_dist, double* r2) {
+    if (!(max_dist > 0.0 && finite_d(max_dist))) return fail(LMC_ERR_INVALID, "max_dist must be finite and > 0");
+    for (int c = 0; c < 3; ++c)
+        if (max_dist > m->leaf[c]) return fail(LMC_ERR_INVALID, "max_dist must be <= min(leaf)");
+    *r2 = max_dist * max_dist;
+    return LMC_OK;
+}
+int lmc_map_build(const lmc_point_map* map, void* stream) {
+    int rc = map_check(map);
+    if (rc != LMC_OK) return rc;
+    cudaError_t e = lmc::launch_map_build(map->pts_m4, map->vox_off, map->n_voxels, map->leaf, map->origin, map->table,
+                                          static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_map_insert");
+}
+static int map_nearest(bool f64, const void* pts, int64_t n, const lmc_point_map* m, double max_dist, int64_t* idx_out, double* d2_out,
+                       uint32_t* status, void* stream) {
+    int rc = map_check(m);
+    if (rc != LMC_OK) return rc;
+    double r2;
+    if ((rc = gate_check(m, max_dist, &r2)) != LMC_OK) return rc;
+    if (n < 0 || n > kMax31) return fail(LMC_ERR_INVALID, "n_points must be 0 .. 2^31 - 1");
+    if (!status || (n > 0 && (!pts || !idx_out || !d2_out))) return fail(LMC_ERR_INVALID, "NULL argument");
+    if (!aligned32(pts) || !aligned32(idx_out) || !aligned32(d2_out)) return fail(LMC_ERR_ALIGN, "points and outputs must be 32-byte aligned");
+    cudaError_t e = lmc::launch_map_nearest(f64, pts, n, m->pts_m4, m->index, m->vox_off, m->table, m->n_voxels, m->leaf, m->origin, r2,
+                                            idx_out, d2_out, status, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_map_nearest");
+}
+int lmc_map_nearest_f64(const double* pts_n4, int64_t n_points, const lmc_point_map* map, double max_dist, int64_t* index_out,
+                        double* d2_out, uint32_t* status, void* stream) {
+    return map_nearest(true, pts_n4, n_points, map, max_dist, index_out, d2_out, status, stream);
+}
+int lmc_map_nearest_f32(const float* pts_n4, int64_t n_points, const lmc_point_map* map, double max_dist, int64_t* index_out,
+                        double* d2_out, uint32_t* status, void* stream) {
+    return map_nearest(false, pts_n4, n_points, map, max_dist, index_out, d2_out, status, stream);
+}
+int64_t lmc_register_workspace_bytes(int64_t n_points, int32_t n_frames) {
+    if (n_points < 0 || n_points > kMax31 || n_frames < 0) return fail(LMC_ERR_INVALID, "n_points must be 0 .. 2^31 - 1, n_frames >= 0");
+    if (lmc::register_max_chunks(n_points, n_frames) > kMax31) return fail(LMC_ERR_INVALID, "more than 2^31 - 1 point chunks");
+    return (int64_t)lmc::register_workspace_bytes(n_points, n_frames);
+}
+static int register_frames(bool f64, const void* pts, int64_t n, const int64_t* frame_off, int32_t F, const double* pose_in,
+                           const lmc_point_map* m, double max_dist, int32_t iters, double tol_t, double tol_r, void* ws, double* pose_out,
+                           int32_t* inliers, double* rms, int32_t* iterations, int32_t* flags, uint32_t* status, void* stream) {
+    int rc = map_check(m);
+    if (rc != LMC_OK) return rc;
+    double r2;
+    if ((rc = gate_check(m, max_dist, &r2)) != LMC_OK) return rc;
+    if (n < 0 || n > kMax31 || F < 0) return fail(LMC_ERR_INVALID, "n_points must be 0 .. 2^31 - 1, n_frames >= 0");
+    if (n > 0 && F < 1) return fail(LMC_ERR_INVALID, "points without frames");
+    if (lmc::register_max_chunks(n, F) > kMax31) return fail(LMC_ERR_INVALID, "more than 2^31 - 1 point chunks");
+    if (iters < 1) return fail(LMC_ERR_INVALID, "iters must be >= 1");
+    if (!(tol_t >= 0.0 && finite_d(tol_t) && tol_r >= 0.0 && finite_d(tol_r))) return fail(LMC_ERR_INVALID, "tol_t / tol_r must be finite and >= 0");
+    if (!frame_off || !ws || !status || (n > 0 && !pts) ||
+        (F > 0 && (!pose_in || !pose_out || !inliers || !rms || !iterations || !flags)))
+        return fail(LMC_ERR_INVALID, "NULL argument");
+    if (!aligned32(pts) || !aligned32(frame_off) || !aligned32(pose_in) || !aligned32(ws) || !aligned32(pose_out) || !aligned32(inliers) ||
+        !aligned32(rms) || !aligned32(iterations) || !aligned32(flags))
+        return fail(LMC_ERR_ALIGN, "buffers must be 32-byte aligned");
+    cudaError_t e = lmc::launch_register_frames(f64, pts, n, frame_off, F, pose_in, m->pts_m4, m->index, m->vox_off, m->table, m->n_voxels,
+                                                m->leaf, m->origin, r2, iters, tol_t, tol_r, ws, pose_out, inliers, rms, iterations, flags,
+                                                status, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_reg_accum / k_reg_solve");
+}
+int lmc_register_frames_f64(const double* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames, const double* pose_Rt,
+                            const lmc_point_map* map, double max_dist, int32_t iters, double tol_t, double tol_r, void* workspace,
+                            double* pose_out, int32_t* inliers, double* rms_m, int32_t* iterations, int32_t* flags, uint32_t* status,
+                            void* stream) {
+    return register_frames(true, pts_n4, n_points, frame_off, n_frames, pose_Rt, map, max_dist, iters, tol_t, tol_r, workspace, pose_out,
+                           inliers, rms_m, iterations, flags, status, stream);
+}
+int lmc_register_frames_f32(const float* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames, const double* pose_Rt,
+                            const lmc_point_map* map, double max_dist, int32_t iters, double tol_t, double tol_r, void* workspace,
+                            double* pose_out, int32_t* inliers, double* rms_m, int32_t* iterations, int32_t* flags, uint32_t* status,
+                            void* stream) {
+    return register_frames(false, pts_n4, n_points, frame_off, n_frames, pose_Rt, map, max_dist, iters, tol_t, tol_r, workspace, pose_out,
+                           inliers, rms_m, iterations, flags, status, stream);
 }
 
 // ---- host-side staging helpers (no device work): the reference hands over / expects lists of small per-frame

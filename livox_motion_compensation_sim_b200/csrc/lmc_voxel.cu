@@ -12,18 +12,15 @@
 //           k_voxel_rank    the rank of every first point into its slot, and the voxel's key by rank
 //   reduce  k_voxel_accum   q_x q_y q_z q_I 1 of every point into its voxel's u64 sums (red.global.add.u64), point_voxel
 //           k_voxel_finalize centroid o_c + (k_c + (S_c / n) 2^-32) L_c and mean intensity (S_I / n) 2^-24, count
-#include "lmc_device.cuh"
+#include "lmc_voxel.cuh"
 
 namespace lmc {
 cudaError_t launch_tile_scan(int64_t* tile_off, int64_t tiles, cudaStream_t st);    // lmc_pcd.cu
 
 constexpr int kVoxTile = 256;                        // points (= threads) per tile of every pass
-constexpr uint64_t kVoxEmpty = ~0ull;                // a packed key has 63 bits: all-ones marks an empty slot
 constexpr uint32_t kVoxNoSlot = ~0u;                 // slot of a dropped point
-constexpr double kVoxKeyLim = 1048576.0;             // |k_c| range: [-2^20, 2^20), 21 bits per axis
 constexpr int kVoxAcc = 5;                           // u64 sums per voxel: q_x q_y q_z q_I n
 
-struct VoxGrid { double o[3], L[3]; };
 struct VoxWs {
     unsigned long long* keys;       // [cap] packed key of the slot, kVoxEmpty
     uint32_t* first;                // [cap] smallest point index in the slot
@@ -36,7 +33,6 @@ struct VoxWs {
 };
 
 static inline size_t vox_align(size_t b) { return (b + 255) & ~size_t(255); }
-static uint64_t vox_cap(int64_t n) { uint64_t c = 64; while (c < 2 * (uint64_t)n) c <<= 1; return c; }
 static VoxWs vox_layout(void* ws, int64_t n, size_t& total) {
     const uint64_t cap = vox_cap(n), tiles = ((uint64_t)n + kVoxTile - 1) / kVoxTile;
     uint8_t* b = static_cast<uint8_t*>(ws);
@@ -55,43 +51,6 @@ static VoxWs vox_layout(void* ws, int64_t n, size_t& total) {
     return W;
 }
 size_t voxel_workspace_bytes(int64_t n) { size_t t; vox_layout(nullptr, n, t); return t; }
-
-template <bool F64>
-__device__ __forceinline__ void vox_load(const void* __restrict__ pts, int64_t i, double (&v)[4]) {
-    if constexpr (F64) ldg256(reinterpret_cast<const double*>(pts) + 4 * i, v[0], v[1], v[2], v[3]);
-    else { const float4 f = __ldg(reinterpret_cast<const float4*>(pts) + i); v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w; }
-}
-
-struct VoxPt { unsigned long long key; unsigned long long q[3]; long long qi; };
-
-// 0 for a kept point, else the flag that drops it (a non-finite value: NAN, before the range checks: OVERFLOW)
-__device__ __forceinline__ uint32_t vox_point(const VoxGrid& G, const double (&v)[4], VoxPt& p) {
-    if (!(isfinite(v[0]) && isfinite(v[1]) && isfinite(v[2]) && isfinite(v[3]))) return LMC_FLAG_NAN;
-    double u[3], k[3];
-    bool ok = fabs(v[3]) < 256.0;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        u[c] = __ddiv_rn(__dsub_rn(v[c], G.o[c]), G.L[c]);
-        k[c] = floor(u[c]);
-        ok &= k[c] >= -kVoxKeyLim && k[c] < kVoxKeyLim;          // (an infinite u fails here)
-    }
-    if (!ok) return LMC_FLAG_OVERFLOW;
-    p.key = 0;
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        p.key |= (unsigned long long)((long long)k[c] + (1 << 20)) << (21 * c);
-        // u - k rounds up to 1.0 for a tiny negative u: the clamp keeps q inside the voxel
-        const unsigned long long q = (unsigned long long)__dmul_rn(__dsub_rn(u[c], k[c]), 4294967296.0);
-        p.q[c] = q < 0xffffffffull ? q : 0xffffffffull;
-    }
-    p.qi = __double2ll_rn(__dmul_rn(v[3], 16777216.0));
-    return 0;
-}
-
-__device__ __forceinline__ uint64_t vox_hash(uint64_t k) {         // murmur3 / splitmix finaliser: neighbouring voxels scatter
-    k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
-    return k;
-}
 
 template <bool F64>
 __global__ void __launch_bounds__(kVoxTile) k_voxel_insert(const void* __restrict__ pts, int64_t n, const VoxGrid G, const VoxWs W,

@@ -521,6 +521,150 @@ def voxel_downsample(pts: torch.Tensor, leaf, origin=(0.0, 0.0, 0.0), *, point_v
     return cent, counts, pv, status
 
 
+@dataclass
+class PointMap:
+    """A prior point map on the device (build_point_map): the map points sorted by voxel on the voxel map's grid, their
+    original rows, CSR voxel offsets and the key -> voxel-rank lookup table (keys int64[cap] | ranks int32[cap], an empty
+    slot has key -1)."""
+    pts: torch.Tensor                # (M,4) f64, sorted by voxel rank
+    index: torch.Tensor              # int64[M] original row
+    vox_off: torch.Tensor            # int64[V+1]
+    table: torch.Tensor              # uint8 lookup table, lmc_map_workspace_bytes(V) bytes
+    leaf: tuple
+    origin: tuple
+
+    @property
+    def n_voxels(self) -> int:
+        return self.vox_off.shape[0] - 1
+
+    @property
+    def keys(self) -> torch.Tensor:
+        cap = self._cap()
+        return self.table[:8 * cap].view(torch.int64)
+
+    @property
+    def ranks(self) -> torch.Tensor:
+        cap = self._cap()
+        b = (8 * cap + 255) // 256 * 256
+        return self.table[b:b + 4 * cap].view(torch.int32)
+
+    def _cap(self) -> int:
+        c = 64
+        while c < 2 * self.n_voxels:
+            c <<= 1
+        return c
+
+    def _c(self) -> "C.LmcPointMap":
+        m = C.LmcPointMap()
+        m.pts_m4, m.index, m.vox_off = self.pts.data_ptr() or None, self.index.data_ptr() or None, self.vox_off.data_ptr()
+        m.table = self.table.data_ptr()
+        m.n_points, m.n_voxels = self.pts.shape[0], self.n_voxels
+        for c in range(3):
+            m.leaf[c], m.origin[c] = self.leaf[c], self.origin[c]
+        return m
+
+
+@_on_tensor_device
+def build_point_map(map_pts: torch.Tensor, leaf, origin=(0.0, 0.0, 0.0)) -> PointMap:
+    """Build a prior point map of the (M,4) cloud `map_pts` on the voxel map's grid (`leaf`: three values or one, anchored
+    at `origin`; keys limited to 2^20 cells from the origin per axis, so a UTM-scale map needs an origin near the data).
+    The voxel ranks and counts come from voxel_downsample, the rows are sorted stably by voxel, and k_map_insert fills
+    the lookup table.  ValueError for a NaN / inf map point, OverflowError for one beyond the key range or with
+    |intensity| >= 256, as voxel_map."""
+    L, O = _grid3(leaf, "leaf"), _grid3(origin, "origin")
+    _, counts, pv, status = voxel_downsample(map_pts, leaf, origin, point_voxel=True)
+    ExportBuffers(status=status).raise_for_flags()
+    dev = map_pts.device
+    order = torch.argsort(pv.long(), stable=True)
+    pts = map_pts.index_select(0, order).to(torch.float64).contiguous()
+    vox_off = torch.zeros(counts.shape[0] + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(counts, 0, out=vox_off[1:])
+    lib = C.lib()
+    table = torch.empty(int(lib.lmc_map_workspace_bytes(counts.shape[0])), dtype=torch.uint8, device=dev)
+    pm = PointMap(pts, order.contiguous(), vox_off, table, tuple(L), tuple(O))
+    m = pm._c()
+    C.check(lib.lmc_map_build(C.ctypes.byref(m), _stream_ptr()))
+    return pm
+
+
+def _gate(pmap: PointMap, max_dist) -> float:
+    d = float(max_dist)
+    if not (d > 0.0 and d < float("inf")) or d > min(pmap.leaf):
+        raise ValueError("max_dist must be finite, > 0 and <= min(leaf): the 27 cells around a query must cover its ball")
+    return d
+
+
+@_on_tensor_device
+def map_nearest(pts: torch.Tensor, pmap: PointMap, max_dist: float):
+    """Exact fixed-radius nearest neighbour of every query row of the (N,4) cloud `pts` in `pmap`: the map point with the
+    smallest d2 = (dx dx + dy dy) + dz dz (f64, every operation rounded to nearest) among those with d2 <= max_dist^2;
+    equal distances go to the smaller original map row.  max_dist <= min(leaf) is required.  A query with a non-finite
+    coordinate (which sets C.FLAG_NAN in status) or outside the key range has no match.
+    Returns (index int64[N] original map row or -1, d2 f64[N] (+inf without a match), status (1) int32)."""
+    f64 = _layout(pts)
+    d = _gate(pmap, max_dist)
+    n, dev = pts.shape[0], pts.device
+    idx = torch.empty(n, dtype=torch.int64, device=dev)
+    d2 = torch.empty(n, dtype=torch.float64, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    m = pmap._c()
+    fn = C.lib().lmc_map_nearest_f64 if f64 else C.lib().lmc_map_nearest_f32
+    C.check(fn(_req(pts, pts.dtype, "pts", (4,)) if n else None, n, C.ctypes.byref(m), d, idx.data_ptr() or None,
+               d2.data_ptr() or None, status.data_ptr(), _stream_ptr()))
+    return idx, d2, status
+
+
+@dataclass
+class RegStats:
+    """Per-frame results of register_frames."""
+    inliers: torch.Tensor            # int32[F] inliers of the last iteration
+    rms_m: torch.Tensor              # f64[F] rms point-to-point residual of the last iteration (NaN without inliers)
+    iterations: torch.Tensor         # int32[F] iterations the frame ran
+    flags: torch.Tensor              # int32[F] C.REG_CONVERGED | C.REG_DEGENERATE
+    status: torch.Tensor             # (1) int32, C.FLAG_NAN for a non-finite point
+
+    @property
+    def converged(self) -> torch.Tensor:
+        return (self.flags & C.REG_CONVERGED) != 0
+
+    @property
+    def degenerate(self) -> torch.Tensor:
+        return (self.flags & C.REG_DEGENERATE) != 0
+
+
+@_on_tensor_device
+def register_frames(pts: torch.Tensor, frame_off: torch.Tensor, pose_Rt: torch.Tensor, pmap: PointMap, max_dist: float,
+                    iters: int = 30, tol_t: float = 1e-9, tol_r: float = 1e-12):
+    """Refine every frame's pose against the map by point-to-point Gauss-Newton on the device.  pts: sensor-frame clouds
+    (raw hold-next scans, or deskew_slerp_local's output), frame-major with CSR frame_off; pose_Rt: the initial (F,12)
+    [R | t] table (align_rigid's layout).  Each iteration pairs every point's w = R p + t with its nearest map point
+    within max_dist (map_nearest's rule), solves the 6x6 normal equations for [tau; phi] (rotation about the sensor
+    position) by Cholesky and applies t += tau, R = Exp(phi) R.  A frame with fewer than 6 inliers or a singular system
+    is degenerate and keeps its pose; one whose step is within tol_t (m) and tol_r (rad) is converged and stops.
+    No float atomics: two calls give identical bytes.  The result is not invariant under a permutation of the points
+    (their order fixes the summation order).  Returns (refined (F,12) f64 pose table, RegStats)."""
+    f64 = _layout(pts)
+    d = _gate(pmap, max_dist)
+    if int(iters) < 1:
+        raise ValueError("iters must be >= 1")
+    n, F, dev = pts.shape[0], frame_off.shape[0] - 1, pts.device
+    if pose_Rt.shape[0] != F:
+        raise ValueError("pose_Rt must have one row per frame")
+    lib = C.lib()
+    ws = torch.empty(max(int(lib.lmc_register_workspace_bytes(n, F)), 1), dtype=torch.uint8, device=dev)
+    pose = torch.empty((F, 12), dtype=torch.float64, device=dev)
+    st = RegStats(torch.empty(F, dtype=torch.int32, device=dev), torch.empty(F, dtype=torch.float64, device=dev),
+                  torch.empty(F, dtype=torch.int32, device=dev), torch.empty(F, dtype=torch.int32, device=dev),
+                  torch.zeros(1, dtype=torch.int32, device=dev))
+    m = pmap._c()
+    fn = lib.lmc_register_frames_f64 if f64 else lib.lmc_register_frames_f32
+    C.check(fn(_req(pts, pts.dtype, "pts", (4,)) if n else None, n, _req(frame_off, torch.int64, "frame_off"), F,
+               _req(pose_Rt, torch.float64, "pose_Rt", (12,)), C.ctypes.byref(m), d, int(iters), float(tol_t), float(tol_r),
+               ws.data_ptr(), pose.data_ptr(), st.inliers.data_ptr(), st.rms_m.data_ptr(), st.iterations.data_ptr(),
+               st.flags.data_ptr(), st.status.data_ptr(), _stream_ptr()))
+    return pose, st
+
+
 def _redecide_uncertain(env, pos, Rm, flags, fov_h, fov_v, range_min) -> int:
     """Host re-decision of the points k_scan_mark flagged uncertain (bit 1), with the NumPy calls of LMC:726-745."""
     import numpy as np

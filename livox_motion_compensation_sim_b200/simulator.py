@@ -67,6 +67,13 @@ class LiDARMotionSimulator:
             # so the point sets and the NumPy noise stream are the reference's.  Needs the device scanner (a frame_source
             # without .scan).
             'motion_distortion': False,
+            # 'measured' (default): the device scanner observes from the measured poses (position_gps / orientation_imu),
+            # as the reference does, and the alignment uses the same poses, so pose noise never reaches the aligned cloud.
+            # 'true': the scanner observes from trajectory['position'] / ['orientation'] (and, with 'motion_distortion',
+            # its sample table comes from those too) while alignment and deskew keep the measured poses: the pose noise
+            # shows in alignment_error, and register_scans can correct it.  Which points a frame sees is then decided at
+            # the true hold-next pose.  Needs the device scanner (a frame_source without .scan).
+            'scan_pose_source': 'measured',
             # False (default): results are ordinary NumPy arrays -- D2H into one reusable pinned staging buffer, then a threaded
             # copy (lmc_host_copy); nothing stays page-locked behind the caller's back.
             # True: opt-in throughput knob -- results ARE page-locked blocks of torch's caching host allocator (no second copy:
@@ -221,6 +228,13 @@ class LiDARMotionSimulator:
         if distort and hasattr(frame_source, 'scan'):
             raise ValueError("motion_distortion needs the device scanner: a frame_source with its own .scan has no environment "
                              "rows to observe from other poses")
+        source = self.config.get('scan_pose_source', 'measured')
+        if source not in ('measured', 'true'):
+            raise ValueError("scan_pose_source must be 'measured' or 'true'")
+        if source == 'true' and hasattr(frame_source, 'scan'):
+            raise ValueError("scan_pose_source 'true' needs the device scanner: a frame_source with its own .scan observes "
+                             "from the poses it is given")
+        scan_keys = ('position', 'orientation') if source == 'true' else ('position_gps', 'orientation_imu')
         trajectory = frame_source.trajectory
         lidar_times = FR.lidar_frame_times(self.config['duration'], self.config['lidar_fps'])
         _, pose_idx = self.lookup_frame_poses(trajectory, lidar_times)
@@ -230,11 +244,11 @@ class LiDARMotionSimulator:
         if not hasattr(frame_source, 'scan'):           # no host scanner supplied: scan every frame on the device (N4)
             motion = None
             if distort:                                 # the pose samples the deskews read (_deskew_inputs), one table
-                s_ts_d, seg = self._slerp_samples(trajectory)
+                s_ts_d, seg = self._slerp_samples(trajectory, scan_keys)
                 motion = (s_ts_d, seg, np.round(np.asarray(lidar_times, np.float64) * 1e9).astype(np.int64),
                           int(round(1e9 / float(self.config['lidar_fps']))))
-            device_scans = self.scan_all(frame_source.environment, trajectory['position_gps'][pose_idx],
-                                         trajectory['orientation_imu'][pose_idx], keep_device=True, motion=motion)
+            device_scans = self.scan_all(frame_source.environment, trajectory[scan_keys[0]][pose_idx],
+                                         trajectory[scan_keys[1]][pose_idx], keep_device=True, motion=motion)
         scan_motion = getattr(self, 'last_scan_motion', None) if distort else None
         scan_off = self._dev_scan[1] if scan_motion is not None else None
         for i, t in enumerate(lidar_times):
@@ -251,7 +265,7 @@ class LiDARMotionSimulator:
         dev_scan = getattr(self, '_dev_scan', None) if device_scans is not None else None
         self._dev_scan = None
         if self.config.get('pose_interpolation', 'hold_next') == 'slerp':
-            aligned = self.deskew_scans(all_scans, trajectory, _device_raw=dev_scan, _samples=motion[:2] if distort else None)
+            aligned = self.deskew_scans(all_scans, trajectory, _device_raw=dev_scan, _samples=motion[:2] if distort and source == 'measured' else None)
         elif dev_scan is not None and self._np_dtype() == np.float64 and dev_scan[0].shape[0] > 0:
             # the scans are still resident: align them where they are (no flatten, no second upload)
             raw_d, off = dev_scan
@@ -286,14 +300,14 @@ class LiDARMotionSimulator:
         self.last_merged, self.last_frame_off, self.last_export = merged, off, bufs
         return FR.split_frames(merged, off)
 
-    def _slerp_samples(self, trajectory: Dict):
-        """The pose samples of Mode C on the device: the trajectory's GPS positions / IMU orientations at their own times
-        -> (int64 ns sample times, the (S,22) pose-segment table)."""
+    def _slerp_samples(self, trajectory: Dict, keys=('position_gps', 'orientation_imu')):
+        """The pose samples of Mode C on the device: the trajectory's GPS positions / IMU orientations (or the `keys`
+        given) at their own times -> (int64 ns sample times, the (S,22) pose-segment table)."""
         from scipy.spatial.transform import Rotation
         s_ts = np.round(np.asarray(trajectory['time'], np.float64) * 1e9).astype(np.int64)
-        quat = Rotation.from_euler('xyz', np.asarray(trajectory['orientation_imu'], np.float64)).as_quat()
+        quat = Rotation.from_euler('xyz', np.asarray(trajectory[keys[1]], np.float64)).as_quat()
         s_ts_d = self._to_dev(s_ts)
-        seg = ops.build_slerp_table(self._to_dev(quat), self._to_dev(np.asarray(trajectory['position_gps'], np.float64)), s_ts_d)
+        seg = ops.build_slerp_table(self._to_dev(quat), self._to_dev(np.asarray(trajectory[keys[0]], np.float64)), s_ts_d)
         return s_ts_d, seg
 
     def _deskew_inputs(self, raw_scans: List[dict], trajectory: Dict, _device_raw=None, _samples=None):
@@ -366,6 +380,7 @@ class LiDARMotionSimulator:
                 raise bad_ref
             ref_ts = ref_ts.astype(np.int64)
         ref_pose = ops.slerp_pose_at(s_ts_d, seg, self._to_dev(ref_ts))
+        self.last_ref_pose = ref_pose
         out, bufs = ops.deskew_slerp_local(flat_d, self._to_dev(ts), self._to_dev(off), self._to_dev(fstart), s_ts_d, seg, ref_pose,
                                            export=export)
         self.last_merged, self.last_frame_off, self.last_export = self._to_host(out), off, bufs
@@ -411,6 +426,47 @@ class LiDARMotionSimulator:
         cent, counts, _, status = ops.voxel_downsample(self._to_dev(pts), leaf, origin)
         ops.ExportBuffers(status=status).raise_for_flags()
         return {'points': self._to_host(cent), 'counts': counts.cpu().numpy()}
+
+    def register_scans(self, results, leaf=1.0, max_dist=1.0, iters=30, map_points=None, origin=None) -> Dict:
+        """Refine every frame's pose against a prior point map on the device (ops.build_point_map + ops.register_frames:
+        exact nearest neighbours within max_dist, point-to-point Gauss-Newton) and re-align the run with the refined poses.
+        The map defaults to results['environment'] (the prior map) on a grid of edge `leaf` anchored at `origin` (default:
+        the first frame's pose, so UTM-scale maps keep their keys in range); max_dist <= leaf.  A 'hold_next' run
+        registers its raw scans from their hold-next measured poses; a 'slerp' run registers deskew_scans_local(reference=
+        'end') from the Mode C poses at the frames' last point times.  Returns a new results dict: the raw scans untouched,
+        'aligned_pointclouds' = ops.align_rigid of those clouds with the refined poses, and 'registration': {'position'
+        (F,3), 'rotation' (F,3,3), 'inliers', 'rms_m', 'iterations', 'converged', 'degenerate'} (per frame; a frame with
+        fewer than 6 inliers is degenerate and keeps its pose).  alignment_error and voxel_map work on it unchanged."""
+        scans = results['raw_scans']
+        env = results.get('environment') if map_points is None else map_points
+        if env is None:
+            raise ValueError("register_scans needs a map: pass map_points, or a run whose results carry 'environment'")
+        if self.config.get('pose_interpolation', 'hold_next') == 'slerp':
+            local = self.deskew_scans_local(scans, results['trajectory'], reference='end')
+            off = FR.frame_offsets(local)
+            flat = self.last_merged
+            pose0 = self.last_ref_pose if int(off[-1]) else self._to_dev(np.zeros((len(scans), 12)))
+        else:
+            flat, off = FR.flatten_frames([s['points_local'] for s in scans], np.float64)
+            pose0 = self._to_dev(FR.pose_table(np.array([s['sensor_pose']['position'] for s in scans], np.float64).reshape(-1, 3),
+                                               np.array([s['sensor_pose']['orientation'] for s in scans], np.float64).reshape(-1, 3)))
+        if origin is None:
+            origin = tuple(float(v) for v in scans[0]['sensor_pose']['position']) if scans else (0.0, 0.0, 0.0)
+        pmap = ops.build_point_map(self._to_dev(np.asarray(env, np.float64).reshape(-1, 4)), leaf, origin)
+        pts_d = self._to_dev(np.asarray(flat, np.float64).reshape(-1, 4))
+        off_d = self._to_dev(off)
+        pose, st = ops.register_frames(pts_d, off_d, pose0, pmap, max_dist, iters=iters)
+        ops.ExportBuffers(status=st.status).raise_for_flags()
+        if int(off[-1]):
+            out, _ = ops.align_rigid(pts_d if self._np_dtype() == np.float64 else pts_d.float(), off_d, pose)
+            self.last_merged, self.last_frame_off, self.last_export = self._to_host(out), off, None
+        else:
+            self.last_merged, self.last_frame_off, self.last_export = np.zeros((0, 4), self._np_dtype()), off, None
+        ph = pose.cpu().numpy()
+        reg = {'position': ph[:, 9:12].copy(), 'rotation': ph[:, :9].reshape(-1, 3, 3).copy(),
+               'inliers': st.inliers.cpu().numpy(), 'rms_m': st.rms_m.cpu().numpy(), 'iterations': st.iterations.cpu().numpy(),
+               'converged': st.converged.cpu().numpy(), 'degenerate': st.degenerate.cpu().numpy()}
+        return dict(results, aligned_pointclouds=FR.split_frames(self.last_merged, off), registration=reg)
 
     # ------------------------------------------------------------------ (a3) LMC:886-899
     def _merge_flags(self, results):
