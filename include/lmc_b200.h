@@ -567,6 +567,43 @@ int lmc_register_frames_f32(const float* pts_n4, int64_t n_points, const int64_t
                             double tol_r, void* workspace, double* pose_out, int32_t* inliers, double* rms_m,
                             int32_t* iterations, int32_t* flags, uint32_t* status, void* stream);
 
+/*
+ * Normals of a point map (lmc_map_normals; definition: oracle/lmc_oracle_plane.py), one row per map row in the map's
+ * sorted row order.  The neighbours of row p are every map row m with d2 <= r2 (r2 = radius^2 rounded once, d2 as in
+ * lmc_map_nearest, the row itself included), visited in a fixed order: the 27 cells in dz, dy, dx order, then the
+ * rows of each cell in sorted order.  With d = m - p (formed first, so map-scale coordinates never enter a sum), the
+ * sequential sums S d and S dd^T give mu = S d / n and C = S dd^T / n - mu mu^T.  C is diagonalised by cyclic Jacobi
+ * rotations in the pair order (0,1), (0,2), (1,2), a rotation skipped when its off-diagonal entry is exactly 0, until
+ * a sweep leaves every off-diagonal at 0 (at most 32 sweeps).  Every operation is an IEEE-rounded + - x / sqrt, so
+ * the result is bit-identical to its NumPy restatement.  The eigenvalues are sorted ascending (ties in index order) and clamped at 0; the row is
+ * (nx, ny, nz, planarity): the unit eigenvector of lambda_min with its largest-magnitude component positive (the first
+ * on a tie), and planarity = (lambda_mid - lambda_min) / lambda_max (about 1 on a plane, about 0 on a line or a blob).
+ * A row with fewer than min_neighbours neighbours or lambda_max = 0 is (NaN, NaN, NaN, 0).  neighbours (may be NULL):
+ * each row's neighbour count.  Refused with LMC_ERR_INVALID before anything is written: everything lmc_map_build
+ * refuses, radius not finite and > 0 or > min(leaf), min_neighbours < 3, NULL normals for a map with points.
+ *
+ * Point-to-plane registration (lmc_register_frames_plane_*): lmc_register_frames_*'s iteration with the residual along
+ * the nearest map row's normal.  A point is an inlier when its nearest map row q (within max_dist) has planarity >=
+ * min_planarity; then e = (nx rx + ny ry) + nz rz with r = w - q, J = [n; a x n], and the 29 sums n, H = S J J^T,
+ * g = S J e, S e^2 give delta = -H^-1 g.  Degenerate, converged, the update and the outputs are as point-to-point;
+ * rms_m is the rms plane distance.  A frame that sees planes of one orientation only (ground alone) is DEGENERATE and
+ * keeps its pose.  Refused as lmc_register_frames_*, and also for min_planarity outside (0, 1] or NULL normals for a
+ * map with points.  The workspace is lmc_register_plane_workspace_bytes(n_points, n_frames).
+ */
+int lmc_map_normals(const lmc_point_map* map, double radius, int32_t min_neighbours, double* normals_m4, int32_t* neighbours,
+                    void* stream);
+int64_t lmc_register_plane_workspace_bytes(int64_t n_points, int32_t n_frames);
+int lmc_register_frames_plane_f64(const double* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames,
+                                  const double* pose_Rt, const lmc_point_map* map, const double* normals_m4, double max_dist,
+                                  double min_planarity, int32_t iters, double tol_t, double tol_r, void* workspace,
+                                  double* pose_out, int32_t* inliers, double* rms_m, int32_t* iterations, int32_t* flags,
+                                  uint32_t* status, void* stream);
+int lmc_register_frames_plane_f32(const float* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames,
+                                  const double* pose_Rt, const lmc_point_map* map, const double* normals_m4, double max_dist,
+                                  double min_planarity, int32_t iters, double tol_t, double tol_r, void* workspace,
+                                  double* pose_out, int32_t* inliers, double* rms_m, int32_t* iterations, int32_t* flags,
+                                  uint32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -117,6 +117,10 @@ _SIGNATURES = {
     "lmc_register_workspace_bytes": ([i64, i32], i64),
     "lmc_register_frames_f64": ([vp, i64, vp, i32, vp, vp, f64, i32, f64, f64, vp, vp, vp, vp, vp, vp, vp, vp], ctypes.c_int),
     "lmc_register_frames_f32": ([vp, i64, vp, i32, vp, vp, f64, i32, f64, f64, vp, vp, vp, vp, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_map_normals": ([vp, f64, i32, vp, vp, vp], ctypes.c_int),
+    "lmc_register_plane_workspace_bytes": ([i64, i32], i64),
+    "lmc_register_frames_plane_f64": ([vp, i64, vp, i32, vp, vp, vp, f64, f64, i32, f64, f64, vp, vp, vp, vp, vp, vp, vp, vp], ctypes.c_int),
+    "lmc_register_frames_plane_f32": ([vp, i64, vp, i32, vp, vp, vp, f64, f64, i32, f64, f64, vp, vp, vp, vp, vp, vp, vp, vp], ctypes.c_int),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

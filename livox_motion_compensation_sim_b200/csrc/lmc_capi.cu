@@ -57,6 +57,16 @@ cudaError_t launch_register_frames(bool f64, const void* q, int64_t n, const int
                                    const double* leaf, const double* origin, double r2, int32_t iters, double tol_t, double tol_r,
                                    void* ws, double* pose_out, int32_t* inliers, double* rms, int32_t* iterations, int32_t* flags,
                                    uint32_t* status, cudaStream_t st);
+size_t register_plane_workspace_bytes(int64_t n, int64_t F);
+cudaError_t launch_map_normals(const double* pts, const int64_t* idx, const int64_t* vox_off, const void* table, int64_t M_rows,
+                               int64_t V, const double* leaf, const double* origin, double r2, int32_t min_nb, double* normals,
+                               int32_t* neighbours, cudaStream_t st);
+cudaError_t launch_register_frames_plane(bool f64, const void* q, int64_t n, const int64_t* frame_off, int64_t F, const double* pose_in,
+                                         const double* pts, const int64_t* idx, const int64_t* vox_off, const void* table, int64_t V,
+                                         const double* leaf, const double* origin, double r2, const double* normals,
+                                         double min_planarity, int32_t iters, double tol_t, double tol_r, void* ws, double* pose_out,
+                                         int32_t* inliers, double* rms, int32_t* iterations, int32_t* flags, uint32_t* status,
+                                         cudaStream_t st);
 }
 
 namespace {
@@ -570,10 +580,10 @@ static int map_check(const lmc_point_map* m) {
     return LMC_OK;
 }
 // r2 = max_dist^2 rounded once; max_dist <= min(leaf) keeps the ball inside the 27 cells around the query's
-static int gate_check(const lmc_point_map* m, double max_dist, double* r2) {
-    if (!(max_dist > 0.0 && finite_d(max_dist))) return fail(LMC_ERR_INVALID, "max_dist must be finite and > 0");
+static int gate_check(const lmc_point_map* m, double max_dist, double* r2, const char* name = "max_dist") {
+    if (!(max_dist > 0.0 && finite_d(max_dist))) return fail(LMC_ERR_INVALID, "%s must be finite and > 0", name);
     for (int c = 0; c < 3; ++c)
-        if (max_dist > m->leaf[c]) return fail(LMC_ERR_INVALID, "max_dist must be <= min(leaf)");
+        if (max_dist > m->leaf[c]) return fail(LMC_ERR_INVALID, "%s must be <= min(leaf)", name);
     *r2 = max_dist * max_dist;
     return LMC_OK;
 }
@@ -610,13 +620,13 @@ int64_t lmc_register_workspace_bytes(int64_t n_points, int32_t n_frames) {
     if (lmc::register_max_chunks(n_points, n_frames) > kMax31) return fail(LMC_ERR_INVALID, "more than 2^31 - 1 point chunks");
     return (int64_t)lmc::register_workspace_bytes(n_points, n_frames);
 }
-static int register_frames(bool f64, const void* pts, int64_t n, const int64_t* frame_off, int32_t F, const double* pose_in,
-                           const lmc_point_map* m, double max_dist, int32_t iters, double tol_t, double tol_r, void* ws, double* pose_out,
-                           int32_t* inliers, double* rms, int32_t* iterations, int32_t* flags, uint32_t* status, void* stream) {
+// The arguments both metrics refuse, before anything is written.
+static int register_check(const void* pts, int64_t n, const int64_t* frame_off, int32_t F, const double* pose_in, const lmc_point_map* m,
+                          double max_dist, int32_t iters, double tol_t, double tol_r, void* ws, double* pose_out, int32_t* inliers,
+                          double* rms, int32_t* iterations, int32_t* flags, uint32_t* status, double* r2) {
     int rc = map_check(m);
     if (rc != LMC_OK) return rc;
-    double r2;
-    if ((rc = gate_check(m, max_dist, &r2)) != LMC_OK) return rc;
+    if ((rc = gate_check(m, max_dist, r2)) != LMC_OK) return rc;
     if (n < 0 || n > kMax31 || F < 0) return fail(LMC_ERR_INVALID, "n_points must be 0 .. 2^31 - 1, n_frames >= 0");
     if (n > 0 && F < 1) return fail(LMC_ERR_INVALID, "points without frames");
     if (lmc::register_max_chunks(n, F) > kMax31) return fail(LMC_ERR_INVALID, "more than 2^31 - 1 point chunks");
@@ -628,6 +638,15 @@ static int register_frames(bool f64, const void* pts, int64_t n, const int64_t* 
     if (!aligned32(pts) || !aligned32(frame_off) || !aligned32(pose_in) || !aligned32(ws) || !aligned32(pose_out) || !aligned32(inliers) ||
         !aligned32(rms) || !aligned32(iterations) || !aligned32(flags))
         return fail(LMC_ERR_ALIGN, "buffers must be 32-byte aligned");
+    return LMC_OK;
+}
+static int register_frames(bool f64, const void* pts, int64_t n, const int64_t* frame_off, int32_t F, const double* pose_in,
+                           const lmc_point_map* m, double max_dist, int32_t iters, double tol_t, double tol_r, void* ws, double* pose_out,
+                           int32_t* inliers, double* rms, int32_t* iterations, int32_t* flags, uint32_t* status, void* stream) {
+    double r2;
+    int rc = register_check(pts, n, frame_off, F, pose_in, m, max_dist, iters, tol_t, tol_r, ws, pose_out, inliers, rms, iterations, flags,
+                            status, &r2);
+    if (rc != LMC_OK) return rc;
     cudaError_t e = lmc::launch_register_frames(f64, pts, n, frame_off, F, pose_in, m->pts_m4, m->index, m->vox_off, m->table, m->n_voxels,
                                                 m->leaf, m->origin, r2, iters, tol_t, tol_r, ws, pose_out, inliers, rms, iterations, flags,
                                                 status, static_cast<cudaStream_t>(stream));
@@ -646,6 +665,55 @@ int lmc_register_frames_f32(const float* pts_n4, int64_t n_points, const int64_t
                             void* stream) {
     return register_frames(false, pts_n4, n_points, frame_off, n_frames, pose_Rt, map, max_dist, iters, tol_t, tol_r, workspace, pose_out,
                            inliers, rms_m, iterations, flags, status, stream);
+}
+
+int lmc_map_normals(const lmc_point_map* map, double radius, int32_t min_neighbours, double* normals_m4, int32_t* neighbours,
+                    void* stream) {
+    int rc = map_check(map);
+    if (rc != LMC_OK) return rc;
+    double r2;
+    if ((rc = gate_check(map, radius, &r2, "radius")) != LMC_OK) return rc;
+    if (min_neighbours < 3) return fail(LMC_ERR_INVALID, "min_neighbours must be >= 3");
+    if (map->n_points > 0 && !normals_m4) return fail(LMC_ERR_INVALID, "NULL normals");
+    if (!aligned32(normals_m4) || !aligned32(neighbours)) return fail(LMC_ERR_ALIGN, "normals and neighbours must be 32-byte aligned");
+    cudaError_t e = lmc::launch_map_normals(map->pts_m4, map->index, map->vox_off, map->table, map->n_points, map->n_voxels, map->leaf,
+                                            map->origin, r2, min_neighbours, normals_m4, neighbours, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_map_normals");
+}
+int64_t lmc_register_plane_workspace_bytes(int64_t n_points, int32_t n_frames) {
+    if (n_points < 0 || n_points > kMax31 || n_frames < 0) return fail(LMC_ERR_INVALID, "n_points must be 0 .. 2^31 - 1, n_frames >= 0");
+    if (lmc::register_max_chunks(n_points, n_frames) > kMax31) return fail(LMC_ERR_INVALID, "more than 2^31 - 1 point chunks");
+    return (int64_t)lmc::register_plane_workspace_bytes(n_points, n_frames);
+}
+static int register_frames_plane(bool f64, const void* pts, int64_t n, const int64_t* frame_off, int32_t F, const double* pose_in,
+                                 const lmc_point_map* m, const double* normals, double max_dist, double min_planarity, int32_t iters,
+                                 double tol_t, double tol_r, void* ws, double* pose_out, int32_t* inliers, double* rms, int32_t* iterations,
+                                 int32_t* flags, uint32_t* status, void* stream) {
+    double r2;
+    int rc = register_check(pts, n, frame_off, F, pose_in, m, max_dist, iters, tol_t, tol_r, ws, pose_out, inliers, rms, iterations, flags,
+                            status, &r2);
+    if (rc != LMC_OK) return rc;
+    if (!(min_planarity > 0.0 && min_planarity <= 1.0)) return fail(LMC_ERR_INVALID, "min_planarity must be in (0, 1]");
+    if (m->n_points > 0 && !normals) return fail(LMC_ERR_INVALID, "NULL normals");
+    if (!aligned32(normals)) return fail(LMC_ERR_ALIGN, "normals must be 32-byte aligned");
+    cudaError_t e = lmc::launch_register_frames_plane(f64, pts, n, frame_off, F, pose_in, m->pts_m4, m->index, m->vox_off, m->table,
+                                                      m->n_voxels, m->leaf, m->origin, r2, normals, min_planarity, iters, tol_t, tol_r, ws,
+                                                      pose_out, inliers, rms, iterations, flags, status, static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? LMC_OK : cuda_fail(e, "k_reg_accum_plane / k_reg_solve_plane");
+}
+int lmc_register_frames_plane_f64(const double* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames, const double* pose_Rt,
+                                  const lmc_point_map* map, const double* normals_m4, double max_dist, double min_planarity, int32_t iters,
+                                  double tol_t, double tol_r, void* workspace, double* pose_out, int32_t* inliers, double* rms_m,
+                                  int32_t* iterations, int32_t* flags, uint32_t* status, void* stream) {
+    return register_frames_plane(true, pts_n4, n_points, frame_off, n_frames, pose_Rt, map, normals_m4, max_dist, min_planarity, iters, tol_t,
+                                 tol_r, workspace, pose_out, inliers, rms_m, iterations, flags, status, stream);
+}
+int lmc_register_frames_plane_f32(const float* pts_n4, int64_t n_points, const int64_t* frame_off, int32_t n_frames, const double* pose_Rt,
+                                  const lmc_point_map* map, const double* normals_m4, double max_dist, double min_planarity, int32_t iters,
+                                  double tol_t, double tol_r, void* workspace, double* pose_out, int32_t* inliers, double* rms_m,
+                                  int32_t* iterations, int32_t* flags, uint32_t* status, void* stream) {
+    return register_frames_plane(false, pts_n4, n_points, frame_off, n_frames, pose_Rt, map, normals_m4, max_dist, min_planarity, iters, tol_t,
+                                 tol_r, workspace, pose_out, inliers, rms_m, iterations, flags, status, stream);
 }
 
 // ---- host-side staging helpers (no device work): the reference hands over / expects lists of small per-frame

@@ -618,7 +618,7 @@ def map_nearest(pts: torch.Tensor, pmap: PointMap, max_dist: float):
 class RegStats:
     """Per-frame results of register_frames."""
     inliers: torch.Tensor            # int32[F] inliers of the last iteration
-    rms_m: torch.Tensor              # f64[F] rms point-to-point residual of the last iteration (NaN without inliers)
+    rms_m: torch.Tensor              # f64[F] rms residual (point-to-point, or plane distance) of the last iteration (NaN without inliers)
     iterations: torch.Tensor         # int32[F] iterations the frame ran
     flags: torch.Tensor              # int32[F] C.REG_CONVERGED | C.REG_DEGENERATE
     status: torch.Tensor             # (1) int32, C.FLAG_NAN for a non-finite point
@@ -632,9 +632,38 @@ class RegStats:
         return (self.flags & C.REG_DEGENERATE) != 0
 
 
+# On the C3 environment at a 2 m radius, rows below planarity 0.1 are near-collinear neighbourhoods (sparse ground rows
+# with a handful of neighbours) whose smallest eigenvector is not the surface normal.
+MIN_PLANARITY = 0.1
+
+
+@_on_tensor_device
+def estimate_normals(pmap: PointMap, radius: float, min_neighbours: int = 5):
+    """Surface normal and planarity of every map row on the device (k_map_normals): the covariance of the map rows within
+    `radius` (<= min(leaf); the row itself included), its eigenvector of the smallest eigenvalue (cyclic Jacobi from
+    IEEE-rounded operations only, so bit-identical to its NumPy restatement) with the largest-magnitude component
+    positive, and planarity = (l_mid - l_min) / l_max (about 1 on a plane, about 0 on a line or a blob).  Rows are in
+    the map's sorted row order: row i belongs to pmap.pts[i], whose original row is pmap.index[i].  A row with fewer
+    than `min_neighbours` (>= 3) neighbours, or whose neighbours all coincide, is (NaN, NaN, NaN, 0).
+    Returns (normals (M,4) f64 (nx, ny, nz, planarity), neighbours int32[M])."""
+    d = float(radius)
+    if not (d > 0.0 and d < float("inf")) or d > min(pmap.leaf):
+        raise ValueError("radius must be finite, > 0 and <= min(leaf): the 27 cells around a row must cover its ball")
+    if int(min_neighbours) < 3:
+        raise ValueError("min_neighbours must be >= 3")
+    M, dev = pmap.pts.shape[0], pmap.pts.device
+    normals = torch.empty((M, 4), dtype=torch.float64, device=dev)
+    nb = torch.empty(M, dtype=torch.int32, device=dev)
+    m = pmap._c()
+    C.check(C.lib().lmc_map_normals(C.ctypes.byref(m), d, int(min_neighbours), normals.data_ptr() or None, nb.data_ptr() or None,
+                                    _stream_ptr()))
+    return normals, nb
+
+
 @_on_tensor_device
 def register_frames(pts: torch.Tensor, frame_off: torch.Tensor, pose_Rt: torch.Tensor, pmap: PointMap, max_dist: float,
-                    iters: int = 30, tol_t: float = 1e-9, tol_r: float = 1e-12):
+                    iters: int = 30, tol_t: float = 1e-9, tol_r: float = 1e-12, *, normals: Optional[torch.Tensor] = None,
+                    min_planarity: float = MIN_PLANARITY):
     """Refine every frame's pose against the map by point-to-point Gauss-Newton on the device.  pts: sensor-frame clouds
     (raw hold-next scans, or deskew_slerp_local's output), frame-major with CSR frame_off; pose_Rt: the initial (F,12)
     [R | t] table (align_rigid's layout).  Each iteration pairs every point's w = R p + t with its nearest map point
@@ -642,7 +671,11 @@ def register_frames(pts: torch.Tensor, frame_off: torch.Tensor, pose_Rt: torch.T
     position) by Cholesky and applies t += tau, R = Exp(phi) R.  A frame with fewer than 6 inliers or a singular system
     is degenerate and keeps its pose; one whose step is within tol_t (m) and tol_r (rad) is converged and stops.
     No float atomics: two calls give identical bytes.  The result is not invariant under a permutation of the points
-    (their order fixes the summation order).  Returns (refined (F,12) f64 pose table, RegStats)."""
+    (their order fixes the summation order).
+    normals (estimate_normals(pmap, ...)[0]) selects point-to-plane: the residual is the distance along the nearest map
+    row's normal, and only map rows with planarity >= min_planarity (in (0, 1]) pair; rms_m is then the rms plane
+    distance.  A frame that sees one plane orientation only (ground alone) is degenerate under this metric.
+    Returns (refined (F,12) f64 pose table, RegStats)."""
     f64 = _layout(pts)
     d = _gate(pmap, max_dist)
     if int(iters) < 1:
@@ -651,12 +684,26 @@ def register_frames(pts: torch.Tensor, frame_off: torch.Tensor, pose_Rt: torch.T
     if pose_Rt.shape[0] != F:
         raise ValueError("pose_Rt must have one row per frame")
     lib = C.lib()
-    ws = torch.empty(max(int(lib.lmc_register_workspace_bytes(n, F)), 1), dtype=torch.uint8, device=dev)
+    if normals is not None:
+        if not (0.0 < float(min_planarity) <= 1.0):
+            raise ValueError("min_planarity must be in (0, 1]")
+        if tuple(normals.shape) != (pmap.pts.shape[0], 4):
+            raise ValueError("normals must have one (4,) row per map row (estimate_normals)")
+        ws = torch.empty(max(int(lib.lmc_register_plane_workspace_bytes(n, F)), 1), dtype=torch.uint8, device=dev)
+    else:
+        ws = torch.empty(max(int(lib.lmc_register_workspace_bytes(n, F)), 1), dtype=torch.uint8, device=dev)
     pose = torch.empty((F, 12), dtype=torch.float64, device=dev)
     st = RegStats(torch.empty(F, dtype=torch.int32, device=dev), torch.empty(F, dtype=torch.float64, device=dev),
                   torch.empty(F, dtype=torch.int32, device=dev), torch.empty(F, dtype=torch.int32, device=dev),
                   torch.zeros(1, dtype=torch.int32, device=dev))
     m = pmap._c()
+    if normals is not None:
+        fn = lib.lmc_register_frames_plane_f64 if f64 else lib.lmc_register_frames_plane_f32
+        C.check(fn(_req(pts, pts.dtype, "pts", (4,)) if n else None, n, _req(frame_off, torch.int64, "frame_off"), F,
+                   _req(pose_Rt, torch.float64, "pose_Rt", (12,)), C.ctypes.byref(m), _req(normals, torch.float64, "normals", (4,)), d,
+                   float(min_planarity), int(iters), float(tol_t), float(tol_r), ws.data_ptr(), pose.data_ptr(), st.inliers.data_ptr(),
+                   st.rms_m.data_ptr(), st.iterations.data_ptr(), st.flags.data_ptr(), st.status.data_ptr(), _stream_ptr()))
+        return pose, st
     fn = lib.lmc_register_frames_f64 if f64 else lib.lmc_register_frames_f32
     C.check(fn(_req(pts, pts.dtype, "pts", (4,)) if n else None, n, _req(frame_off, torch.int64, "frame_off"), F,
                _req(pose_Rt, torch.float64, "pose_Rt", (12,)), C.ctypes.byref(m), d, int(iters), float(tol_t), float(tol_r),

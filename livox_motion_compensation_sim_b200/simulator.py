@@ -427,9 +427,13 @@ class LiDARMotionSimulator:
         ops.ExportBuffers(status=status).raise_for_flags()
         return {'points': self._to_host(cent), 'counts': counts.cpu().numpy()}
 
-    def register_scans(self, results, leaf=1.0, max_dist=1.0, iters=30, map_points=None, origin=None) -> Dict:
+    def register_scans(self, results, leaf=1.0, max_dist=1.0, iters=30, map_points=None, origin=None, metric='point',
+                       normal_radius=None, min_planarity=ops.MIN_PLANARITY) -> Dict:
         """Refine every frame's pose against a prior point map on the device (ops.build_point_map + ops.register_frames:
-        exact nearest neighbours within max_dist, point-to-point Gauss-Newton) and re-align the run with the refined poses.
+        exact nearest neighbours within max_dist, Gauss-Newton) and re-align the run with the refined poses.  metric
+        'point' minimises point-to-point distances; 'plane' estimates the map's normals within normal_radius (default
+        min(leaf); ops.estimate_normals) and minimises the distances along them, pairing only map rows with planarity >=
+        min_planarity.
         The map defaults to results['environment'] (the prior map) on a grid of edge `leaf` anchored at `origin` (default:
         the first frame's pose, so UTM-scale maps keep their keys in range); max_dist <= leaf.  A 'hold_next' run
         registers its raw scans from their hold-next measured poses; a 'slerp' run registers deskew_scans_local(reference=
@@ -437,6 +441,8 @@ class LiDARMotionSimulator:
         'aligned_pointclouds' = ops.align_rigid of those clouds with the refined poses, and 'registration': {'position'
         (F,3), 'rotation' (F,3,3), 'inliers', 'rms_m', 'iterations', 'converged', 'degenerate'} (per frame; a frame with
         fewer than 6 inliers is degenerate and keeps its pose).  alignment_error and voxel_map work on it unchanged."""
+        if metric not in ('point', 'plane'):
+            raise ValueError("metric must be 'point' or 'plane'")
         scans = results['raw_scans']
         env = results.get('environment') if map_points is None else map_points
         if env is None:
@@ -455,7 +461,12 @@ class LiDARMotionSimulator:
         pmap = ops.build_point_map(self._to_dev(np.asarray(env, np.float64).reshape(-1, 4)), leaf, origin)
         pts_d = self._to_dev(np.asarray(flat, np.float64).reshape(-1, 4))
         off_d = self._to_dev(off)
-        pose, st = ops.register_frames(pts_d, off_d, pose0, pmap, max_dist, iters=iters)
+        if metric == 'plane':
+            radius = min(pmap.leaf) if normal_radius is None else normal_radius
+            normals, _ = ops.estimate_normals(pmap, radius)
+            pose, st = ops.register_frames(pts_d, off_d, pose0, pmap, max_dist, iters=iters, normals=normals, min_planarity=min_planarity)
+        else:
+            pose, st = ops.register_frames(pts_d, off_d, pose0, pmap, max_dist, iters=iters)
         ops.ExportBuffers(status=st.status).raise_for_flags()
         if int(off[-1]):
             out, _ = ops.align_rigid(pts_d if self._np_dtype() == np.float64 else pts_d.float(), off_d, pose)
